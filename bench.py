@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — fused joint + RNN-T loss forward/backward throughput (BASELINE.json `metric`).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--precision bf16|fp32]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--precision bf16|fp32] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Workload = BASELINE.json configs[1]: synthetic B=32, T=250 (post-subsampling), U=40, H=D=512, V=412 per
@@ -16,6 +16,11 @@ weights, per-utterance costs compared with the GPU step; `gpu_reference` - the r
 through the library kernels it would use (cuBLAS + torchaudio's rnnt_loss CUDA kernels, ATen ctc_loss); `fp32` - the
 reference-precision path; `eager` - the ungraphed ragged-batch public API; `predictor` - the LSTM sequence kernels of
 section 8f row 2 beside the library LSTM on the same GPU; `decode` - the A4-A10 rows with RTF.
+
+`--dump-outputs DIR` writes what the last timed step handed its caller (rank 0): the loss and the gradients of the
+inputs and of the joint's parameters, as DIR/<name>.npy in float32.  Inputs and weights are seeded, so two builds run
+with the same arguments can be compared output for output; compare with a tolerance, since the summation order of
+d_ffn_out.bias varies from run to run (two runs of the same build on one B200 differed by 6e-5 at a magnitude of 249).
 """
 import argparse
 import json
@@ -25,10 +30,13 @@ import sys
 import threading
 import time
 
+import numpy as np
 import torch
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+
+DUMP_LIMIT_BYTES = 64 * 10**6
 
 CFG = dict(B=32, T=250, U=40, D=512, V=412, blank=5)
 METRIC = "fused joint+RNN-T loss fwd/bwd throughput"
@@ -145,6 +153,21 @@ def bench_weights(device=None):
     lin = lambda o, i: torch.nn.Linear(i, o)
     mods = {"enc_ffn": lin(D, D), "pred_ffn": lin(D, D), "ffn_out": lin(V, D)}
     return {f"{k}.{n}": p.detach().clone() for k, m in mods.items() for n, p in m.named_parameters()}
+
+
+def dump_outputs(path, outputs, limit=DUMP_LIMIT_BYTES):
+    """Write {name: tensor} as path/<name>.npy in float32, at most `limit` bytes in all.  Smallest first, each output
+    gets an equal share of what is left; one larger than its share is replaced by a seeded sample of its flattened
+    elements (in index order), so that runs with the same arguments write the same elements."""
+    os.makedirs(path, exist_ok=True)
+    arrays = sorted(((n, t.detach().float().cpu().numpy()) for n, t in outputs.items()), key=lambda kv: kv[1].size)
+    left = limit - 256 * len(arrays)                   # room for the .npy headers
+    for i, (name, a) in enumerate(arrays):
+        share = left // (len(arrays) - i) // a.itemsize
+        if a.size > share:
+            a = a.reshape(-1)[np.sort(np.random.default_rng(0).choice(a.size, share, replace=False))]
+        np.save(os.path.join(path, name + ".npy"), a)
+        left -= a.nbytes
 
 
 def cpu_reference_step(threads, seed=1234):
@@ -355,6 +378,11 @@ def run_ours(args):
         barrier()
         tot_ms = sum(s.elapsed_time(e_) for s, e_ in evs)
         launches = _lib.lib().ctcvr_launch_count() - l0
+        if args.dump_outputs and rank == 0:
+            e_in, p_in = (graphed.enc, graphed.pred) if graphed is not None else (enc, pred)
+            outs = {"loss": loss, "d_enc_out": e_in.grad, "d_pred_out": p_in.grad}
+            outs.update({f"d_{n}": p.grad for n, p in joint.named_parameters()})
+            dump_outputs(args.dump_outputs, outs)
         if graphed is not None:      # replays do not pass through the C ABI: the captured launches, counted above
             launches = args.steps * launches_per_step
         # ---- e2e: host (pinned) inputs -> H2D -> step -> D2H of the loss, every step.  As in a real input pipeline the
@@ -823,6 +851,7 @@ def time_kernels(C, joint, enc, pred, tgt, tl, ul, blank, precision, flush, reps
 
 
 def main():
+    sys.dont_write_bytecode = True      # the tree may be read-only: the benchmark writes nothing into it
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
     ap.add_argument("--steps", type=int, default=10)
@@ -835,7 +864,13 @@ def main():
     ap.add_argument("--allreduce", default="peer", choices=["peer", "nccl"],
                     help="N>1: gradient sum by the in-graph NVLink peer kernel (default) or by NCCL behind the graph")
     ap.add_argument("--no-decode", action="store_true", help="skip the A4-A10 rows (bench_decode.py) in the JSON line")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the loss and gradients of the last timed step as DIR/<name>.npy (float32, <= 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -294,3 +294,27 @@ def test_mm3_fallback_and_precision_switch_restored(monkeypatch):
     CF._mm3(a.t().contiguous(), b.t().contiguous(), out=out, a_t=True, b_t=True)
     assert torch.allclose(out, a @ b)
     assert torch.backends.cuda.matmul.fp32_precision == before
+
+
+def test_bench_dump_outputs_float32_bounded_and_repeatable(tmp_path):
+    """bench.py --dump-outputs: every output lands as float32 <name>.npy; over the byte limit the large outputs are
+    cut to a seeded sample of their elements, the same one on every run, and the files stay within the limit."""
+    import numpy as np
+    import bench
+    g = torch.Generator().manual_seed(0)
+    outs = {"loss": torch.tensor(1.5), "d_w": torch.randn(40, 30, generator=g).bfloat16(),
+            "d_x": torch.randn(100, 100, generator=g)}
+    bench.dump_outputs(str(tmp_path / "all"), outs)
+    for n, t in outs.items():
+        a = np.load(tmp_path / "all" / f"{n}.npy")
+        assert a.dtype == np.float32 and np.array_equal(a, t.float().numpy())
+    limit = 20000
+    for run in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / run), outs, limit=limit)
+    files = sorted(os.listdir(tmp_path / "a"))
+    assert files == ["d_w.npy", "d_x.npy", "loss.npy"]
+    assert sum(os.path.getsize(tmp_path / "a" / f) for f in files) <= limit
+    a, b = np.load(tmp_path / "a" / "d_x.npy"), np.load(tmp_path / "b" / "d_x.npy")
+    assert 0 < a.size < 100 * 100 and np.array_equal(a, b)
+    assert np.isin(a, outs["d_x"].numpy().ravel()).all()
+    assert np.array_equal(np.load(tmp_path / "a" / "loss.npy"), np.float32(1.5))

@@ -26,12 +26,12 @@ size_t joint_bwd_f32_ws_bytes(int, int, int, int, int);
 int joint_bwd_f32(const float*, const float*, const float*, const float*, const int32_t*, const int32_t*,
                   const int32_t*, const float*, const float*, const float*, const float*, const float*, float, float*,
                   float*, float*, float*, int, int, int, int, int, int, void*, size_t, cudaStream_t);
-size_t joint_fwd_tc_ws_bytes(int, int, int, int, int);
-int joint_fwd_tc(const void*, const void*, int, const float*, const float*, const int32_t*, const int32_t*,
+size_t joint_fwd_tc_ws_bytes(int, int, int, int, int, int);
+int joint_fwd_tc(const void*, const void*, int, int, const float*, const float*, const int32_t*, const int32_t*,
                  const int32_t*, float*, float*, float*, int, int, int, int, int, int, void*, size_t, cudaStream_t);
 bool joint_tc_bwd_supported(int, int, int);
-size_t joint_bwd_tc_ws_bytes(int, int, int, int, int);
-int joint_bwd_tc(const void*, const void*, int, const float*, const float*, const int32_t*, const int32_t*,
+size_t joint_bwd_tc_ws_bytes(int, int, int, int, int, int);
+int joint_bwd_tc(const void*, const void*, int, int, const float*, const float*, const int32_t*, const int32_t*,
                  const int32_t*, const float*, const float*, const float*, const float*, const float*, const float*,
                  const float*, float, float*,
                  float*, float*, float*, int, int, int, int, int, int, void*, size_t, cudaStream_t);
@@ -122,7 +122,9 @@ int ctcvr_joint_logits(const float* enc_proj, const float* pred_proj, const floa
 }
 
 size_t ctcvr_joint_rnnt_fwd_ws_bytes(int B, int T, int U1, int D, int V, int precision) {
-  return precision == CTCVR_BF16 ? joint_fwd_tc_ws_bytes(B, T, U1, D, V) : 256;
+  if (precision == CTCVR_BF16 || precision == CTCVR_BF16X3)
+    return joint_fwd_tc_ws_bytes(B, T, U1, D, V, precision == CTCVR_BF16X3);
+  return 256;
 }
 
 int ctcvr_joint_rnnt_fwd(const float* enc_proj, const float* pred_proj, const float* w_out, const float* b_out,
@@ -133,8 +135,8 @@ int ctcvr_joint_rnnt_fwd(const float* enc_proj, const float* pred_proj, const fl
   CTCVR_REQUIRE(enc_proj && pred_proj && w_out && b_out && t_len && u_len && lse && lp_blank && lp_label &&
                     (targets || U1 == 1), "joint_rnnt_fwd: NULL pointer");
   CTCVR_REQUIRE(blank >= 0 && blank < V, "joint_rnnt_fwd: blank %d must be within [0, %d)", blank, V);
-  if (precision == CTCVR_BF16)
-    return joint_fwd_tc(enc_proj, pred_proj, 0, w_out, b_out, targets, t_len, u_len, lse, lp_blank, lp_label, B, T, U1, D,
+  if (precision == CTCVR_BF16 || precision == CTCVR_BF16X3)
+    return joint_fwd_tc(enc_proj, pred_proj, 0, precision == CTCVR_BF16X3, w_out, b_out, targets, t_len, u_len, lse, lp_blank, lp_label, B, T, U1, D,
                         V, blank, ws, ws_bytes, ST(stream));
   CTCVR_REQUIRE(precision == CTCVR_F32, "joint_rnnt_fwd: unknown precision %d", precision);
   return joint_fwd_f32(enc_proj, pred_proj, w_out, b_out, targets, t_len, u_len, lse, lp_blank, lp_label, B, T, U1, D,
@@ -149,7 +151,9 @@ int ctcvr_rnnt_lattice(const float* lp_blank, const float* lp_label, const int32
 }
 
 size_t ctcvr_joint_rnnt_bwd_ws_bytes(int B, int T, int U1, int D, int V, int precision) {
-  return precision == CTCVR_BF16 ? joint_bwd_tc_ws_bytes(B, T, U1, D, V) : joint_bwd_f32_ws_bytes(B, T, U1, D, V);
+  if (precision == CTCVR_BF16 || precision == CTCVR_BF16X3)
+    return joint_bwd_tc_ws_bytes(B, T, U1, D, V, precision == CTCVR_BF16X3);
+  return joint_bwd_f32_ws_bytes(B, T, U1, D, V);
 }
 
 int ctcvr_joint_rnnt_bwd(const float* enc_proj, const float* pred_proj, const float* w_out, const float* b_out,
@@ -164,8 +168,8 @@ int ctcvr_joint_rnnt_bwd(const float* enc_proj, const float* pred_proj, const fl
                     beta && costs && grad_costs && d_enc_proj && d_pred_proj && d_w_out && d_b_out && ws,
                 "joint_rnnt_bwd: NULL pointer");
   CTCVR_REQUIRE(blank >= 0 && blank < V, "joint_rnnt_bwd: blank %d must be within [0, %d)", blank, V);
-  if (precision == CTCVR_BF16)
-    return joint_bwd_tc(enc_proj, pred_proj, 0, w_out, b_out, targets, t_len, u_len, lse, lp_blank, lp_label, alpha, beta, costs, grad_costs,
+  if (precision == CTCVR_BF16 || precision == CTCVR_BF16X3)
+    return joint_bwd_tc(enc_proj, pred_proj, 0, precision == CTCVR_BF16X3, w_out, b_out, targets, t_len, u_len, lse, lp_blank, lp_label, alpha, beta, costs, grad_costs,
                         clamp, d_enc_proj, d_pred_proj, d_w_out, d_b_out, B, T, U1, D, V, blank, ws, ws_bytes,
                         ST(stream));
   CTCVR_REQUIRE(precision == CTCVR_F32, "joint_rnnt_bwd: unknown precision %d", precision);
@@ -184,7 +188,7 @@ int ctcvr_joint_rnnt_fwd_bf16in(const void* enc_proj_bf16, const void* pred_proj
   CTCVR_REQUIRE(enc_proj_bf16 && pred_proj_bf16 && w_out && b_out && t_len && u_len && lse && lp_blank && lp_label &&
                     (targets || U1 == 1), "joint_rnnt_fwd_bf16in: NULL pointer");
   CTCVR_REQUIRE(blank >= 0 && blank < V, "joint_rnnt_fwd_bf16in: blank %d must be within [0, %d)", blank, V);
-  return joint_fwd_tc(enc_proj_bf16, pred_proj_bf16, 1, w_out, b_out, targets, t_len, u_len, lse, lp_blank, lp_label, B,
+  return joint_fwd_tc(enc_proj_bf16, pred_proj_bf16, 1, 0, w_out, b_out, targets, t_len, u_len, lse, lp_blank, lp_label, B,
                       T, U1, D, V, blank, ws, ws_bytes, ST(stream));
 }
 
@@ -199,7 +203,7 @@ int ctcvr_joint_rnnt_bwd_bf16in(const void* enc_proj_bf16, const void* pred_proj
   CTCVR_REQUIRE(enc_proj_bf16 && pred_proj_bf16 && w_out && b_out && t_len && u_len && lse && lp_blank && lp_label &&
                     alpha && beta && costs && grad_costs && d_enc_proj_bf16 && d_pred_proj_bf16 && d_w_out && d_b_out && ws, "joint_rnnt_bwd_bf16in: NULL pointer");
   CTCVR_REQUIRE(blank >= 0 && blank < V, "joint_rnnt_bwd_bf16in: blank %d must be within [0, %d)", blank, V);
-  return joint_bwd_tc(enc_proj_bf16, pred_proj_bf16, 1, w_out, b_out, targets, t_len, u_len, lse, lp_blank, lp_label, alpha, beta, costs,
+  return joint_bwd_tc(enc_proj_bf16, pred_proj_bf16, 1, 0, w_out, b_out, targets, t_len, u_len, lse, lp_blank, lp_label, alpha, beta, costs,
                       grad_costs, clamp, reinterpret_cast<float*>(d_enc_proj_bf16), reinterpret_cast<float*>(d_pred_proj_bf16),
                       d_w_out, d_b_out, B, T, U1, D, V, blank, ws, ws_bytes, ST(stream));
 }

@@ -185,25 +185,45 @@ __device__ __forceinline__ void dwr_rows(const uint32_t (&e)[TT], const uint32_t
   }
 }
 
+// bf16x3: the same rows as hi / lo pairs of the fp32 tanh(e + p)
+template <int P, int TT, int R0, int NP>
+__device__ __forceinline__ void dwr_rows_x3(const float (&e)[TT], const float (&pr)[P], uint32_t (&hi)[NP], uint32_t (&lo)[NP]) {
+#pragma unroll
+  for (int c = 0; c < NP; ++c) {
+    const int r0 = R0 + 2 * c, r1 = r0 + 1;
+    const int tl0 = (r0 / P < TT) ? r0 / P : TT - 1, tl1 = (r1 / P < TT) ? r1 / P : TT - 1;
+    const float z0 = tanhf(e[tl0] + pr[r0 % P]), z1 = tanhf(e[tl1] + pr[r1 % P]);
+    const __nv_bfloat162 h = __floats2bfloat162_rn(z0, z1);
+    hi[c] = *reinterpret_cast<const uint32_t*>(&h);
+    lo[c] = pack_bf16(z0 - __low2float(h), z1 - __high2float(h));
+  }
+}
+
 constexpr int DWR_S_STAGES = 3;
+constexpr int DW_STAGES_X3 = 4;                  // bf16x3: the G_hi and G_lo stages of two k-blocks (no slab ring)
 template <int P>
 __host__ __device__ constexpr uint32_t dwr_slab_bytes() {          // [d half][pred region | enc region], 1 KB aligned (SW128)
   return 2u * (bwd_pred_region<P>() + 1024u);
 }
 
-template <int P, int TT>
-__global__ void __launch_bounds__(DWR_THREADS, 1)
-dw_gemm_rz_kernel(const __grid_constant__ CUtensorMap tmap_e, const __grid_constant__ CUtensorMap tmap_p,
-                  const __nv_bfloat16* __restrict__ gr, const int4* __restrict__ tile_rows,
-                  const int* __restrict__ ntiles_ptr, float* __restrict__ partials, int D, int Vp, int KBG, int KS) {
+// SPLIT = true (precision bf16x3): dW^T = z_hi^T G_hi + z_hi^T G_lo + z_lo^T G_hi.  Per 64-row k-block the G loader
+// brings a G_hi and a G_lo stage (from the two spills), the producers write a z_hi and a z_lo A stage (z in fp32 from
+// the fp32 rows, read straight from global memory: no slab ring, warp 3 idles).
+template <int P, int TT, bool SPLIT>
+__device__ __forceinline__ void dw_gemm_rz_body(const CUtensorMap& tmap_e, const CUtensorMap& tmap_p,
+                                                const __nv_bfloat16* __restrict__ gr, const __nv_bfloat16* __restrict__ gr_lo,
+                                                const float* __restrict__ enc, const float* __restrict__ pred,
+                                                const int4* __restrict__ tile_rows, const int* __restrict__ ntiles_ptr,
+                                                float* __restrict__ partials, int D, int Vp, int KBG, int KS) {
   static_assert(TT <= 8, "enc region is one 1 KB swizzle atom");
+  constexpr int NS = SPLIT ? DW_STAGES_X3 : DW_STAGES;
   extern __shared__ uint8_t smem_raw[];
   const uint32_t base = smem_u32(smem_raw);
   const uint32_t al = (base + 1023u) & ~1023u;
   const uint32_t b_bytes = (uint32_t)KBG * 8192u;          // one 64-row half of a G tile: [KBG][64 rows][64 v]
-  const uint32_t slab = al + DW_STAGES * b_bytes;          // DWR_S_STAGES slabs of enc / pred rows (one per row tile)
-  const uint32_t bar = slab + DWR_S_STAGES * dwr_slab_bytes<P>();
-  uint32_t* tmem_ptr = reinterpret_cast<uint32_t*>(smem_raw + (bar + 192 - base));
+  const uint32_t slab = al + NS * b_bytes;                 // DWR_S_STAGES slabs of enc / pred rows (one per row tile)
+  const uint32_t bar = slab + (SPLIT ? 0u : DWR_S_STAGES * dwr_slab_bytes<P>());
+  uint32_t* tmem_ptr = reinterpret_cast<uint32_t*>(smem_raw + (bar + (NS + 6) * 16 + 48 - base));
   const int tid = threadIdx.x, warp = uniform_warp_idx(), lane = tid & 31;
   const int mb = blockIdx.x, ks = blockIdx.y;
   const int kblocks = (*ntiles_ptr) * 2;                   // 64-row k-blocks written by kernel 1
@@ -211,16 +231,18 @@ dw_gemm_rz_kernel(const __grid_constant__ CUtensorMap tmap_e, const __grid_const
   const int rt_begin = kb_begin >> 1, rt_end = (kb_end + 1) >> 1;
   auto full = [&](int i) { return bar + i * 16; };
   auto empty = [&](int i) { return bar + i * 16 + 8; };
-  auto a_full = [&](int i) { return bar + 48 + i * 16; };
-  auto a_empty = [&](int i) { return bar + 48 + i * 16 + 8; };
-  auto s_full = [&](int i) { return bar + 96 + i * 16; };
-  auto s_empty = [&](int i) { return bar + 96 + i * 16 + 8; };
-  const uint32_t done = bar + 144;
+  auto a_full = [&](int i) { return bar + NS * 16 + i * 16; };
+  auto a_empty = [&](int i) { return bar + NS * 16 + i * 16 + 8; };
+  auto s_full = [&](int i) { return bar + (NS + 3) * 16 + i * 16; };
+  auto s_empty = [&](int i) { return bar + (NS + 3) * 16 + i * 16 + 8; };
+  const uint32_t done = bar + (NS + 6) * 16;
 
   if (warp == 0 && lane == 0) {
-    tma_prefetch_desc(&tmap_e);
-    tma_prefetch_desc(&tmap_p);
-    for (int i = 0; i < DW_STAGES; ++i) { mbar_init(full(i), 1); mbar_init(empty(i), 1); }
+    if (!SPLIT) {                    // the split form gets placeholder tensor maps
+      tma_prefetch_desc(&tmap_e);
+      tma_prefetch_desc(&tmap_p);
+    }
+    for (int i = 0; i < NS; ++i) { mbar_init(full(i), 1); mbar_init(empty(i), 1); }
     for (int i = 0; i < DWR_A_STAGES; ++i) { mbar_init(a_full(i), 4 * DWR_ROW_PARTS); mbar_init(a_empty(i), 1); }
     for (int i = 0; i < DWR_S_STAGES; ++i) { mbar_init(s_full(i), 1); mbar_init(s_empty(i), 4 * DWR_ROW_PARTS); }
     mbar_init(done, 1);
@@ -235,16 +257,17 @@ dw_gemm_rz_kernel(const __grid_constant__ CUtensorMap tmap_e, const __grid_const
   if (warp == 0) {
     // ---- G loader: one 1-D bulk copy per stage
     Pipe sp;
-    for (int kb = kb_begin; kb < kb_end; ++kb) {
-      mbar_wait(empty(sp.stage), sp.phase ^ 1u, 50);
-      if (elect_one()) {
-        mbar_arrive_expect_tx(full(sp.stage), b_bytes);
-        bulk_load(al + sp.stage * b_bytes, gr + (size_t)kb * KBG * 4096, b_bytes, full(sp.stage));
+    for (int kb = kb_begin; kb < kb_end; ++kb)
+      for (int part = 0; part < (SPLIT ? 2 : 1); ++part) {     // bf16x3: G_hi, then G_lo
+        mbar_wait(empty(sp.stage), sp.phase ^ 1u, 50);
+        if (elect_one()) {
+          mbar_arrive_expect_tx(full(sp.stage), b_bytes);
+          bulk_load(al + sp.stage * b_bytes, (part ? gr_lo : gr) + (size_t)kb * KBG * 4096, b_bytes, full(sp.stage));
+        }
+        __syncwarp();
+        sp.advance(NS);
       }
-      __syncwarp();
-      sp.advance(DW_STAGES);
-    }
-  } else if (warp == 3) {
+  } else if (warp == 3 && !SPLIT) {
     // ---- slab loader: the P pred rows and TT enc rows of each row tile, this CTA's 128 d as two 64-wide boxes
     Pipe ss;
     for (int rt = rt_begin; rt < rt_end; ++rt) {
@@ -271,6 +294,39 @@ dw_gemm_rz_kernel(const __grid_constant__ CUtensorMap tmap_e, const __grid_const
     const uint32_t idesc1 = make_idesc_bf16_bmn(128, N1 > 0 ? N1 : 16);
     const uint64_t b_desc0 = make_desc_mn_sw128(al, 8192u, 1024u);
     const uint32_t st_step = b_bytes >> 4;
+    if constexpr (SPLIT) {
+      for (int kb = kb_begin; kb < kb_end; ++kb) {
+        Pipe sl = sp, al2 = ap;                              // the lo stages follow the hi stages
+        sl.advance(NS);
+        al2.advance(DWR_A_STAGES);
+        mbar_wait(a_full(ap.stage), ap.phase, 53);
+        mbar_wait(a_full(al2.stage), al2.phase, 53);
+        mbar_wait(full(sp.stage), sp.phase, 51);
+        mbar_wait(full(sl.stage), sl.phase, 51);
+        tc_fence_after();
+        if (elect_one()) {
+          const uint32_t a = tmem_base + DWR_ACC_COLS + ap.stage * 32, a2 = tmem_base + DWR_ACC_COLS + al2.stage * 32;
+          const uint64_t bh = b_desc0 + (uint64_t)(sp.stage * st_step), bl = b_desc0 + (uint64_t)(sl.stage * st_step);
+#pragma unroll
+          for (int k4 = 0; k4 < 4; ++k4) {
+            const uint32_t acc = (kb > kb_begin || k4 > 0) ? 1u : 0u;
+            umma_bf16_ts(tmem_base, a + 8 * k4, bh + 128 * k4, idesc0, acc);                       // z_hi G_hi
+            if (N1 > 0) umma_bf16_ts(tmem_base + 256, a + 8 * k4, bh + 2048 + 128 * k4, idesc1, acc);
+            umma_bf16_ts(tmem_base, a + 8 * k4, bl + 128 * k4, idesc0, 1u);                         // z_hi G_lo
+            if (N1 > 0) umma_bf16_ts(tmem_base + 256, a + 8 * k4, bl + 2048 + 128 * k4, idesc1, 1u);
+            umma_bf16_ts(tmem_base, a2 + 8 * k4, bh + 128 * k4, idesc0, 1u);                        // z_lo G_hi
+            if (N1 > 0) umma_bf16_ts(tmem_base + 256, a2 + 8 * k4, bh + 2048 + 128 * k4, idesc1, 1u);
+          }
+          umma_commit(empty(sp.stage));
+          umma_commit(empty(sl.stage));
+          umma_commit(a_empty(ap.stage));
+          umma_commit(a_empty(al2.stage));
+        }
+        __syncwarp();
+        sp.advance(NS); sp.advance(NS);
+        ap.advance(DWR_A_STAGES); ap.advance(DWR_A_STAGES);
+      }
+    } else
     for (int kb = kb_begin; kb < kb_end; ++kb) {
       mbar_wait(a_full(ap.stage), ap.phase, 53);
       mbar_wait(full(sp.stage), sp.phase, 51);
@@ -303,6 +359,51 @@ dw_gemm_rz_kernel(const __grid_constant__ CUtensorMap tmap_e, const __grid_const
     const uint32_t s_off = (uint32_t)(dl >> 6) * (bwd_pred_region<P>() + 1024u) + (uint32_t)(dl & 7) * 2u;
     const uint32_t s_chunk = (uint32_t)((dl & 63) >> 3);
     Pipe ap, ss;
+    if constexpr (SPLIT) {
+      for (int rt = rt_begin; rt < rt_end; ++rt) {
+        float e[TT], pr[P];
+        {
+          const int4 tr = __ldg(tile_rows + rt);           // {first enc row, first pred row, rows readable past them}
+#pragma unroll
+          for (int i = 0; i < P; ++i) pr[i] = __ldg(pred + (size_t)(tr.y + min(i, tr.w)) * D + d);
+#pragma unroll
+          for (int i = 0; i < TT; ++i) e[i] = __ldg(enc + (size_t)(tr.x + min(i, tr.z)) * D + d);
+        }
+#pragma unroll
+        for (int hh = 0; hh < 2; ++hh) {
+          const int kb = rt * 2 + hh;
+          if (kb < kb_begin || kb >= kb_end) continue;
+          constexpr int NP = 32 / DWR_ROW_PARTS;
+          uint32_t wh[NP], wl[NP];
+          auto rows = [&](auto HH) {
+            constexpr int R = decltype(HH)::value * 64;
+            if (rh == 0) dwr_rows_x3<P, TT, R, NP>(e, pr, wh, wl);
+            else if (rh == 1) dwr_rows_x3<P, TT, R + 2 * NP, NP>(e, pr, wh, wl);
+            else if (rh == 2) dwr_rows_x3<P, TT, R + 4 * NP, NP>(e, pr, wh, wl);
+            else dwr_rows_x3<P, TT, R + 6 * NP, NP>(e, pr, wh, wl);
+          };
+          if (hh == 0) rows(std::integral_constant<int, 0>{}); else rows(std::integral_constant<int, 1>{});
+          Pipe al2 = ap;
+          al2.advance(DWR_A_STAGES);
+          mbar_wait(a_empty(ap.stage), ap.phase ^ 1u, 54);
+          mbar_wait(a_empty(al2.stage), al2.phase ^ 1u, 54);
+          tc_fence_after();
+          if constexpr (NP == 16) {
+            tmem_st16(tq + (uint32_t)(DWR_ACC_COLS + ap.stage * 32 + rh * NP), wh);
+            tmem_st16(tq + (uint32_t)(DWR_ACC_COLS + al2.stage * 32 + rh * NP), wl);
+          } else {
+            tmem_st8(tq + (uint32_t)(DWR_ACC_COLS + ap.stage * 32 + rh * NP), wh);
+            tmem_st8(tq + (uint32_t)(DWR_ACC_COLS + al2.stage * 32 + rh * NP), wl);
+          }
+          tmem_st_wait();
+          tc_fence_before();
+          warp_arrive(a_full(ap.stage));
+          warp_arrive(a_full(al2.stage));
+          ap.advance(DWR_A_STAGES);
+          ap.advance(DWR_A_STAGES);
+        }
+      }
+    } else
     for (int rt = rt_begin; rt < rt_end; ++rt) {
       uint32_t e[TT], pr[P];
       mbar_wait(s_full(ss.stage), ss.phase, 56);
@@ -369,6 +470,29 @@ dw_gemm_rz_kernel(const __grid_constant__ CUtensorMap tmap_e, const __grid_const
   tc_fence_before();
   __syncthreads();
   if (warp == 2) tmem_dealloc(tmem_base, TMEM_COLS);
+}
+
+template <int P, int TT>
+__global__ void __launch_bounds__(DWR_THREADS, 1)
+dw_gemm_rz_kernel(const __grid_constant__ CUtensorMap tmap_e, const __grid_constant__ CUtensorMap tmap_p,
+                  const __nv_bfloat16* __restrict__ gr, const int4* __restrict__ tile_rows,
+                  const int* __restrict__ ntiles_ptr, float* __restrict__ partials, int D, int Vp, int KBG, int KS) {
+  dw_gemm_rz_body<P, TT, false>(tmap_e, tmap_p, gr, nullptr, nullptr, nullptr, tile_rows, ntiles_ptr, partials, D, Vp, KBG, KS);
+}
+// precision bf16x3 (the tensor maps are unused)
+template <int P, int TT>
+__global__ void __launch_bounds__(DWR_THREADS, 1)
+dw_gemm_rz_x3_kernel(const __grid_constant__ CUtensorMap tmap_e, const __grid_constant__ CUtensorMap tmap_p,
+                     const __nv_bfloat16* __restrict__ gr, const __nv_bfloat16* __restrict__ gr_lo,
+                     const float* __restrict__ enc, const float* __restrict__ pred, const int4* __restrict__ tile_rows,
+                     const int* __restrict__ ntiles_ptr, float* __restrict__ partials, int D, int Vp, int KBG, int KS) {
+  dw_gemm_rz_body<P, TT, true>(tmap_e, tmap_p, gr, gr_lo, enc, pred, tile_rows, ntiles_ptr, partials, D, Vp, KBG, KS);
+}
+
+// dW GEMM shared memory: G stages, slab ring (bf16 only), barriers
+template <int P>
+static size_t dwr_smem_bytes(int KBG, bool split) {
+  return 1024 + (size_t)(split ? DW_STAGES_X3 : DW_STAGES) * ((size_t)KBG * 8192) + (split ? 0 : DWR_S_STAGES * dwr_slab_bytes<P>()) + 256;
 }
 
 // d_w[v][d] = sum_ks partials[ks][d][v].  Block = 8 d x 32 v (warp = d row, lanes = consecutive v: coalesced
@@ -467,11 +591,30 @@ __device__ void to_bf16_part(long first_i, long stride, const float4* __restrict
 //   w_t  [KB][2][NH][64]   stage (kb,h): rows v' = v - h*NH, k' = k - 64 kb; chunk (k'>>3) stored at (k'>>3) ^ (v'&7)
 //   wt_t [MB][KBG][128][64] stage (mb,kb): rows d' = d - 128 mb, v' = v - 64 kb; chunk (v'>>3) at (v'>>3) ^ (d'&7)
 // plus bias_pad / bias_l2.  One thread per (v, d) of the zero-padded [KBG*64][D] weight.
+// SPLIT (bf16x3): x = hi + lo with hi = bf16(x), lo = bf16(x - hi); each stage block is followed by its lo twin:
+//   w_t  [KB][hi, lo][2][NH][64]        wt_t [MB][KBG][hi, lo][128][64]
+template <bool SPLIT>
 __device__ void prep_weights3_part(int i, const float* __restrict__ w, const float* __restrict__ bias,
                                    __nv_bfloat16* __restrict__ w_t, __nv_bfloat16* __restrict__ wt_t,
                                    float* __restrict__ bias_pad, float* __restrict__ bias_l2, int V, int Vp, int D) {
   const int KBG = (Vp + 63) / 64, NH = Vp / 2;
-  if (i < KBG * 64 * D) {
+  if (SPLIT && i < KBG * 64 * D) {
+    const int v = i / D, d = i - v * D;
+    const float xf = (v < V) ? w[(size_t)v * D + d] : 0.f;
+    const __nv_bfloat16 hi = __float2bfloat16(xf), lo = __float2bfloat16(xf - __bfloat162float(hi));
+    if (v < Vp) {
+      const int h = v / NH, vl = v - h * NH, kb = d >> 6, kl = d & 63;
+      const size_t o = (size_t)vl * 64 + (((kl >> 3) ^ (vl & 7)) << 3) + (kl & 7);
+      w_t[(size_t)(kb * 4 + h) * NH * 64 + o] = hi;
+      w_t[(size_t)(kb * 4 + 2 + h) * NH * 64 + o] = lo;
+    }
+    if (wt_t) {
+      const int mb = d >> 7, dl = d & 127, kb = v >> 6, vl = v & 63;
+      const size_t o = (size_t)(mb * KBG + kb) * 16384 + dl * 64 + (((vl >> 3) ^ (dl & 7)) << 3) + (vl & 7);
+      wt_t[o] = hi;
+      wt_t[o + 8192] = lo;
+    }
+  } else if (!SPLIT && i < KBG * 64 * D) {
     const int v = i / D, d = i - v * D;
     const __nv_bfloat16 x = __float2bfloat16((v < V) ? w[(size_t)v * D + d] : 0.f);
     if (v < Vp) {
@@ -519,10 +662,11 @@ struct PrepArgs {
   float* zero0; long n0; float* zero1; long n1;
   const float4* a; uint2* ab; long na4; const float4* b4; uint2* bb; long nb4;
 };
+template <bool SPLIT>
 __global__ void __launch_bounds__(256) prep_kernel(const PrepArgs q) {
   const int blk = blockIdx.x;
   if (blk < q.nW) {
-    prep_weights3_part(blk * 256 + threadIdx.x, q.w, q.bias, q.w_t, q.wt_t, q.bias_pad, q.bias_l2, q.V, q.Vp, q.D);
+    prep_weights3_part<SPLIT>(blk * 256 + threadIdx.x, q.w, q.bias, q.w_t, q.wt_t, q.bias_pad, q.bias_l2, q.V, q.Vp, q.D);
   } else if (blk < q.nW + q.B) {
     if (q.geom) build_tiles_block(blk - q.nW, q.t_len, q.u_len, q.B, q.T, q.U1, q.geom, q.tiles, q.tile_rows, q.ntiles, q.max_tiles);
     else build_tiles_fwd_block(blk - q.nW, q.t_len, q.u_len, q.B, q.T, q.U1, q.tiles, q.ntiles, q.max_tiles, q.fwd_pair);
@@ -628,15 +772,16 @@ struct FwdWs {
   int* ntiles;
   size_t bytes;
 };
-static FwdWs carve_fwd_ws(void* ws, int B, int T, int U1, int D, int V) {
+// split (bf16x3): hi and lo copies of W_out; the fp32 activations are read in place (no bf16 copies)
+static FwdWs carve_fwd_ws(void* ws, int B, int T, int U1, int D, int V, bool split = false) {
   int Vp = pad_v(V);
   uint8_t* p = reinterpret_cast<uint8_t*>(ws);
   size_t off = 0;
   FwdWs w;
   auto take = [&](size_t n) { void* r = p + off; off = align_up(off + n, 1024); return r; };
-  w.wb = reinterpret_cast<__nv_bfloat16*>(take((size_t)Vp * D * 2));
-  w.eb = reinterpret_cast<__nv_bfloat16*>(take((size_t)B * T * D * 2));
-  w.pb = reinterpret_cast<__nv_bfloat16*>(take((size_t)B * U1 * D * 2));
+  w.wb = reinterpret_cast<__nv_bfloat16*>(take((size_t)Vp * D * 2 * (split ? 2 : 1)));
+  w.eb = split ? nullptr : reinterpret_cast<__nv_bfloat16*>(take((size_t)B * T * D * 2));
+  w.pb = split ? nullptr : reinterpret_cast<__nv_bfloat16*>(take((size_t)B * U1 * D * 2));
   w.bias_pad = reinterpret_cast<float*>(take((size_t)Vp * 4));
   w.bias_l2 = reinterpret_cast<float*>(take((size_t)Vp * 4));
   const int mt = max_tiles_flat(B, T, U1) > max_tiles_fwd2(B, T, U1) ? max_tiles_flat(B, T, U1) : max_tiles_fwd2(B, T, U1);
@@ -646,9 +791,9 @@ static FwdWs carve_fwd_ws(void* ws, int B, int T, int U1, int D, int V) {
   return w;
 }
 
-size_t joint_fwd_tc_ws_bytes(int B, int T, int U1, int D, int V) {
+size_t joint_fwd_tc_ws_bytes(int B, int T, int U1, int D, int V, int split) {
   if (!joint_tc_bwd_supported(U1, D, V)) return 256;      // the call itself fails with the reason
-  return carve_fwd_ws(nullptr, B, T, U1, D, V).bytes;
+  return carve_fwd_ws(nullptr, B, T, U1, D, V, split != 0).bytes;
 }
 
 static int sm_count() {
@@ -665,20 +810,48 @@ static int sm_count() {
 int joint_fwd_f32(const float*, const float*, const float*, const float*, const int32_t*, const int32_t*,
                   const int32_t*, float*, float*, float*, int, int, int, int, int, int, cudaStream_t);
 
-int joint_fwd_tc(const void* enc_v, const void* pred_v, int in_bf16, const float* w, const float* bias, const int32_t* targets,
-                 const int32_t* t_len, const int32_t* u_len, float* lse, float* lp_blank, float* lp_label, int B, int T,
-                 int U1, int D, int V, int blank, void* ws, size_t ws_bytes, cudaStream_t st) {
+// split = 1: precision bf16x3 (fp32 inputs, hi / lo operand split, joint_fwd2_x3_kernel)
+int joint_fwd_tc(const void* enc_v, const void* pred_v, int in_bf16, int split, const float* w, const float* bias,
+                 const int32_t* targets, const int32_t* t_len, const int32_t* u_len, float* lse, float* lp_blank,
+                 float* lp_label, int B, int T, int U1, int D, int V, int blank, void* ws, size_t ws_bytes, cudaStream_t st) {
   const float* enc = reinterpret_cast<const float*>(enc_v);
   const float* pred = reinterpret_cast<const float*>(pred_v);
   // one predicate for both directions, and no silent change of arithmetic: a shape outside the tensor-core tiling is
   // an error here (the fp32 kernels are ~40x slower and round differently - the caller has to ask for them)
-  CTCVR_REQUIRE(joint_tc_bwd_supported(U1, D, V), "%s: precision = bf16 needs D %% 128 == 0, D <= 512, V <= 416 and U+1 <= 128 (got D=%d V=%d U+1=%d); use precision = fp32 for this shape", "joint_rnnt_fwd", D, V, U1);
+  CTCVR_REQUIRE(joint_tc_bwd_supported(U1, D, V), "%s: precision = %s needs D %% 128 == 0, D <= 512, V <= 416 and U+1 <= 128 (got D=%d V=%d U+1=%d); use precision = fp32 for this shape", "joint_rnnt_fwd", split ? "bf16x3" : "bf16", D, V, U1);
   if (check_tc_error("joint_rnnt_fwd")) return 1;
-  CTCVR_REQUIRE(ws && ws_bytes >= joint_fwd_tc_ws_bytes(B, T, U1, D, V), "joint_rnnt_fwd bf16: workspace too small");
-  CTCVR_REQUIRE(((uintptr_t)enc & 15) == 0 && ((uintptr_t)pred & 15) == 0, "joint_rnnt_fwd bf16: enc_proj / pred_proj must be 16-byte aligned");
+  CTCVR_REQUIRE(ws && ws_bytes >= joint_fwd_tc_ws_bytes(B, T, U1, D, V, split), "joint_rnnt_fwd %s: workspace too small", split ? "bf16x3" : "bf16");
+  CTCVR_REQUIRE(((uintptr_t)enc & 15) == 0 && ((uintptr_t)pred & 15) == 0, "joint_rnnt_fwd %s: enc_proj / pred_proj must be 16-byte aligned", split ? "bf16x3" : "bf16");
   const int Vp = pad_v(V), NH = Vp / 2;
-  FwdWs W = carve_fwd_ws(ws, B, T, U1, D, V);
+  FwdWs W = carve_fwd_ws(ws, B, T, U1, D, V, split != 0);
   const int mt = max_tiles_fwd2(B, T, U1);
+  if (split) {
+    PrepArgs q{};
+    q.w = w; q.bias = bias; q.w_t = W.wb; q.bias_l2 = W.bias_l2; q.V = V; q.Vp = Vp; q.D = D;
+    q.nW = cdiv((long)((Vp + 63) / 64) * 64 * D, 256);
+    q.t_len = t_len; q.u_len = u_len; q.B = B; q.T = T; q.U1 = U1; q.geom = 0; q.max_tiles = mt;
+    q.tiles = W.tiles; q.ntiles = W.ntiles;
+    prep_kernel<true><<<q.nW + B, 256, 0, st>>>(q);
+    CTCVR_LAUNCH_CHECK();
+    FwdParams p{};
+    p.w_t = W.wb; p.enc = enc; p.pred = pred;
+    p.bias = bias; p.bias_l2 = W.bias_l2; p.targets = targets; p.t_len = t_len; p.u_len = u_len;
+    p.tiles = W.tiles; p.ntiles = W.ntiles;
+    p.B = B; p.T = T; p.U1 = U1; p.D = D; p.V = V; p.Vp = Vp; p.NH = NH; p.blank = blank;
+    p.lse = lse; p.lp_blank = lp_blank; p.lp_label = lp_label;
+    p.prof = g_prof_buf;
+    tc_error_host_word(&p.err_host);
+    int ws_n = F_MAX_W_STAGES;
+    while (ws_n > 2 && fwd2_smem_bytes(NH, Vp, ws_n) > 232448) --ws_n;
+    p.w_stages = ws_n;
+    const size_t smem = fwd2_smem_bytes(NH, Vp, ws_n);
+    CTCVR_REQUIRE(smem <= 232448, "joint_rnnt_fwd bf16x3: shared memory budget exceeded (%zu B)", smem);
+    CTCVR_CHECK_CUDA(cudaFuncSetAttribute(joint_fwd2_x3_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    const CUtensorMap unused{};             // the bf16x3 producers read the fp32 rows directly
+    joint_fwd2_x3_kernel<<<min(sm_count(), mt), F_THREADS, smem, st>>>(unused, unused, p);
+    CTCVR_LAUNCH_CHECK();
+    return 0;
+  }
   const bool use_pair = fwdp_smem_bytes(NH, D) <= 232448 && sm_count() >= 2 && !g_force_single_cta;
   {
     PrepArgs q{};
@@ -696,7 +869,7 @@ int joint_fwd_tc(const void* enc_v, const void* pred_v, int in_bf16, const float
       q.b4 = reinterpret_cast<const float4*>(pred); q.bb = reinterpret_cast<uint2*>(W.pb); q.nb4 = (long)B * U1 * D / 4;
       extra = (int)std::min<long>((q.na4 + q.nb4 + 255) / 256, 148L * 8);
     }
-    prep_kernel<<<q.nW + B + extra, 256, 0, st>>>(q);
+    prep_kernel<false><<<q.nW + B + extra, 256, 0, st>>>(q);
     CTCVR_LAUNCH_CHECK();
   }
   if (use_pair) {
@@ -746,7 +919,7 @@ int joint_bwd_f32(const float*, const float*, const float*, const float*, const 
 
 
 struct BwdWs {
-  __nv_bfloat16 *wb, *wtb, *gt, *eb, *pb;
+  __nv_bfloat16 *wb, *wtb, *gt, *gt_lo, *eb, *pb;
   float *bias_pad, *bias_l2, *d_enc_part, *partials, *d_pred_acc;
   int4 *tiles, *tile_rows;
   int* ntiles;
@@ -754,7 +927,8 @@ struct BwdWs {
   int KS, S_max, mt;
   size_t bytes;
 };
-static BwdWs carve_bwd_ws(void* ws, int B, int T, int U1, int D, int V) {
+// split (bf16x3): hi / lo copies of W_out and W_out^T and a second G spill (G_lo); no bf16 activation copies
+static BwdWs carve_bwd_ws(void* ws, int B, int T, int U1, int D, int V, bool split = false) {
   const int Vp = pad_v(V);
   uint8_t* p = reinterpret_cast<uint8_t*>(ws);
   size_t off = 0;
@@ -766,16 +940,18 @@ static BwdWs carve_bwd_ws(void* ws, int B, int T, int U1, int D, int V) {
   w.KS = MB > 0 ? sm_count() / MB : 1;
   if (w.KS < 1) w.KS = 1;
   auto take = [&](size_t n) { void* r = p + off; off = align_up(off + n, 1024); return r; };
-  w.wb = reinterpret_cast<__nv_bfloat16*>(take((size_t)Vp * D * 2));
-  w.wtb = reinterpret_cast<__nv_bfloat16*>(take((size_t)((Vp + 63) / 64) * 64 * D * 2));
-  w.eb = reinterpret_cast<__nv_bfloat16*>(take((size_t)B * T * D * 2));
-  w.pb = reinterpret_cast<__nv_bfloat16*>(take((size_t)B * U1 * D * 2));
+  const size_t nw = split ? 2 : 1;
+  w.wb = reinterpret_cast<__nv_bfloat16*>(take((size_t)Vp * D * 2 * nw));
+  w.wtb = reinterpret_cast<__nv_bfloat16*>(take((size_t)((Vp + 63) / 64) * 64 * D * 2 * nw));
+  w.eb = split ? nullptr : reinterpret_cast<__nv_bfloat16*>(take((size_t)B * T * D * 2));
+  w.pb = split ? nullptr : reinterpret_cast<__nv_bfloat16*>(take((size_t)B * U1 * D * 2));
   w.bias_pad = reinterpret_cast<float*>(take((size_t)Vp * 4));
   w.bias_l2 = reinterpret_cast<float*>(take((size_t)Vp * 4));
   w.tiles = reinterpret_cast<int4*>(take((size_t)w.mt * 16));
   w.tile_rows = reinterpret_cast<int4*>(take((size_t)w.mt * 16));
   w.ntiles = reinterpret_cast<int*>(take(4));
   w.gt = reinterpret_cast<__nv_bfloat16*>(take((size_t)((Vp + 63) / 64) * 64 * w.Rpad * 2));
+  w.gt_lo = split ? reinterpret_cast<__nv_bfloat16*>(take((size_t)((Vp + 63) / 64) * 64 * w.Rpad * 2)) : nullptr;
   w.d_enc_part = reinterpret_cast<float*>(take((size_t)w.S_max * B * T * D * 4));
   w.partials = reinterpret_cast<float*>(take((size_t)w.KS * D * Vp * 4));
   w.d_pred_acc = reinterpret_cast<float*>(take((size_t)B * U1 * D * 4));
@@ -783,27 +959,76 @@ static BwdWs carve_bwd_ws(void* ws, int B, int T, int U1, int D, int V) {
   return w;
 }
 
-size_t joint_bwd_tc_ws_bytes(int B, int T, int U1, int D, int V) {
+size_t joint_bwd_tc_ws_bytes(int B, int T, int U1, int D, int V, int split) {
   if (!joint_tc_bwd_supported(U1, D, V)) return 256;      // the call itself fails with the reason
-  return carve_bwd_ws(nullptr, B, T, U1, D, V).bytes;
+  return carve_bwd_ws(nullptr, B, T, U1, D, V, split != 0).bytes;
 }
 
-int joint_bwd_tc(const void* enc_v, const void* pred_v, int in_bf16, const float* w, const float* bias, const int32_t* targets,
+// precision bf16x3: the single-CTA backward kernel and the dW GEMM in their split forms (fp32 inputs and gradients)
+template <int P, int TT>
+static int joint_bwd_x3(const float* enc, const float* pred, BwdParams& p, const BwdWs& W, const int32_t* t_len,
+                        const int32_t* u_len, float* d_enc, float* d_w, int B, int T, int U1, int D, int V, cudaStream_t st) {
+  const int Vp = p.Vp, KBG = (Vp + 63) / 64, MB = D / 128;
+  const CUtensorMap unused{};               // the split kernels read the fp32 rows directly
+  const size_t smem = bwd3_smem_bytes(p.NH, Vp, D, true);
+  CTCVR_REQUIRE(smem <= 232448 && p.r1_stages >= 2, "joint_rnnt_bwd bf16x3: shared memory budget exceeded (%zu B)", smem);
+  CTCVR_CHECK_CUDA(cudaFuncSetAttribute(joint_bwd3_x3_kernel<P, TT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  joint_bwd3_x3_kernel<P, TT><<<min(sm_count(), W.mt), NTHREADS, smem, st>>>(unused, unused, p);
+  CTCVR_LAUNCH_CHECK();
+  reduce_denc_kernel<false><<<B * T, 128, 0, st>>>(W.d_enc_part, t_len, u_len, d_enc, B, T, U1, D, P, nullptr, nullptr);
+  CTCVR_LAUNCH_CHECK();
+  const size_t smem2 = dwr_smem_bytes<P>(KBG, true);
+  CTCVR_REQUIRE(smem2 <= 232448, "dW GEMM bf16x3: shared memory budget exceeded (%zu B)", smem2);
+  CTCVR_CHECK_CUDA(cudaFuncSetAttribute(dw_gemm_rz_x3_kernel<P, TT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem2));
+  dw_gemm_rz_x3_kernel<P, TT><<<dim3(MB, W.KS), DWR_THREADS, smem2, st>>>(unused, unused, W.gt, W.gt_lo, enc, pred, W.tile_rows,
+                                                                        W.ntiles, W.partials, D, Vp, KBG, W.KS);
+  CTCVR_LAUNCH_CHECK();
+  reduce_dw_kernel<<<dim3(cdiv(D, 8), cdiv(Vp, 32)), 256, 0, st>>>(W.partials, d_w, D, V, Vp, W.KS);
+  CTCVR_LAUNCH_CHECK();
+  return 0;
+}
+
+int joint_bwd_tc(const void* enc_v, const void* pred_v, int in_bf16, int split, const float* w, const float* bias, const int32_t* targets,
                  const int32_t* t_len, const int32_t* u_len, const float* lse, const float* lp_blank, const float* lp_label,
                  const float* alpha, const float* beta,
                  const float* costs, const float* grad_costs, float clamp, float* d_enc, float* d_pred, float* d_w,
                  float* d_b, int B, int T, int U1, int D, int V, int blank, void* ws, size_t ws_bytes, cudaStream_t st) {
   const float* enc = reinterpret_cast<const float*>(enc_v);
   const float* pred = reinterpret_cast<const float*>(pred_v);
-  CTCVR_REQUIRE(joint_tc_bwd_supported(U1, D, V), "%s: precision = bf16 needs D %% 128 == 0, D <= 512, V <= 416 and U+1 <= 128 (got D=%d V=%d U+1=%d); use precision = fp32 for this shape", "joint_rnnt_bwd", D, V, U1);
+  CTCVR_REQUIRE(joint_tc_bwd_supported(U1, D, V), "%s: precision = %s needs D %% 128 == 0, D <= 512, V <= 416 and U+1 <= 128 (got D=%d V=%d U+1=%d); use precision = fp32 for this shape", "joint_rnnt_bwd", split ? "bf16x3" : "bf16", D, V, U1);
   if (check_tc_error("joint_rnnt_bwd")) return 1;
-  CTCVR_REQUIRE(ws && ws_bytes >= joint_bwd_tc_ws_bytes(B, T, U1, D, V), "joint_rnnt_bwd bf16: workspace too small");
-  CTCVR_REQUIRE(((uintptr_t)enc & 15) == 0 && ((uintptr_t)pred & 15) == 0, "joint_rnnt_bwd bf16: enc_proj / pred_proj must be 16-byte aligned");
+  CTCVR_REQUIRE(ws && ws_bytes >= joint_bwd_tc_ws_bytes(B, T, U1, D, V, split), "joint_rnnt_bwd %s: workspace too small", split ? "bf16x3" : "bf16");
+  CTCVR_REQUIRE(((uintptr_t)enc & 15) == 0 && ((uintptr_t)pred & 15) == 0, "joint_rnnt_bwd %s: enc_proj / pred_proj must be 16-byte aligned", split ? "bf16x3" : "bf16");
   const int Vp = pad_v(V), NH = Vp / 2, MB = D / 128;
-  BwdWs W = carve_bwd_ws(ws, B, T, U1, D, V);
+  BwdWs W = carve_bwd_ws(ws, B, T, U1, D, V, split != 0);
   const int KBG = (Vp + 63) / 64;
   const int mt = W.mt;
   RectGeom G = pick_rect_geom(T, U1);
+  if (split) {
+    PrepArgs q{};
+    q.w = w; q.bias = bias; q.w_t = W.wb; q.wt_t = W.wtb; q.bias_pad = W.bias_pad; q.bias_l2 = W.bias_l2;
+    q.V = V; q.Vp = Vp; q.D = D; q.nW = cdiv((long)KBG * 64 * D, 256);
+    q.t_len = t_len; q.u_len = u_len; q.B = B; q.T = T; q.U1 = U1; q.geom = G.P | (G.TT << 8);
+    q.max_tiles = mt; q.tiles = W.tiles; q.tile_rows = W.tile_rows; q.ntiles = W.ntiles;
+    q.zero0 = d_pred; q.n0 = (long)B * U1 * D; q.zero1 = d_b; q.n1 = V;
+    const int extra = (int)std::min<long>((q.n0 + 1023) / 1024, 148L * 8);
+    prep_kernel<true><<<q.nW + B + extra, 256, 0, st>>>(q);
+    CTCVR_LAUNCH_CHECK();
+    BwdParams p{};
+    p.w_t = W.wb; p.wt_t = W.wtb; p.enc = enc; p.pred = pred; p.gt_lo = W.gt_lo;
+    p.bias_l2 = W.bias_l2; p.targets = targets; p.t_len = t_len; p.u_len = u_len;
+    p.tiles = W.tiles; p.ntiles = W.ntiles;
+    p.B = B; p.T = T; p.U1 = U1; p.D = D; p.V = V; p.Vp = Vp; p.NH = NH; p.blank = blank;
+    p.r1_stages = bwd3_r1_stages(NH, Vp);
+    p.lse = lse; p.lp_blank = lp_blank; p.lp_label = lp_label;
+    p.alpha = alpha; p.beta = beta; p.costs = costs; p.grad_costs = grad_costs; p.clamp = clamp;
+    p.gt = W.gt;
+    p.d_enc_part = W.d_enc_part; p.d_pred = d_pred; p.d_bias = d_b;
+    p.prof = g_prof_buf;
+    tc_error_host_word(&p.err_host);
+    return G.P == 21 ? joint_bwd_x3<21, 6>(enc, pred, p, W, t_len, u_len, d_enc, d_w, B, T, U1, D, V, st)
+                     : joint_bwd_x3<16, 8>(enc, pred, p, W, t_len, u_len, d_enc, d_w, B, T, U1, D, V, st);
+  }
   // CTA-pair kernel (joint_tc_bwd_pair.cuh): D in 256-row blocks of dZ^T, tiles paired along the frame axis
   const size_t smem_pair = G.P == 21 ? bwd4_smem_bytes<21>(NH, Vp, D) : bwd4_smem_bytes<16>(NH, Vp, D);
   const bool use_pair = D % 256 == 0 && smem_pair <= 232448 && sm_count() >= 2 && bwd4_r1_stages(NH, Vp) >= 4 &&
@@ -826,7 +1051,7 @@ int joint_bwd_tc(const void* enc_v, const void* pred_v, int in_bf16, const float
       q.b4 = reinterpret_cast<const float4*>(pred); q.bb = reinterpret_cast<uint2*>(W.pb); q.nb4 = (long)B * U1 * D / 4;
     }
     const int extra = (int)std::min<long>((q.n0 + q.na4 * 4 + q.nb4 * 4 + 1023) / 1024, 148L * 8);
-    prep_kernel<<<q.nW + B + extra, 256, 0, st>>>(q);
+    prep_kernel<false><<<q.nW + B + extra, 256, 0, st>>>(q);
     CTCVR_LAUNCH_CHECK();
   }
   {

@@ -98,6 +98,10 @@ struct BwdParams {
   float* d_bias;            // [V] atomic accumulate
   long long* prof;
   unsigned int* err_host;   // mapped host word for bounded-wait time-outs (tc_common.cuh)
+  // bf16x3 only: the fp32 activations (read in place) and the spill of G_lo = bf16(G - G_hi), laid out as gt
+  const float* enc;
+  const float* pred;
+  __nv_bfloat16* gt_lo;
 };
 
 // Shared memory: [weight ring: 4 W^T stages][G tile (P2/P3)]  -- P1 views both as one W ring --
@@ -126,8 +130,13 @@ struct Bwd3Smem {
   __device__ __forceinline__ uint32_t tmem_empty() const { return bar_base + 288; }
   __device__ __forceinline__ uint32_t gs_done() const { return bar_base + 296; }   // G spilled and column-summed
   __device__ __forceinline__ uint32_t p4_full() const { return bar_base + 304; }
+  // bf16x3 only
+  __device__ __forceinline__ uint32_t p3a_done() const { return bar_base + 312; }   // the G_hi MMAs have completed
+  __device__ __forceinline__ uint32_t gs_hi_done() const { return bar_base + 320; } // G_hi column-summed
+  __device__ __forceinline__ uint32_t glo_full() const { return bar_base + 328; }   // G_lo reloaded into the G tile
 };
 constexpr uint32_t B_BAR_BYTES = 320;
+constexpr uint32_t B_BAR_BYTES_X3 = 352;
 
 __host__ __device__ inline uint32_t bwd3_g_bytes(int Vp) { return (uint32_t)((Vp + 63) / 64) * A_STAGE_BYTES; }
 // W_out stages that fit the ring + G region (the G tile is dead during P1)
@@ -136,27 +145,33 @@ __host__ __device__ inline int bwd3_r1_stages(int NH, int Vp) {
   return n > B_R1_MAX ? B_R1_MAX : n;
 }
 
-__host__ __device__ inline size_t bwd3_smem_bytes(int NH, int Vp, int D) {
+// split = true (bf16x3): no slab regions (the workers read the fp32 rows from global memory), three more barriers
+__host__ __device__ inline size_t bwd3_smem_bytes(int NH, int Vp, int D, bool split = false) {
   size_t s = 1024;
   s += B_RING_BYTES + bwd3_g_bytes(Vp);
-  s += (size_t)B_S_STAGES * B_SLAB_MAX;
-  s += (size_t)(D / BK) * B_SLAB_MAX;
+  if (!split) {
+    s += (size_t)B_S_STAGES * B_SLAB_MAX;
+    s += (size_t)(D / BK) * B_SLAB_MAX;
+  }
   s += (size_t)Vp * 4 + (size_t)4 * Vp * 4;
-  s += 16 + B_BAR_BYTES + 16;          // alignment + barriers + tmem pointer
+  s += 16 + (split ? B_BAR_BYTES_X3 : B_BAR_BYTES) + 16;          // alignment + barriers + tmem pointer
   return s;
 }
 
+template <bool SPLIT = false>
 __device__ __forceinline__ void carve_bwd3(Bwd3Smem& L, uint8_t* raw, int NH, int Vp, int D) {
   const uint32_t base = smem_u32(raw);
   uint32_t a = (base + 1023u) & ~1023u;
   L.r_base = a; L.r1_bytes = (uint32_t)NH * 128u; a += B_RING_BYTES;
   L.g_base = a; a += bwd3_g_bytes(Vp);
-  L.s_base = a; a += B_S_STAGES * B_SLAB_MAX;
-  L.p4_base = a; a += (uint32_t)(D / BK) * B_SLAB_MAX;
+  if (!SPLIT) {
+    L.s_base = a; a += B_S_STAGES * B_SLAB_MAX;
+    L.p4_base = a; a += (uint32_t)(D / BK) * B_SLAB_MAX;
+  }
   L.bias_l2 = reinterpret_cast<float*>(raw + (a - base)); a += Vp * 4;
   L.dbp = reinterpret_cast<float*>(raw + (a - base)); a += 4 * Vp * 4;
   a = (a + 15u) & ~15u;
-  L.bar_base = a; a += B_BAR_BYTES;
+  L.bar_base = a; a += SPLIT ? B_BAR_BYTES_X3 : B_BAR_BYTES;
   L.tmem_ptr = reinterpret_cast<uint32_t*>(raw + (a - base));
 }
 
@@ -188,13 +203,36 @@ __device__ __forceinline__ void p4_chunk(const float (&w)[16], const uint32_t (&
   }
 }
 
-template <int P, int TT>
-__global__ void __launch_bounds__(NTHREADS, 1)
-joint_bwd3_kernel(const __grid_constant__ CUtensorMap tmap_e, const __grid_constant__ CUtensorMap tmap_p,
-                  const BwdParams p) {
+// bf16x3 form of p4_chunk: z = tanh(e + p) in fp32 from the fp32 rows
+template <int P, int TT, int C0>
+__device__ __forceinline__ void p4_chunk(const float (&w)[16], const float (&e)[TT], const float (&pr)[P],
+                                             float (&es)[TT], float (&pa)[P]) {
+#pragma unroll
+  for (int j = 0; j < 16; ++j) {
+    const int c = C0 + j;
+    if (c < TT * P) {
+      const int tl = c / P, u = c % P;
+      const float z = tanhf(e[tl] + pr[u]);
+      const float h = w[j] * fmaf(-z, z, 1.f);
+      es[tl] += h;
+      pa[u] += h;
+    }
+  }
+}
+
+// SPLIT = false: the bf16 kernel.  SPLIT = true (precision bf16x3), per tile:
+//   P1  logits = z_hi W_hi + z_lo W_hi + z_hi W_lo (as the bf16x3 forward; fp32 rows read from global memory)
+//   P2  G in fp32 -> G_hi = bf16(G) into the shared G tile, G_lo = bf16(G - G_hi) straight to its global spill (gt_lo)
+//   P3  pass 1: dZ^T = W_hi^T G_hi^T + W_lo^T G_hi^T (ring: [MB][KBG][hi, lo] blocks of wt_t); then warp 0 reloads G_lo
+//       from the spill (L2) into the G tile and pass 2 adds W_hi^T G_lo^T, committing the d blocks to P4 one by one
+//   P4  dH = dZ (1 - z^2) with z = tanh(e + p) in fp32 from the fp32 rows (global memory)
+//   d_bias = column sums of G_hi plus column sums of G_lo (after the reload)
+// Shared memory: the bf16 layout without the two slab regions (P1 ring / P4 slab).
+template <int P, int TT, bool SPLIT>
+__device__ __forceinline__ void joint_bwd3_body(const CUtensorMap& tmap_e, const CUtensorMap& tmap_p, const BwdParams& p) {
   extern __shared__ uint8_t smem_raw[];
   Bwd3Smem L;
-  carve_bwd3(L, smem_raw, p.NH, p.Vp, p.D);
+  carve_bwd3<SPLIT>(L, smem_raw, p.NH, p.Vp, p.D);
   const int tid = threadIdx.x, warp = uniform_warp_idx(), lane = tid & 31;
   const int KB = p.D / BK;                 // k-blocks of the logits GEMM
   const int KBG = (p.Vp + 63) / 64;        // k-blocks (over v) of the dZ GEMM
@@ -206,8 +244,10 @@ joint_bwd3_kernel(const __grid_constant__ CUtensorMap tmap_e, const __grid_const
 
   if (warp == 0 && lane == 0) {
     g_tc_error_host = p.err_host;
-    tma_prefetch_desc(&tmap_e);
-    tma_prefetch_desc(&tmap_p);
+    if (!SPLIT) {                    // the split form gets placeholder tensor maps
+      tma_prefetch_desc(&tmap_e);
+      tma_prefetch_desc(&tmap_p);
+    }
     for (int i = 0; i < B_A_STAGES; ++i) { mbar_init(L.a_full(i), 8); mbar_init(L.a_empty(i), 1); }
     for (int i = 0; i < B_S_STAGES; ++i) { mbar_init(L.s_full(i), 1); mbar_init(L.s_empty(i), 8); }
     for (int i = 0; i < B_R1_MAX; ++i) { mbar_init(L.r1_full(i), 1); mbar_init(L.r1_empty(i), 1); }
@@ -218,6 +258,7 @@ joint_bwd3_kernel(const __grid_constant__ CUtensorMap tmap_e, const __grid_const
     mbar_init(L.tmem_empty(), 8);
     mbar_init(L.gs_done(), 1);
     mbar_init(L.p4_full(), 1);
+    if (SPLIT) { mbar_init(L.p3a_done(), 1); mbar_init(L.gs_hi_done(), 1); mbar_init(L.glo_full(), 1); }
     fence_barrier_init();
   }
   if (warp == 2) tmem_alloc(smem_u32(L.tmem_ptr), TMEM_COLS);
@@ -236,7 +277,7 @@ joint_bwd3_kernel(const __grid_constant__ CUtensorMap tmap_e, const __grid_const
     for (int tile = tile_begin; tile < tile_end; ++tile) {
       if (lane == 0) TC_PROF(0, 1);
       // ring + G region are dead here: the previous tile's last dZ block and its G spill / column sums were observed below
-      for (int i = 0; i < 2 * KB; ++i) {
+      for (int i = 0; i < (SPLIT ? 4 : 2) * KB; ++i) {
         mbar_wait(L.r1_empty(r1.stage), r1.phase ^ 1u, 11);
         if (elect_one()) {
           mbar_arrive_expect_tx(L.r1_full(r1.stage), r1_bytes);
@@ -259,7 +300,7 @@ joint_bwd3_kernel(const __grid_constant__ CUtensorMap tmap_e, const __grid_const
         if (CTCVR_EXP & 1) return;
         bulk_store(gdst + ((size_t)(j & 1) * KBG + (j >> 1)) * 4096, L.g_kblock(j >> 1) + (uint32_t)(j & 1) * 8192u, 8192u);
       };
-      for (int i = 0; i < MB * KBG; ++i) {
+      for (int i = 0; i < (SPLIT ? 2 : 1) * MB * KBG; ++i) {
         mbar_wait(L.r3_empty(r3.stage), r3.phase ^ 1u, 13);
         if (elect_one()) {
           mbar_arrive_expect_tx(L.r3_full(r3.stage), 16384u);
@@ -276,6 +317,30 @@ joint_bwd3_kernel(const __grid_constant__ CUtensorMap tmap_e, const __grid_const
         bulk_commit();
       }
       __syncwarp();
+      if constexpr (SPLIT) {
+        // G_lo into the G tile once the pass-1 MMAs, the G_hi column sums and the G_hi spill are done with it.  The
+        // P2 threads wrote G_lo with generic stores, fenced for the async proxy before their g_full arrival (seen above)
+        const __nv_bfloat16* gsrc = p.gt_lo + ((size_t)p.tiles[tile].w * 2) * (size_t)KBG * 4096;
+        mbar_wait(L.p3a_done(), ph, 60);
+        mbar_wait(L.gs_hi_done(), ph, 61);
+        if (elect_one()) {
+          bulk_wait_read<0>();
+          mbar_arrive_expect_tx(L.glo_full(), (uint32_t)KBG * 16384u);
+          for (int j = 0; j < 2 * KBG; ++j)
+            bulk_load(L.g_kblock(j >> 1) + (uint32_t)(j & 1) * 8192u, gsrc + ((size_t)(j & 1) * KBG + (j >> 1)) * 4096, 8192u,
+                      L.glo_full());
+        }
+        __syncwarp();
+        for (int i = 0; i < MB * KBG; ++i) {          // pass 2: the W_hi^T blocks again
+          mbar_wait(L.r3_empty(r3.stage), r3.phase ^ 1u, 62);
+          if (elect_one()) {
+            mbar_arrive_expect_tx(L.r3_full(r3.stage), 16384u);
+            bulk_load(L.r3_stage(r3.stage), p.wt_t + (size_t)(2 * i) * 8192, 16384u, L.r3_full(r3.stage));
+          }
+          __syncwarp();
+          r3.advance(B_R3_STAGES);
+        }
+      }
       if (lane == 0) TC_PROF(0, 4);
       mbar_wait(L.dz_full(MB - 1), ph, 14);       // every P3 MMA has completed: G tile and the W^T view are dead
       mbar_wait(L.gs_done(), ph, 16);             // ... the d_bias column sums have read G
@@ -284,7 +349,7 @@ joint_bwd3_kernel(const __grid_constant__ CUtensorMap tmap_e, const __grid_const
       if (lane == 0) TC_PROF(0, 5);
       ph ^= 1u;
     }
-  } else if (warp == 3) {
+  } else if (warp == 3 && !SPLIT) {
     // ------------------------------------------------------------------ TMA: enc / pred slabs (P1 ring + the P4 slab)
     Pipe sp;
     uint32_t ph = 0;
@@ -336,6 +401,36 @@ joint_bwd3_kernel(const __grid_constant__ CUtensorMap tmap_e, const __grid_const
       mbar_wait(L.tmem_empty(), ph ^ 1u, 20);
       if (lane == 0) TC_PROF(1, 2);
       tc_fence_after();
+      if constexpr (SPLIT) {
+        for (int kb = 0; kb < KB; ++kb) {
+          Pipe al = ap;                                // z_lo stage follows the z_hi stage
+          al.advance(B_A_STAGES);
+          mbar_wait(L.a_full(ap.stage), ap.phase, 21);
+          mbar_wait(L.a_full(al.stage), al.phase, 21);
+          for (int j = 0; j < 4; ++j) {                // W_hi half 0, 1, W_lo half 0, 1
+            mbar_wait(L.r1_full(r1.stage), r1.phase, 22);
+            tc_fence_after();
+            if (elect_one()) {
+              const uint32_t a = tmem_base + B_ACC_COLS + ap.stage * 32;
+              const uint32_t a2 = tmem_base + B_ACC_COLS + al.stage * 32;
+              const uint64_t bd = r1_desc0 + (uint64_t)(r1.stage * r1_step);
+              const uint32_t d = tmem_base + (j & 1) * p.NH;
+#pragma unroll
+              for (int k4 = 0; k4 < 4; ++k4) umma_bf16_ts(d, a + 8 * k4, bd + 2 * k4, idesc1, (kb || j >= 2 || k4) ? 1u : 0u);
+              if (j < 2) {
+#pragma unroll
+                for (int k4 = 0; k4 < 4; ++k4) umma_bf16_ts(d, a2 + 8 * k4, bd + 2 * k4, idesc1, 1u);
+              }
+              umma_commit(L.r1_empty(r1.stage));
+              if (j == 3) { umma_commit(L.a_empty(ap.stage)); umma_commit(L.a_empty(al.stage)); }
+            }
+            __syncwarp();
+            r1.advance(R1);
+          }
+          ap.advance(B_A_STAGES);
+          ap.advance(B_A_STAGES);
+        }
+      } else
       for (int kb = 0; kb < KB; ++kb) {
         mbar_wait(L.a_full(ap.stage), ap.phase, 21);
         if (lane == 0) TC_PROF(1, 50 + kb);
@@ -366,6 +461,30 @@ joint_bwd3_kernel(const __grid_constant__ CUtensorMap tmap_e, const __grid_const
       mbar_wait(L.g_full(), ph, 23);
       if (lane == 0) TC_PROF(1, 4);
       tc_fence_after();
+      if constexpr (SPLIT) {
+        // pass 1: W_hi^T G_hi^T + W_lo^T G_hi^T into every d block
+        for (int mb = 0; mb < MB; ++mb)
+          for (int kb = 0; kb < KBG; ++kb)
+            for (int hl = 0; hl < 2; ++hl) {
+              mbar_wait(L.r3_full(r3.stage), r3.phase, 24);
+              tc_fence_after();
+              if (elect_one()) {
+                const uint64_t ad = r3_desc0 + (uint64_t)(r3.stage * 1024);
+                const uint64_t bd = g_desc0 + (uint64_t)(kb * 1024);
+                const uint32_t d = tmem_base + mb * 128;
+                const int nks = kb == KBG - 1 ? last_nks : 4;
+                for (int k4 = 0; k4 < nks; ++k4) umma_bf16(d, ad + 2 * k4, bd + 2 * k4, idesc2, (kb || hl || k4) ? 1u : 0u);
+                umma_commit(L.r3_empty(r3.stage));
+              }
+              __syncwarp();
+              r3.advance(B_R3_STAGES);
+            }
+        if (elect_one()) umma_commit(L.p3a_done());
+        __syncwarp();
+        // pass 2: + W_hi^T G_lo^T once G_lo is in the tile; d block mb goes to P4 as soon as it is complete
+        mbar_wait(L.glo_full(), ph, 63);
+        tc_fence_after();
+      }
       for (int mb = 0; mb < MB; ++mb) {
         for (int kb = 0; kb < KBG; ++kb) {
           mbar_wait(L.r3_full(r3.stage), r3.phase, 24);
@@ -375,7 +494,7 @@ joint_bwd3_kernel(const __grid_constant__ CUtensorMap tmap_e, const __grid_const
             const uint64_t bd = g_desc0 + (uint64_t)(kb * 1024);
             const uint32_t d = tmem_base + mb * 128;
             const int nks = kb == KBG - 1 ? last_nks : 4;
-            if (nks > 0) umma_bf16(d, ad, bd, idesc2, kb ? 1u : 0u);
+            if (nks > 0) umma_bf16(d, ad, bd, idesc2, (kb || SPLIT) ? 1u : 0u);
             if (nks > 1) umma_bf16(d, ad + 2, bd + 2, idesc2, 1u);
             if (nks > 2) umma_bf16(d, ad + 4, bd + 4, idesc2, 1u);
             if (nks > 3) umma_bf16(d, ad + 6, bd + 6, idesc2, 1u);
@@ -441,6 +560,38 @@ joint_bwd3_kernel(const __grid_constant__ CUtensorMap tmap_e, const __grid_const
         // the A columns overlay the dZ^T accumulator of the previous tile: wait until its readers (P4) are done
         mbar_wait(L.tmem_empty(), ph ^ 1u, 40);
         if (tid == 128) TC_PROF(3, 1);
+        if constexpr (SPLIT) {
+          // slot = 32 k of row r: 16 z_hi columns in A stage 2 kbc, 16 z_lo columns in A stage 2 kbc + 1
+          const float4* er = reinterpret_cast<const float4*>(p.enc + ((size_t)g.b * p.T + min(g.t0 + p_tloc, p.T - 1)) * p.D);
+          const float4* pr4 = reinterpret_cast<const float4*>(p.pred + ((size_t)g.b * p.U1 + min(g.ubase + p_ul, p.U1 - 1)) * p.D);
+          for (int s = wg; s < 2 * KB; s += 3) {
+            const int kb = s >> 1, kh = s & 1;
+            const uint32_t n_hi = 2u * (kb_base + (uint32_t)kb), n_lo = n_hi + 1u;
+            const uint32_t s_hi = n_hi % B_A_STAGES, ph_hi = (n_hi / B_A_STAGES) & 1u;
+            const uint32_t s_lo = n_lo % B_A_STAGES, ph_lo = (n_lo / B_A_STAGES) & 1u;
+#pragma unroll
+            for (int c = 0; c < 2; ++c) {
+              const float4* e4 = er + kb * 16 + kh * 8 + c * 4;
+              const float4* p4 = pr4 + kb * 16 + kh * 8 + c * 4;
+              const float4 e0 = __ldg(e4), e1 = __ldg(e4 + 1), e2 = __ldg(e4 + 2), e3 = __ldg(e4 + 3);
+              const float4 q0 = __ldg(p4), q1 = __ldg(p4 + 1), q2 = __ldg(p4 + 2), q3 = __ldg(p4 + 3);
+              uint32_t hi[8], lo[8];
+              tanh_split8(e0, e1, q0, q1, hi, lo);
+              tanh_split8(e2, e3, q2, q3, hi + 4, lo + 4);
+              if (c == 0) {
+                mbar_wait(L.a_empty(s_hi), ph_hi ^ 1u, 42);
+                mbar_wait(L.a_empty(s_lo), ph_lo ^ 1u, 42);
+                tc_fence_after();
+              }
+              tmem_st8(tq + (uint32_t)(B_ACC_COLS + s_hi * 32 + kh * 16 + c * 8), hi);
+              tmem_st8(tq + (uint32_t)(B_ACC_COLS + s_lo * 32 + kh * 16 + c * 8), lo);
+            }
+            tmem_st_wait();
+            tc_fence_before();
+            warp_arrive(L.a_full(s_hi));
+            warp_arrive(L.a_full(s_lo));
+          }
+        } else
         for (int s = wg; s < 2 * KB; s += 3) {
           const int kb = s >> 1, kh = s & 1;
           const uint32_t kbc = kb_base + (uint32_t)kb;
@@ -523,7 +674,28 @@ joint_bwd3_kernel(const __grid_constant__ CUtensorMap tmap_e, const __grid_const
         }
         if (pi + 1 < npieces) tmem_ld16(tq + piece_col(pi + 1), v);
         uint32_t pk[8];
-        if (fast) {
+        uint32_t pl[8];                               // bf16x3: G_lo pairs
+        if constexpr (SPLIT) {
+#pragma unroll
+          for (int j = 0; j < 16; j += 2) {
+            float gg[2];
+#pragma unroll
+            for (int e = 0; e < 2; ++e) {
+              float gv;
+              if (fast) {
+                gv = ex2_fast(y[j + e] + kr);
+              } else {
+                gv = ex2_fast(y[j + e] + k_all * LOG2E);
+                if (p.clamp > 0.f) gv = fminf(gv, p.clamp);
+                gv = valid ? gv * scale : 0.f;
+              }
+              gg[e] = gv;
+            }
+            const __nv_bfloat162 h = __floats2bfloat162_rn(gg[0], gg[1]);
+            pk[j >> 1] = *reinterpret_cast<const uint32_t*>(&h);
+            pl[j >> 1] = pack_bf16(gg[0] - __low2float(h), gg[1] - __high2float(h));
+          }
+        } else if (fast) {
 #pragma unroll
           for (int j = 0; j < 16; j += 2) pk[j >> 1] = pack_bf16(ex2_fast(y[j] + kr), ex2_fast(y[j + 1] + kr));
         } else {
@@ -546,6 +718,11 @@ joint_bwd3_kernel(const __grid_constant__ CUtensorMap tmap_e, const __grid_const
 #pragma unroll
         for (int i = 0; i < 2; ++i)
           sts128(gb + (((ch0 + i) ^ (r & 7)) << 4), pk[4 * i], pk[4 * i + 1], pk[4 * i + 2], pk[4 * i + 3]);
+        if constexpr (SPLIT) {                        // G_lo: the same bytes the G tile's bulk store would write
+          uint4* gl = reinterpret_cast<uint4*>(p.gt_lo + (((size_t)ti.w * 2 + (r >> 6)) * KBG + (c0 >> 6)) * 4096 + (r & 63) * 64);
+#pragma unroll
+          for (int i = 0; i < 2; ++i) gl[(ch0 + i) ^ (r & 7)] = make_uint4(pl[4 * i], pl[4 * i + 1], pl[4 * i + 2], pl[4 * i + 3]);
+        }
       }
       // exact (fp32, single rounding) blank and label entries of row r, from the forward's log-probs: the warp group that
       // wrote the 16-column piece of the column patches it (program order within the thread - no barrier needed)
@@ -557,14 +734,19 @@ joint_bwd3_kernel(const __grid_constant__ CUtensorMap tmap_e, const __grid_const
           return gv * scale;
         };
         auto put = [&](int col, float val) {
-          const unsigned short h = __bfloat16_as_ushort(__float2bfloat16(val));
+          const __nv_bfloat16 hb = __float2bfloat16(val);
+          const unsigned short h = __bfloat16_as_ushort(hb);
           const uint32_t a = L.g_kblock(col >> 6) + r * 128 + ((((col & 63) >> 3) ^ (r & 7)) << 4) + (col & 7) * 2;
           asm volatile("st.shared.u16 [%0], %1;" ::"r"(a), "h"(h) : "memory");
+          if constexpr (SPLIT)                        // after this thread's own 16-byte store of the same chunk
+            p.gt_lo[(((size_t)ti.w * 2 + (r >> 6)) * KBG + (col >> 6)) * 4096 + (r & 63) * 64 +
+                    ((((col & 63) >> 3) ^ (r & 7)) << 3) + (col & 7)] = __float2bfloat16(val - __bfloat162float(hb));
         };
         if (((p.blank >> 4) % 3) == wg) put(p.blank, entry(lpb, bnext, (lab == p.blank) ? bl1 : kNegInf));
         if (lab >= 0 && lab != p.blank && ((lab >> 4) % 3) == wg) put(lab, entry(lpl, bl1, kNegInf));
       }
       fence_proxy_async();
+      if (SPLIT) asm volatile("fence.proxy.async.global;" ::: "memory");   // G_lo is read back by a bulk copy
       tc_fence_before();
       warp_arrive(L.g_full());
       if (tid == 128) TC_PROF(2, 3);
@@ -573,6 +755,7 @@ joint_bwd3_kernel(const __grid_constant__ CUtensorMap tmap_e, const __grid_const
         // ---------------- P3 side work (warps 12-15): spill the G tile, d_bias = its column sums
         mbar_wait(L.g_full(), ph, 31);
         const int nchunk = p.Vp >> 3;
+        auto colsum = [&]() {
         for (int it = r; it < ((CTCVR_EXP & 2) ? 0 : 4 * nchunk); it += 128) {
           const int rg = it / nchunk, c = it - rg * nchunk;
           const uint32_t gb = L.g_kblock(c >> 3) + (uint32_t)(rg * 32) * 128u;
@@ -596,20 +779,33 @@ joint_bwd3_kernel(const __grid_constant__ CUtensorMap tmap_e, const __grid_const
           if (col < p.Vp) db[i] += (L.dbp[col] + L.dbp[p.Vp + col]) + (L.dbp[2 * p.Vp + col] + L.dbp[3 * p.Vp + col]);
         }
         named_barrier_sync(2, 128);                   // partials consumed (the next tile overwrites them)
+        };
+        colsum();
+        if constexpr (SPLIT) {                        // + the column sums of G_lo once it is in the tile
+          if (r == 0) mbar_arrive(L.gs_hi_done());
+          mbar_wait(L.glo_full(), ph, 64);
+          colsum();
+        }
         if (r == 0) mbar_arrive(L.gs_done());
       } else {
         // ---------------- P4 (warps 4-11), overlapped with P3: dH = dZ * (1 - z^2); reductions.  Warp group wg owns
         // d blocks wg, wg+2.  TMEM column c of a d block = tile row c = (frame slot c / P, label slot c % P): everything
         // is static after unrolling, so any (P, TT) works with aligned 32-column loads.
-        mbar_wait(L.p4_full(), ph, 34);
+        if (!SPLIT) mbar_wait(L.p4_full(), ph, 34);
 #pragma unroll
         for (int mbl = 0; mbl < 2; ++mbl) {
           const int mb = wg + 2 * mbl;
           if (mb < MB) {
             const int d = mb * 128 + r;
             // this thread's joint dim of the tile's enc / pred rows: slab stage d/64, 16-byte chunk ((d&63)>>3) ^ (row&7)
-            uint32_t e[TT], pr[P];
-            {
+            // (bf16x3: the fp32 values, coalesced loads from global memory over the lanes = consecutive d)
+            std::conditional_t<SPLIT, float, uint32_t> e[TT], pr[P];
+            if constexpr (SPLIT) {
+#pragma unroll
+              for (int i = 0; i < P; ++i) pr[i] = __ldg(p.pred + ((size_t)g.b * p.U1 + min(g.ubase + i, p.U1 - 1)) * p.D + d);
+#pragma unroll
+              for (int i = 0; i < TT; ++i) e[i] = __ldg(p.enc + ((size_t)g.b * p.T + min(g.t0 + i, p.T - 1)) * p.D + d);
+            } else {
               const uint32_t st = L.p4_stage(d >> 6) + (uint32_t)(d & 7) * 2u;
               const uint32_t chn = (uint32_t)((d & 63) >> 3);
 #pragma unroll
@@ -681,6 +877,20 @@ joint_bwd3_kernel(const __grid_constant__ CUtensorMap tmap_e, const __grid_const
   tc_fence_before();
   __syncthreads();
   if (warp == 2) tmem_dealloc(tmem_base, TMEM_COLS);
+}
+
+template <int P, int TT>
+__global__ void __launch_bounds__(NTHREADS, 1)
+joint_bwd3_kernel(const __grid_constant__ CUtensorMap tmap_e, const __grid_constant__ CUtensorMap tmap_p,
+                  const BwdParams p) {
+  joint_bwd3_body<P, TT, false>(tmap_e, tmap_p, p);
+}
+// precision bf16x3 (the tensor maps are unused)
+template <int P, int TT>
+__global__ void __launch_bounds__(NTHREADS, 1)
+joint_bwd3_x3_kernel(const __grid_constant__ CUtensorMap tmap_e, const __grid_constant__ CUtensorMap tmap_p,
+                     const BwdParams p) {
+  joint_bwd3_body<P, TT, true>(tmap_e, tmap_p, p);
 }
 
 }  // namespace tc

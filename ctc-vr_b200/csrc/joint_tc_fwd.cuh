@@ -52,6 +52,8 @@ struct FwdParams {
   float* lp_label;
   long long* prof;
   unsigned int* err_host;   // mapped host word for bounded-wait time-outs (tc_common.cuh)
+  const float* enc;         // bf16x3 only: the fp32 activations [B,T,D] / [B,U1,D], read in place
+  const float* pred;
 };
 
 struct FwdSmem {
@@ -97,9 +99,27 @@ __device__ __forceinline__ void carve_fwd2(FwdSmem& L, uint8_t* raw, int NH, int
 }
 
 
-__global__ void __launch_bounds__(F_THREADS, 1)
-joint_fwd2_kernel(const __grid_constant__ CUtensorMap tmap_e, const __grid_constant__ CUtensorMap tmap_p,
-                  const FwdParams p) {
+// z = tanh(e + p) in fp32 (tanhf: accurate, the build does not use fast-math) for 8 consecutive k, split into
+// hi = bf16_rn(z) and lo = bf16_rn(z - hi) as packed pairs (low half = even k, the TMEM operand layout)
+__device__ __forceinline__ void tanh_split8(const float4& e0, const float4& e1, const float4& p0, const float4& p1,
+                                            uint32_t* hi, uint32_t* lo) {
+  const float z[8] = {tanhf(e0.x + p0.x), tanhf(e0.y + p0.y), tanhf(e0.z + p0.z), tanhf(e0.w + p0.w),
+                      tanhf(e1.x + p1.x), tanhf(e1.y + p1.y), tanhf(e1.z + p1.z), tanhf(e1.w + p1.w)};
+#pragma unroll
+  for (int j = 0; j < 4; ++j) {
+    const __nv_bfloat162 h = __floats2bfloat162_rn(z[2 * j], z[2 * j + 1]);
+    hi[j] = *reinterpret_cast<const uint32_t*>(&h);
+    lo[j] = pack_bf16(z[2 * j] - __low2float(h), z[2 * j + 1] - __high2float(h));
+  }
+}
+
+// SPLIT = false: the bf16 kernel.  SPLIT = true (precision bf16x3): every operand x is hi + lo (bf16 each) and the
+// logits accumulate z_hi W_hi + z_lo W_hi + z_hi W_lo, three MMA passes per k-block into the same accumulators.
+//   W ring   : per k-block four stages (W_hi half 0, 1, W_lo half 0, 1) from w_t = [KB][hi, lo][2][NH][64]
+//   A stages : per k-block two TMEM stages (z_hi, z_lo of its 64 k): the same 3 x 32 columns as bf16
+//   producers: read the fp32 enc / pred rows straight from global memory (L2-resident), no slab ring (warp 3 idles)
+template <bool SPLIT>
+__device__ __forceinline__ void joint_fwd2_body(const CUtensorMap& tmap_e, const CUtensorMap& tmap_p, const FwdParams& p) {
   extern __shared__ uint8_t smem_raw[];
   FwdSmem L;
   carve_fwd2(L, smem_raw, p.NH, p.Vp, p.w_stages);
@@ -110,8 +130,10 @@ joint_fwd2_kernel(const __grid_constant__ CUtensorMap tmap_e, const __grid_const
 
   if (warp == 0 && lane == 0) {
     g_tc_error_host = p.err_host;
-    tma_prefetch_desc(&tmap_e);
-    tma_prefetch_desc(&tmap_p);
+    if (!SPLIT) {                    // the split form gets placeholder tensor maps
+      tma_prefetch_desc(&tmap_e);
+      tma_prefetch_desc(&tmap_p);
+    }
     for (int i = 0; i < F_A_STAGES; ++i) { mbar_init(L.a_full(i), PROD_THREADS / 32); mbar_init(L.a_empty(i), 1); }
     for (int i = 0; i < F_S_STAGES; ++i) { mbar_init(L.s_full(i), 1); mbar_init(L.s_empty(i), PROD_THREADS / 32); }
     for (int i = 0; i < F_MAX_W_STAGES; ++i) { mbar_init(L.w_full(i), 1); mbar_init(L.w_empty(i), 1); }
@@ -131,7 +153,7 @@ joint_fwd2_kernel(const __grid_constant__ CUtensorMap tmap_e, const __grid_const
     Pipe wp;
     const uint32_t w_bytes = (uint32_t)p.NH * 128u;
     for (int tile = blockIdx.x; tile < ntiles; tile += gridDim.x)
-      for (int i = 0; i < 2 * KB; ++i) {
+      for (int i = 0; i < (SPLIT ? 4 : 2) * KB; ++i) {
         mbar_wait(L.w_empty(wp.stage), wp.phase ^ 1u, 1);
         if (elect_one()) {
           mbar_arrive_expect_tx(L.w_full(wp.stage), w_bytes);
@@ -140,7 +162,7 @@ joint_fwd2_kernel(const __grid_constant__ CUtensorMap tmap_e, const __grid_const
         __syncwarp();
         wp.advance(WS);
       }
-  } else if (warp == 3) {
+  } else if (warp == 3 && !SPLIT) {
     // ------------------------------------------------------------------ TMA: enc / pred slabs
     Pipe sp;
     for (int tile = blockIdx.x; tile < ntiles; tile += gridDim.x) {
@@ -174,6 +196,37 @@ joint_fwd2_kernel(const __grid_constant__ CUtensorMap tmap_e, const __grid_const
       mbar_wait(L.tmem_empty(), tphase ^ 1u, 3);
       if (lane == 0) TC_PROF(1, 101);
       tc_fence_after();
+      if constexpr (SPLIT) {
+        for (int kb = 0; kb < KB; ++kb) {
+          Pipe al = ap;                                  // z_lo stage follows the z_hi stage
+          al.advance(F_A_STAGES);
+          mbar_wait(L.a_full(ap.stage), ap.phase, 4);
+          mbar_wait(L.a_full(al.stage), al.phase, 4);
+          for (int j = 0; j < 4; ++j) {                  // W_hi half 0, 1, W_lo half 0, 1
+            const int h = j & 1;
+            mbar_wait(L.w_full(wp.stage), wp.phase, 5);
+            tc_fence_after();
+            if (elect_one()) {
+              const uint64_t bd = w_desc0 + (uint64_t)(wp.stage * w_step);
+              const uint32_t d = tmem_base + h * p.NH;
+              const uint32_t a = tmem_base + F_ACC_COLS + ap.stage * 32;
+              const uint32_t a2 = tmem_base + F_ACC_COLS + al.stage * 32;
+#pragma unroll
+              for (int k4 = 0; k4 < 4; ++k4) umma_bf16_ts(d, a + 8 * k4, bd + 2 * k4, idesc, (kb || j >= 2 || k4) ? 1u : 0u);
+              if (j < 2) {
+#pragma unroll
+                for (int k4 = 0; k4 < 4; ++k4) umma_bf16_ts(d, a2 + 8 * k4, bd + 2 * k4, idesc, 1u);
+              }
+              umma_commit(L.w_empty(wp.stage));
+              if (j == 3) { umma_commit(L.a_empty(ap.stage)); umma_commit(L.a_empty(al.stage)); }
+            }
+            __syncwarp();
+            wp.advance(WS);
+          }
+          ap.advance(F_A_STAGES);
+          ap.advance(F_A_STAGES);
+        }
+      } else
       for (int kb = 0; kb < KB; ++kb) {
         mbar_wait(L.a_full(ap.stage), ap.phase, 4);
         for (int h = 0; h < 2; ++h) {
@@ -291,6 +344,49 @@ joint_fwd2_kernel(const __grid_constant__ CUtensorMap tmap_e, const __grid_const
       named_barrier_sync(3, F_EPI_WARPS * 32);             // partials consumed before the next tile overwrites them
       tphase ^= 1u;
     }
+  } else if (warp >= F_PROD_WARP0 && SPLIT) {
+    // ------------------------------------------------------------------ bf16x3 A producers: fp32 rows from global
+    // thread = tile row 32q + lane, k-half kh: 32 k per k-block -> 16 hi columns (stage a) + 16 lo columns (stage a + 1)
+    const int q = warp & 3, kh = (warp - F_PROD_WARP0) >> 2;
+    const uint32_t tq = tmem_base + ((uint32_t)(q * 32) << 16);
+    Pipe ap;
+    for (int tile = blockIdx.x; tile < ntiles; tile += gridDim.x) {
+      int4 ti = p.tiles[tile];
+      pin(ti.x); pin(ti.y); pin(ti.z); pin(ti.w);
+      const int lognu = ti.w >> 1;
+      const int u = ti.y + (q & (ti.w - 1));
+      const int t = min(ti.z + ((q >> lognu) << 5) + lane, p.T - 1);     // rows past the utterance are discarded
+      const float4* er = reinterpret_cast<const float4*>(p.enc + ((size_t)ti.x * p.T + t) * p.D + kh * 32);
+      const float4* pr = reinterpret_cast<const float4*>(p.pred + ((size_t)ti.x * p.U1 + u) * p.D + kh * 32);
+      for (int kb = 0; kb < KB; ++kb) {
+        Pipe al = ap;
+        al.advance(F_A_STAGES);
+        const uint32_t c_hi = (uint32_t)(F_ACC_COLS + ap.stage * 32 + kh * 16), c_lo = (uint32_t)(F_ACC_COLS + al.stage * 32 + kh * 16);
+#pragma unroll
+        for (int c = 0; c < 2; ++c) {                   // 16 k per round: 8 hi + 8 lo columns
+          const float4* e4 = er + kb * 16 + c * 4;
+          const float4* p4 = pr + kb * 16 + c * 4;
+          const float4 e0 = __ldg(e4), e1 = __ldg(e4 + 1), e2 = __ldg(e4 + 2), e3 = __ldg(e4 + 3);
+          const float4 p0 = __ldg(p4), p1 = __ldg(p4 + 1), p2 = __ldg(p4 + 2), p3 = __ldg(p4 + 3);
+          uint32_t hi[8], lo[8];
+          tanh_split8(e0, e1, p0, p1, hi, lo);
+          tanh_split8(e2, e3, p2, p3, hi + 4, lo + 4);
+          if (c == 0) {
+            mbar_wait(L.a_empty(ap.stage), ap.phase ^ 1u, 8);
+            mbar_wait(L.a_empty(al.stage), al.phase ^ 1u, 8);
+            tc_fence_after();
+          }
+          tmem_st8(tq + c_hi + c * 8, hi);
+          tmem_st8(tq + c_lo + c * 8, lo);
+        }
+        tmem_st_wait();
+        tc_fence_before();
+        warp_arrive(L.a_full(ap.stage));
+        warp_arrive(L.a_full(al.stage));
+        ap.advance(F_A_STAGES);
+        ap.advance(F_A_STAGES);
+      }
+    }
   } else if (warp >= F_PROD_WARP0) {
     // ------------------------------------------------------------------ A producers (A operand lives in TMEM)
     // warp = (TMEM lane quarter q, k-half kh): thread = tile row 32q + lane, 32 of the 64 k of a k-block.
@@ -338,6 +434,18 @@ joint_fwd2_kernel(const __grid_constant__ CUtensorMap tmap_e, const __grid_const
   tc_fence_before();
   __syncthreads();
   if (warp == 2) tmem_dealloc(tmem_base, TMEM_COLS);
+}
+
+__global__ void __launch_bounds__(F_THREADS, 1)
+joint_fwd2_kernel(const __grid_constant__ CUtensorMap tmap_e, const __grid_constant__ CUtensorMap tmap_p,
+                  const FwdParams p) {
+  joint_fwd2_body<false>(tmap_e, tmap_p, p);
+}
+// precision bf16x3 (the tensor maps are unused: the producers read the fp32 rows directly)
+__global__ void __launch_bounds__(F_THREADS, 1)
+joint_fwd2_x3_kernel(const __grid_constant__ CUtensorMap tmap_e, const __grid_constant__ CUtensorMap tmap_p,
+                     const FwdParams p) {
+  joint_fwd2_body<true>(tmap_e, tmap_p, p);
 }
 
 // Tile table of the forward kernel: per utterance (W/4) groups of 4 label columns x 32-frame blocks, then a

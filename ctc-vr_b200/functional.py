@@ -18,8 +18,9 @@ import torch
 from . import _lib
 from ._lib import call, ptr, query, stream
 
-F32, BF16 = 0, 1
-_PREC = {"fp32": F32, "f32": F32, "bf16": BF16, F32: F32, BF16: BF16}
+F32, BF16, BF16X3 = 0, 1, 2
+_PREC = {"fp32": F32, "f32": F32, "bf16": BF16, "bf16x3": BF16X3, F32: F32, BF16: BF16, BF16X3: BF16X3}
+_PREC_NAME = {F32: "fp32", BF16: "bf16", BF16X3: "bf16x3"}
 
 
 def _f32c(t):
@@ -61,9 +62,9 @@ class _FusedJointRnnt(torch.autograd.Function):
             raise RuntimeError("fused_joint_rnnt_loss: blank must be within [0, vocab)")
         # Length / label VALUES are not read back (that would be a host sync in the training step): the kernels clamp
         # lengths to the tensor extents and treat a label outside [0, V) as blank, so bad values cannot fault the GPU.
-        if precision == BF16 and not bool(query("ctcvr_joint_tc_supported", U1, D, V)):
-            raise RuntimeError(f"fused_joint_rnnt_loss: precision='bf16' needs D % 128 == 0, D <= 512, V <= 416 and "
-                               f"U+1 <= 128 (got D={D}, V={V}, U+1={U1}); use precision='fp32' for this shape")
+        if precision in (BF16, BF16X3) and not bool(query("ctcvr_joint_tc_supported", U1, D, V)):
+            raise RuntimeError(f"fused_joint_rnnt_loss: precision='{_PREC_NAME[precision]}' needs D % 128 == 0, D <= 512, "
+                               f"V <= 416 and U+1 <= 128 (got D={D}, V={V}, U+1={U1}); use precision='fp32' for this shape")
         lse = torch.empty((B, T, U1), dtype=torch.float32, device=dev)
         lpb, lpl = torch.empty_like(lse), torch.empty_like(lse)
         alpha, beta = torch.empty_like(lse), torch.empty_like(lse)
@@ -116,7 +117,11 @@ def fused_joint_rnnt_loss(enc_proj, pred_proj, w_out, b_out, targets, logit_leng
 
     precision='fp32' (default) is the reference's arithmetic (loss and gradients within 1e-4 of torchaudio's);
     precision='bf16' is the explicit opt-in to the tcgen05 path (bf16 operands, fp32 accumulation, softmax and
-    lattice; loss within 2e-3, gradients within 3e-2 rel-L2) and raises on shapes outside its tiling."""
+    lattice; loss within 2e-3, gradients within 3e-2 rel-L2) and raises on shapes outside its tiling.
+    precision='bf16x3' runs the same tcgen05 tiling at fp32 accuracy: every fp32 GEMM operand is split into
+    hi = bf16(x) and lo = bf16(x - hi) and each product is hi*hi + hi*lo + lo*hi, with tanh, d cost / d logits and the
+    reductions in fp32.  Loss and gradients are within 1e-4 of the reference, like fp32; inputs are taken as fp32, and
+    the shape limits and the error on other shapes are those of 'bf16'."""
     costs = _FusedJointRnnt.apply(enc_proj, pred_proj, w_out, b_out, targets, logit_lengths, target_lengths,
                                   int(blank), float(clamp), _PREC[precision])
     return _reduce(costs, reduction)

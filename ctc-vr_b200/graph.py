@@ -24,7 +24,8 @@ class GraphedJointRnntStep:
     Construct it before (or after dropping every reference to) eager autograd graphs over the same parameters: a live
     graph pins their AccumulateGrad nodes to the stream it ran on, and the capture may not synchronise with that stream.
     `input_dtype=torch.bfloat16` keeps the captured input buffers in bf16 (the bf16 path rounds its inputs to bf16 in
-    the first kernel anyway): a host pipeline then stages half the bytes per step.
+    the first kernel anyway): a host pipeline then stages half the bytes per step.  `precision="bf16x3"` (tensor cores
+    at fp32 accuracy) needs fp32 inputs.
     `predictor=RNNPredictor(...)` puts the label side of Transducer._compute_rnnt_loss (transducer.py:168-172) into the
     step: `ys_in = [blank, targets]` is built in the captured region, the predictor (embedding, the LSTM sequence kernels
     of csrc/lstm_seq.cu, projection) produces `pred_out`, and its parameters get their gradients (and join the gradient
@@ -33,6 +34,8 @@ class GraphedJointRnntStep:
     def __init__(self, joint, B: int, T: int, U: int, blank: int, global_batch: Optional[int] = None,
                  precision: str = "fp32", clamp: float = -1.0, warmup: int = 3,
                  input_dtype: torch.dtype = torch.float32, grad_exchange=None, predictor=None):
+        if precision == "bf16x3" and input_dtype != torch.float32:
+            raise ValueError("precision='bf16x3' keeps fp32 accuracy end to end: input_dtype must be torch.float32")
         p0 = next(joint.parameters())
         dev = p0.device
         if dev.type != "cuda":

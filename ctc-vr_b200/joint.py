@@ -109,7 +109,8 @@ class TransducerJoint(nn.Module):
                         clamp: float = -1.0, reduction: str = "mean", precision: str = "fp32",
                         pre_project: bool = True):
         """joint + log-softmax + RNN-T lattice loss in one op (the seam of transducer.py:172-187).
-        precision='fp32' keeps the reference's arithmetic; 'bf16' opts into the tcgen05 tensor-core path."""
+        precision='fp32' keeps the reference's arithmetic; 'bf16' opts into the tcgen05 tensor-core path; 'bf16x3'
+        runs the tensor-core path at fp32 accuracy (the pre-projections then stay fp32, as with 'fp32')."""
         if not self.fusable:
             raise RuntimeError("rnnt_loss_fused: only joint_mode='add', activation='tanh', postjoin_linear=False")
         if precision in ("bf16", CF.BF16) and enc_out.is_cuda:

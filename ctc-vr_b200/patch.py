@@ -207,11 +207,12 @@ def _make_prefix_beam_search(seq_cls):
 # ------------------------------------------------------------------------------------------------ install
 def install(namespace=None, precision: Optional[str] = None) -> Dict[str, List[str]]:
     """Patch whatever of the reference is present in `namespace` (None: import it).  Returns what was patched.
-    `precision` ("fp32" | "bf16") becomes the class default of the patched `Transducer` (the fused loss reads
-    `self.precision`, fp32 when absent), so an unchanged train script opts into the tcgen05 path with
-    `install(precision="bf16")`; a model instance can still override it with its own `precision` attribute."""
-    if precision not in (None, "fp32", "bf16"):
-        raise ValueError("precision must be None, 'fp32' or 'bf16'")
+    `precision` ("fp32" | "bf16" | "bf16x3") becomes the class default of the patched `Transducer` (the fused loss
+    reads `self.precision`, fp32 when absent), so an unchanged train script opts into the tcgen05 path with
+    `install(precision="bf16")`, or into the tcgen05 path at fp32 accuracy with `install(precision="bf16x3")`; a model
+    instance can still override it with its own `precision` attribute."""
+    if precision not in (None, "fp32", "bf16", "bf16x3"):
+        raise ValueError("precision must be None, 'fp32', 'bf16' or 'bf16x3'")
     done: Dict[str, List[str]] = {}
 
     def note(mod, name):

@@ -19,6 +19,10 @@
  *   - precision: CTCVR_F32 = fp32 SIMT path (1e-4 parity path), CTCVR_BF16 = tcgen05 path
  *     (bf16 operands - enc_proj / pred_proj are rounded to bf16 too - fp32 accumulate / softmax /
  *     lattice).  enc_proj / pred_proj must be 16-byte aligned in the bf16 path.
+ *     CTCVR_BF16X3 = the tcgen05 path at fp32 accuracy: every fp32 operand x is split into
+ *     hi = bf16(x), lo = bf16(x - hi) and each product is hi*hi + hi*lo + lo*hi (three MMAs into one
+ *     fp32 accumulator); tanh, G = d cost / d logits and the reductions stay fp32.  Loss and gradients
+ *     within 1e-4 of the reference, like CTCVR_F32; same shape limits and alignment as CTCVR_BF16.
  */
 #ifndef CTCVR_H_
 #define CTCVR_H_
@@ -32,6 +36,7 @@ extern "C" {
 
 #define CTCVR_F32 0
 #define CTCVR_BF16 1
+#define CTCVR_BF16X3 2
 
 const char* ctcvr_last_error(void);
 int ctcvr_version(void);

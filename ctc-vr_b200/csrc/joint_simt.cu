@@ -62,7 +62,7 @@ __global__ void __launch_bounds__(JT_THREADS, 1) joint_tile_kernel(JointTileArgs
   const int lane = tid & 31, warp = tid >> 5;
   const int b = a.b0 + blockIdx.y;
   const int D = a.D, V = a.V, U1 = a.U1, T = a.T;
-  const int Tb = a.t_len ? min(a.t_len[b], T) : T;                    // lengths beyond the tensors cannot index outside them
+  const int Tb = a.t_len ? max(min(a.t_len[b], T), 0) : T;                    // lengths beyond the tensors cannot index outside them
   const int Ub = a.u_len ? max(min(a.u_len[b], U1 - 1), 0) : U1 - 1;
   const bool dense_enum = (MODE != MODE_STATS);
   const int width = dense_enum ? U1 : (Ub + 1);

@@ -62,8 +62,8 @@ template <int TILE>
 __device__ __forceinline__ RowMap tile_geometry(const int32_t* t_len, const int32_t* u_len, int T, int U1, int4 ti) {
   RowMap g;
   g.b = ti.x;
-  g.Tb = min(t_len[g.b], T);
-  g.Ub = min(u_len[g.b], U1 - 1);
+  g.Tb = max(min(t_len[g.b], T), 0);
+  g.Ub = max(min(u_len[g.b], U1 - 1), 0);
   g.W = g.Ub + 1;
   if (TILE == TILE_FLAT) {
     int ncell = g.Tb * g.W;
@@ -137,7 +137,7 @@ __global__ void reduce_denc_kernel(const float* __restrict__ part, const int32_t
     return;
   }
   const int b = bt / T, t = bt - b * T;
-  const int Tb = min(t_len[b], T), W = min(u_len[b], U1 - 1) + 1;
+  const int Tb = max(min(t_len[b], T), 0), W = max(min(u_len[b], U1 - 1), 0) + 1;
   const int S = (W + P - 1) / P;
   const size_t row = ((size_t)b * T + t) * D, step = (size_t)B * T * D;
   for (int d = threadIdx.x * 4; d < D; d += blockDim.x * 4) {
@@ -553,11 +553,11 @@ __device__ void build_tiles_block(int b, const int32_t* __restrict__ t_len, cons
   const int P = geom & 0xff, TT = (geom >> 8) & 0xff, even = (geom >> 16) & 1;
   auto ntb_of = [&](int Tb) { const int n = (Tb + TT - 1) / TT; return even ? ((n + 1) & ~1) : n; };
   auto count = [&](int i) {
-    const int Tb = min(t_len[i], T), W = min(u_len[i], U1 - 1) + 1;
+    const int Tb = max(min(t_len[i], T), 0), W = max(min(u_len[i], U1 - 1), 0) + 1;
     return Tb > 0 ? ((W + P - 1) / P) * ntb_of(Tb) : 0;
   };
   const int off = block_prefix(b, count);
-  const int Tb = min(t_len[b], T);
+  const int Tb = max(min(t_len[b], T), 0);
   const int n = count(b);
   const int NTB = ntb_of(Tb);
   for (int i = threadIdx.x; i < n; i += blockDim.x) {
@@ -566,7 +566,7 @@ __device__ void build_tiles_block(int b, const int32_t* __restrict__ t_len, cons
       tiles[off + i] = make_int4(b, s, tb, off + i);
       if (tile_rows) {
         // first enc / pred row of the tile and how many rows may be read past them (kernel 2 recomputes z from these)
-        const int W = min(u_len[b], U1 - 1) + 1, S = (W + P - 1) / P, us = (W + S - 1) / S;
+        const int W = max(min(u_len[b], U1 - 1), 0) + 1, S = (W + P - 1) / P, us = (W + S - 1) / S;
         const int t0 = tb * TT, ub = s * us;
         tile_rows[off + i] = make_int4(b * T + min(t0, T - 1), b * U1 + min(ub, U1 - 1), max(T - 1 - t0, 0), max(U1 - 1 - ub, 0));
       }
@@ -636,8 +636,8 @@ __device__ void prep_weights3_part(int i, const float* __restrict__ w, const flo
 __device__ void build_tiles_fwd_block(int b, const int32_t* __restrict__ t_len, const int32_t* __restrict__ u_len, int B,
                                       int T, int U1, int4* __restrict__ tiles, int* __restrict__ ntiles,
                                       int max_tiles, int pair) {
-  const int off = block_prefix(b, [&](int i) { return fwd_tiles_of(min(t_len[i], T), max(min(u_len[i], U1 - 1), 0) + 1, pair); });
-  const int Tb = min(t_len[b], T), W = max(min(u_len[b], U1 - 1), 0) + 1;
+  const int off = block_prefix(b, [&](int i) { return fwd_tiles_of(max(min(t_len[i], T), 0), max(min(u_len[i], U1 - 1), 0) + 1, pair); });
+  const int Tb = max(min(t_len[b], T), 0), W = max(min(u_len[b], U1 - 1), 0) + 1;
   const int n = fwd_tiles_of(Tb, W, pair);
   const int nb32 = (Tb + 31) >> 5, n4 = (W >> 2) * nb32;
   const int n2 = (W & 2) ? ((Tb + 63) >> 6) : 0;

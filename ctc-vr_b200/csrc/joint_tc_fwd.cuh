@@ -272,7 +272,7 @@ __device__ __forceinline__ void joint_fwd2_body(const CUtensorMap& tmap_e, const
       const int lognu = nu >> 1;                          // 4 -> 2, 2 -> 1, 1 -> 0
       const int u = ti.y + (q & (nu - 1));
       const int t = ti.z + ((q >> lognu) << 5) + lane;
-      int Tb = min(p.t_len[b], p.T), Ub = min(p.u_len[b], p.U1 - 1);
+      int Tb = max(min(p.t_len[b], p.T), 0), Ub = max(min(p.u_len[b], p.U1 - 1), 0);
       pin(Tb); pin(Ub);
       const bool valid = t < Tb;
       int lab = -1;

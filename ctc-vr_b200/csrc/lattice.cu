@@ -47,7 +47,7 @@ __global__ void __launch_bounds__(LAT2_THREADS) rnnt_lattice2_kernel(
     float* __restrict__ costs, int T, int U1, int pitch) {
   extern __shared__ float sm[];
   const int b = blockIdx.x;
-  const int Tb = min(t_len[b], T), Ub = min(u_len[b], U1 - 1);
+  const int Tb = max(min(t_len[b], T), 0), Ub = max(min(u_len[b], U1 - 1), 0);
   const size_t base = (size_t)b * T * U1;
   if (Tb <= 0) { if (threadIdx.x == 0) costs[b] = 0.f; return; }
   const int W = Ub + 1;
@@ -251,7 +251,7 @@ __global__ void __launch_bounds__(LAT3_THREADS) rnnt_lattice3_kernel(
     float* __restrict__ costs, int T, int U1, int pitch, int pad) {
   extern __shared__ float sm[];
   const int b = blockIdx.x;
-  const int Tb = min(t_len[b], T), Ub = min(u_len[b], U1 - 1);
+  const int Tb = max(min(t_len[b], T), 0), Ub = max(min(u_len[b], U1 - 1), 0);
   const size_t base = (size_t)b * T * U1;
   if (Tb <= 0) { if (threadIdx.x == 0) costs[b] = 0.f; return; }
   const int W = Ub + 1;
@@ -393,7 +393,7 @@ __global__ void rnnt_lattice_generic_kernel(const float* __restrict__ lp_blank, 
                                             float* __restrict__ alpha, float* __restrict__ beta,
                                             float* __restrict__ costs, int T, int U1) {
   const int b = blockIdx.x;
-  const int Tb = min(t_len[b], T), Ub = max(min(u_len[b], U1 - 1), 0);
+  const int Tb = max(min(t_len[b], T), 0), Ub = max(min(u_len[b], U1 - 1), 0);
   const size_t base = (size_t)b * T * U1;
   const float* lb = lp_blank + base;
   const float* ll = lp_label + base;

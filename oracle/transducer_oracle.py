@@ -92,6 +92,8 @@ def rnnt_lattice_restated(logits: torch.Tensor, targets: torch.Tensor,
     grads = torch.zeros((B, T, U1, V), dtype=dtype)
     for b in range(B):
         Tb, Ub = int(logit_lengths[b]), int(target_lengths[b])
+        if Tb == 0:                                                    # no frames: cost 0, zero gradient
+            continue
         a = alpha[b]
         a[0, 0] = 0.0
         for t in range(1, Tb):
@@ -132,17 +134,22 @@ def rnnt_lattice_restated(logits: torch.Tensor, targets: torch.Tensor,
 
 
 def fused_joint_rnnt_restated(enc_out, pred_out, w: Weights, targets, logit_lengths, target_lengths,
-                              blank: int, clamp: float = -1.0, dtype=torch.float64):
+                              blank: int, clamp: float = -1.0, dtype=torch.float64, grad_costs=None):
     """model/component/transducer.py:161-189 from predictor output to scalar loss
     (reduction='mean'), with gradients wrt enc_out / pred_out / the six joint tensors,
-    obtained by chaining the closed-form logits gradient through autograd of `joint_forward`."""
+    obtained by chaining the closed-form logits gradient through autograd of `joint_forward`.
+    `grad_costs` [B] is the cotangent of the per-utterance costs (None: 1/B each, the mean).  As in
+    torchaudio, the logits gradient is clamped first and then scaled by it."""
     ws = {k: v.detach().to(dtype).requires_grad_(True) for k, v in w.items()}
     e = enc_out.detach().to(dtype).requires_grad_(True)
     p = pred_out.detach().to(dtype).requires_grad_(True)
     logits = joint_forward(e, p, ws)
     r = rnnt_lattice_restated(logits, targets, logit_lengths, target_lengths, blank, clamp, dtype)
     B = logits.size(0)
-    logits.backward(r["grads"] / B)
+    if grad_costs is None:
+        logits.backward(r["grads"] / B)
+    else:
+        logits.backward(r["grads"] * torch.as_tensor(grad_costs).to(dtype).reshape(B, 1, 1, 1))
     out = dict(loss=r["costs"].mean(), costs=r["costs"], d_enc_out=e.grad, d_pred_out=p.grad)
     for k, v in ws.items():
         out["d_" + k] = v.grad

@@ -18,7 +18,7 @@ class DecoderWeights(ctypes.Structure):
     """Mirror of `ctcvr_decoder_weights` (include/ctcvr.h)."""
     _fields_ = [(n, c_void_p) for n in ("gate_tok", "w_hh_t", "w_ih_t", "b_gate", "proj_t", "proj_b",
                                         "pred_ffn_t", "pred_ffn_b", "out_t", "out_b")] + \
-               [(n, c_int) for n in ("V", "H", "L", "P", "D")]
+               [(n, c_int) for n in ("V", "H", "L", "P", "D", "activation")]   # activation: CTCVR_ACT_*, 0 = tanh
 
 
 _SIGS = {

@@ -133,12 +133,13 @@ __device__ __forceinline__ void warp_topk(F val, int V, int skip, int k, float* 
   }
 }
 
-// logits of all NB slots for frame vector e (enc_proj row): z = tanh(e + pproj), logit = out_t^T z + out_b
+// logits of all NB slots for frame vector e (enc_proj row): z = act(e + pproj), logit = out_t^T z + out_b
 template <int NB>
 __device__ void joint_logits_step(const ctcvr_decoder_weights& w, DecodeSmem<NB>& s, const float* __restrict__ e) {
+  const int act = w.activation >> 8;
   for (int i = threadIdx.x; i < w.D * NB; i += blockDim.x) {
     const int d = i / NB;
-    s.z[i] = tanhf(e[d] + s.pproj[i]);
+    s.z[i] = act_rt(act, e[d] + s.pproj[i]);
   }
   __syncthreads();
   gemv_t<NB>(w.out_t, w.V, w.D, s.z, [&](int j, int n) { return __ldg(w.out_b + j); },

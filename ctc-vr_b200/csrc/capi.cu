@@ -21,17 +21,17 @@ void set_error(const char* fmt, ...) {
 // implemented in the other translation units
 int joint_logits_f32(const float*, const float*, const float*, const float*, float*, int, int, int, int, int, cudaStream_t);
 int joint_fwd_f32(const float*, const float*, const float*, const float*, const int32_t*, const int32_t*,
-                  const int32_t*, float*, float*, float*, int, int, int, int, int, int, cudaStream_t);
+                  const int32_t*, float*, float*, float*, int, int, int, int, int, int, int, cudaStream_t);
 size_t joint_bwd_f32_ws_bytes(int, int, int, int, int);
 int joint_bwd_f32(const float*, const float*, const float*, const float*, const int32_t*, const int32_t*,
                   const int32_t*, const float*, const float*, const float*, const float*, const float*, float, float*,
-                  float*, float*, float*, int, int, int, int, int, int, void*, size_t, cudaStream_t);
+                  float*, float*, float*, int, int, int, int, int, int, int, void*, size_t, cudaStream_t);
 size_t joint_fwd_tc_ws_bytes(int, int, int, int, int, int);
-int joint_fwd_tc(const void*, const void*, int, int, const float*, const float*, const int32_t*, const int32_t*,
+int joint_fwd_tc(const void*, const void*, int, int, int, const float*, const float*, const int32_t*, const int32_t*,
                  const int32_t*, float*, float*, float*, int, int, int, int, int, int, void*, size_t, cudaStream_t);
 bool joint_tc_bwd_supported(int, int, int);
 size_t joint_bwd_tc_ws_bytes(int, int, int, int, int, int);
-int joint_bwd_tc(const void*, const void*, int, int, const float*, const float*, const int32_t*, const int32_t*,
+int joint_bwd_tc(const void*, const void*, int, int, int, const float*, const float*, const int32_t*, const int32_t*,
                  const int32_t*, const float*, const float*, const float*, const float*, const float*, const float*,
                  const float*, float, float*,
                  float*, float*, float*, int, int, int, int, int, int, void*, size_t, cudaStream_t);
@@ -91,12 +91,28 @@ static int check_dims(const char* op, int B, int T, int U1, int D, int V) {
   return 0;
 }
 
+// `precision` of the fused joint entry points: CTCVR_F32 / CTCVR_BF16 / CTCVR_BF16X3 in the low byte, OR'ed with one
+// CTCVR_ACT_* value.  Splits it into (precision, activation); false for any other bit.
+static bool split_precision(int precision, int* prec, int* act) {
+  *prec = precision & 0xff;
+  *act = (precision & ~0xff) >> 8;
+  return (*prec == CTCVR_F32 || *prec == CTCVR_BF16 || *prec == CTCVR_BF16X3) &&
+         (*act == ACT_TANH || *act == ACT_RELU || *act == ACT_GELU);
+}
+#define CTCVR_SPLIT_PRECISION(op, precision, prec, act)                                                          \
+  CTCVR_REQUIRE(split_precision(precision, &prec, &act),                                                          \
+                "%s: unknown precision 0x%x (low byte: CTCVR_F32 / CTCVR_BF16 / CTCVR_BF16X3, OR'ed with one of "  \
+                "CTCVR_ACT_TANH / CTCVR_ACT_RELU / CTCVR_ACT_GELU)", op, (unsigned)(precision))
+
 static int check_weights(const char* op, const ctcvr_decoder_weights* w) {
   CTCVR_REQUIRE(w != nullptr, "%s: weights is NULL", op);
   CTCVR_REQUIRE(w->V > 0 && w->H > 0 && w->L > 0 && w->P > 0 && w->D > 0, "%s: bad weight dims", op);
   CTCVR_REQUIRE(w->gate_tok && w->w_hh_t && w->proj_t && w->proj_b && w->pred_ffn_t && w->pred_ffn_b && w->out_t &&
                     w->out_b && (w->L == 1 || (w->w_ih_t && w->b_gate)),
                 "%s: NULL weight pointer", op);
+  CTCVR_REQUIRE(w->activation == CTCVR_ACT_TANH || w->activation == CTCVR_ACT_RELU || w->activation == CTCVR_ACT_GELU,
+                "%s: unknown activation 0x%x (CTCVR_ACT_TANH / CTCVR_ACT_RELU / CTCVR_ACT_GELU)", op,
+                (unsigned)w->activation);
   return 0;
 }
 
@@ -122,6 +138,7 @@ int ctcvr_joint_logits(const float* enc_proj, const float* pred_proj, const floa
 }
 
 size_t ctcvr_joint_rnnt_fwd_ws_bytes(int B, int T, int U1, int D, int V, int precision) {
+  precision &= 0xff;                        // the activation bits do not change the workspace
   if (precision == CTCVR_BF16 || precision == CTCVR_BF16X3)
     return joint_fwd_tc_ws_bytes(B, T, U1, D, V, precision == CTCVR_BF16X3);
   return 256;
@@ -135,12 +152,14 @@ int ctcvr_joint_rnnt_fwd(const float* enc_proj, const float* pred_proj, const fl
   CTCVR_REQUIRE(enc_proj && pred_proj && w_out && b_out && t_len && u_len && lse && lp_blank && lp_label &&
                     (targets || U1 == 1), "joint_rnnt_fwd: NULL pointer");
   CTCVR_REQUIRE(blank >= 0 && blank < V, "joint_rnnt_fwd: blank %d must be within [0, %d)", blank, V);
+  int prec = 0, act = 0;
+  CTCVR_SPLIT_PRECISION("joint_rnnt_fwd", precision, prec, act);
+  precision = prec;
   if (precision == CTCVR_BF16 || precision == CTCVR_BF16X3)
-    return joint_fwd_tc(enc_proj, pred_proj, 0, precision == CTCVR_BF16X3, w_out, b_out, targets, t_len, u_len, lse, lp_blank, lp_label, B, T, U1, D,
+    return joint_fwd_tc(enc_proj, pred_proj, 0, precision == CTCVR_BF16X3, act, w_out, b_out, targets, t_len, u_len, lse, lp_blank, lp_label, B, T, U1, D,
                         V, blank, ws, ws_bytes, ST(stream));
-  CTCVR_REQUIRE(precision == CTCVR_F32, "joint_rnnt_fwd: unknown precision %d", precision);
   return joint_fwd_f32(enc_proj, pred_proj, w_out, b_out, targets, t_len, u_len, lse, lp_blank, lp_label, B, T, U1, D,
-                       V, blank, ST(stream));
+                       V, blank, act, ST(stream));
 }
 
 int ctcvr_rnnt_lattice(const float* lp_blank, const float* lp_label, const int32_t* t_len, const int32_t* u_len,
@@ -151,6 +170,7 @@ int ctcvr_rnnt_lattice(const float* lp_blank, const float* lp_label, const int32
 }
 
 size_t ctcvr_joint_rnnt_bwd_ws_bytes(int B, int T, int U1, int D, int V, int precision) {
+  precision &= 0xff;                        // the activation bits do not change the workspace
   if (precision == CTCVR_BF16 || precision == CTCVR_BF16X3)
     return joint_bwd_tc_ws_bytes(B, T, U1, D, V, precision == CTCVR_BF16X3);
   return joint_bwd_f32_ws_bytes(B, T, U1, D, V);
@@ -168,13 +188,15 @@ int ctcvr_joint_rnnt_bwd(const float* enc_proj, const float* pred_proj, const fl
                     beta && costs && grad_costs && d_enc_proj && d_pred_proj && d_w_out && d_b_out && ws,
                 "joint_rnnt_bwd: NULL pointer");
   CTCVR_REQUIRE(blank >= 0 && blank < V, "joint_rnnt_bwd: blank %d must be within [0, %d)", blank, V);
+  int prec = 0, act = 0;
+  CTCVR_SPLIT_PRECISION("joint_rnnt_bwd", precision, prec, act);
+  precision = prec;
   if (precision == CTCVR_BF16 || precision == CTCVR_BF16X3)
-    return joint_bwd_tc(enc_proj, pred_proj, 0, precision == CTCVR_BF16X3, w_out, b_out, targets, t_len, u_len, lse, lp_blank, lp_label, alpha, beta, costs, grad_costs,
+    return joint_bwd_tc(enc_proj, pred_proj, 0, precision == CTCVR_BF16X3, act, w_out, b_out, targets, t_len, u_len, lse, lp_blank, lp_label, alpha, beta, costs, grad_costs,
                         clamp, d_enc_proj, d_pred_proj, d_w_out, d_b_out, B, T, U1, D, V, blank, ws, ws_bytes,
                         ST(stream));
-  CTCVR_REQUIRE(precision == CTCVR_F32, "joint_rnnt_bwd: unknown precision %d", precision);
   return joint_bwd_f32(enc_proj, pred_proj, w_out, b_out, targets, t_len, u_len, lse, alpha, beta, costs, grad_costs,
-                       clamp, d_enc_proj, d_pred_proj, d_w_out, d_b_out, B, T, U1, D, V, blank, ws, ws_bytes,
+                       clamp, d_enc_proj, d_pred_proj, d_w_out, d_b_out, B, T, U1, D, V, blank, act, ws, ws_bytes,
                        ST(stream));
 }
 
@@ -188,7 +210,7 @@ int ctcvr_joint_rnnt_fwd_bf16in(const void* enc_proj_bf16, const void* pred_proj
   CTCVR_REQUIRE(enc_proj_bf16 && pred_proj_bf16 && w_out && b_out && t_len && u_len && lse && lp_blank && lp_label &&
                     (targets || U1 == 1), "joint_rnnt_fwd_bf16in: NULL pointer");
   CTCVR_REQUIRE(blank >= 0 && blank < V, "joint_rnnt_fwd_bf16in: blank %d must be within [0, %d)", blank, V);
-  return joint_fwd_tc(enc_proj_bf16, pred_proj_bf16, 1, 0, w_out, b_out, targets, t_len, u_len, lse, lp_blank, lp_label, B,
+  return joint_fwd_tc(enc_proj_bf16, pred_proj_bf16, 1, 0, ACT_TANH, w_out, b_out, targets, t_len, u_len, lse, lp_blank, lp_label, B,
                       T, U1, D, V, blank, ws, ws_bytes, ST(stream));
 }
 
@@ -203,7 +225,7 @@ int ctcvr_joint_rnnt_bwd_bf16in(const void* enc_proj_bf16, const void* pred_proj
   CTCVR_REQUIRE(enc_proj_bf16 && pred_proj_bf16 && w_out && b_out && t_len && u_len && lse && lp_blank && lp_label &&
                     alpha && beta && costs && grad_costs && d_enc_proj_bf16 && d_pred_proj_bf16 && d_w_out && d_b_out && ws, "joint_rnnt_bwd_bf16in: NULL pointer");
   CTCVR_REQUIRE(blank >= 0 && blank < V, "joint_rnnt_bwd_bf16in: blank %d must be within [0, %d)", blank, V);
-  return joint_bwd_tc(enc_proj_bf16, pred_proj_bf16, 1, 0, w_out, b_out, targets, t_len, u_len, lse, lp_blank, lp_label, alpha, beta, costs,
+  return joint_bwd_tc(enc_proj_bf16, pred_proj_bf16, 1, 0, ACT_TANH, w_out, b_out, targets, t_len, u_len, lse, lp_blank, lp_label, alpha, beta, costs,
                       grad_costs, clamp, reinterpret_cast<float*>(d_enc_proj_bf16), reinterpret_cast<float*>(d_pred_proj_bf16),
                       d_w_out, d_b_out, B, T, U1, D, V, blank, ws, ws_bytes, ST(stream));
 }

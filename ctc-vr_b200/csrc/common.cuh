@@ -68,6 +68,34 @@ __device__ __forceinline__ double log_add_exp(double a, double b) {
   return m + log1p(exp(-fabs(a - b)));
 }
 
+// Joint activation z = act(h), h = enc_proj + pred_proj (CTCVR_ACT_* >> 8).  tanh is nn.Tanh, relu nn.ReLU (derivative
+// h > 0, torch's 0 at h = 0), gelu the exact erf form of nn.GELU(): h Phi(h), derivative Phi(h) + h phi(h).
+enum { ACT_TANH = 0, ACT_RELU = 1, ACT_GELU = 2 };
+
+__device__ __forceinline__ float gelu_f32(float h) { return 0.5f * h * (1.f + erff(h * 0.70710678118654752f)); }
+__device__ __forceinline__ float gelu_grad_f32(float h) {
+  const float cdf = 0.5f * (1.f + erff(h * 0.70710678118654752f));
+  return fmaf(h * 0.39894228040143268f, expf(-0.5f * h * h), cdf);
+}
+template <int ACT>
+__device__ __forceinline__ float act_f32(float h) {
+  if constexpr (ACT == ACT_RELU) return fmaxf(h, 0.f);
+  else if constexpr (ACT == ACT_GELU) return gelu_f32(h);
+  else return tanhf(h);
+}
+// act'(h) for relu / gelu (the tanh paths use 1 - z^2 from z)
+template <int ACT>
+__device__ __forceinline__ float act_grad_f32(float h) {
+  if constexpr (ACT == ACT_RELU) return h > 0.f ? 1.f : 0.f;
+  else return gelu_grad_f32(h);
+}
+// run-time form for the decoders (the branch is uniform across the launch)
+__device__ __forceinline__ float act_rt(int act, float h) {
+  if (act == ACT_RELU) return fmaxf(h, 0.f);
+  if (act == ACT_GELU) return gelu_f32(h);
+  return tanhf(h);
+}
+
 static inline size_t align_up(size_t x, size_t a) { return (x + a - 1) / a * a; }
 static inline int cdiv(long a, long b) { return (int)((a + b - 1) / b); }
 

@@ -63,11 +63,12 @@ __global__ void __launch_bounds__(DEC_THREADS, 1) rnnt_greedy_kernel(
     __syncthreads();
     if (!flags[1]) break;
     if (flags[0]) predictor_step<NB>(w, s, tok);
-    // joint: z = tanh(enc_proj[t] + pproj)
+    // joint: z = act(enc_proj[t] + pproj)
+    const int act = w.activation >> 8;
     for (int i = tid; i < D * NB; i += DEC_THREADS) {
       int d = i / NB, n = i - d * NB;
       float zz = 0.f;
-      if (tcur[n] < len[n]) zz = tanhf(enc_proj[((size_t)(n0 + n) * T + tcur[n]) * D + d] + s.pproj[i]);
+      if (tcur[n] < len[n]) zz = act_rt(act, enc_proj[((size_t)(n0 + n) * T + tcur[n]) * D + d] + s.pproj[i]);
       s.z[i] = zz;
     }
     __syncthreads();

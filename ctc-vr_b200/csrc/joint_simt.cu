@@ -6,6 +6,7 @@
 //         torchaudio.functional.rnnt_loss, model/component/transducer.py:180-187)
 //   bwd : recompute logits per utterance chunk, closed-form d cost/d logits (SURVEY.md §8 A2),
 //         then dZ = g.W, dW += g^T.z, dH = dZ*(1-z^2), d_enc = sum_u dH, d_pred = sum_t dH.
+//   relu / gelu joints: z = act(h) in the z tile, dH = dZ*act'(h) (joint.py:64-67, `activation`).
 //
 // The forward never writes logits to HBM.  The fp32 backward materialises g and z for a bounded
 // chunk of utterances in the caller's workspace (the bf16 tcgen05 path in joint_tc.cu is the
@@ -50,8 +51,11 @@ struct JointTileArgs {
   float* z;              // [nb*T*U1, D]
 };
 
-template <int MODE>
+// KIND = MODE | (joint activation << 4): the tanh kernels are joint_tile_kernel<MODE> (ACT_TANH = 0), the relu and gelu
+// kernels joint_tile_kernel<MODE + 16> and <MODE + 32>.
+template <int KIND>
 __global__ void __launch_bounds__(JT_THREADS, 1) joint_tile_kernel(JointTileArgs a) {
+  constexpr int MODE = KIND & 15, ACT = KIND >> 4;
   extern __shared__ __align__(16) float smem[];
   float* zs = smem;                         // [D][TMP]
   float* ws = zs + (size_t)a.D * TMP;       // [TK][TNP]
@@ -101,13 +105,13 @@ __global__ void __launch_bounds__(JT_THREADS, 1) joint_tile_kernel(JointTileArgs
   }
   __syncthreads();
 
-  // ---- z tile: zs[k][row] = tanh(enc[b,t,k] + pred[b,u,k]); lanes run along k (coalesced)
+  // ---- z tile: zs[k][row] = act(enc[b,t,k] + pred[b,u,k]); lanes run along k (coalesced)
   for (int r = warp; r < TM; r += JT_THREADS / 32) {
     int t = rowi[TM + r], u = rowi[2 * TM + r];
     if (t >= 0) {
       const float* e = a.enc + ((size_t)b * T + t) * D;
       const float* p = a.pred + ((size_t)b * U1 + u) * D;
-      for (int k = lane; k < D; k += 32) zs[(size_t)k * TMP + r] = tanhf(e[k] + p[k]);
+      for (int k = lane; k < D; k += 32) zs[(size_t)k * TMP + r] = act_f32<ACT>(e[k] + p[k]);
     } else {
       for (int k = lane; k < D; k += 32) zs[(size_t)k * TMP + r] = 0.f;
     }
@@ -257,12 +261,14 @@ static size_t joint_tile_smem(int D) {
 }
 
 template <int MODE>
-static int launch_joint_tile(const JointTileArgs& a, int nb, cudaStream_t st) {
+static int launch_joint_tile(const JointTileArgs& a, int nb, cudaStream_t st, int act = ACT_TANH) {
   size_t smem = joint_tile_smem(a.D);
   CTCVR_REQUIRE(smem <= 227 * 1024, "joint fp32 path: join_dim %d too large for one SM's shared memory", a.D);
-  CTCVR_CHECK_CUDA(cudaFuncSetAttribute(joint_tile_kernel<MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  const auto kern = act == ACT_RELU ? joint_tile_kernel<MODE | (ACT_RELU << 4)>
+                    : act == ACT_GELU ? joint_tile_kernel<MODE | (ACT_GELU << 4)> : joint_tile_kernel<MODE>;
+  CTCVR_CHECK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   dim3 grid(cdiv((long)a.T * a.U1, TM), nb);
-  joint_tile_kernel<MODE><<<grid, JT_THREADS, smem, st>>>(a);
+  kern<<<grid, JT_THREADS, smem, st>>>(a);
   CTCVR_LAUNCH_CHECK();
   return 0;
 }
@@ -346,6 +352,27 @@ __global__ void dh_enc_kernel(float* __restrict__ dz, const float* __restrict__ 
     d_enc[((size_t)(b0 + bl) * T + t) * D + k] = s;
   }
 }
+// Other activations: dH = dZ act'(h), h = enc + pred recomputed (gelu's derivative needs h, not z); rows outside the
+// utterance (dZ = 0 there) are skipped.
+template <int ACT>
+__global__ void dh_enc_act_kernel(float* __restrict__ dz, const float* __restrict__ enc, const float* __restrict__ pred,
+                                  const int32_t* __restrict__ t_len, const int32_t* __restrict__ u_len,
+                                  float* __restrict__ d_enc, int b0, int T, int U1, int D) {
+  int t = blockIdx.x, bl = blockIdx.y, b = b0 + bl;
+  const int Tb = max(min(t_len[b], T), 0), Ub = max(min(u_len[b], U1 - 1), 0);
+  size_t row0 = ((size_t)bl * T + t) * U1;
+  for (int k = threadIdx.x; k < D; k += blockDim.x) {
+    const float e = enc[((size_t)b * T + t) * D + k];
+    float s = 0.f;
+    for (int u = 0; u < U1; ++u) {
+      size_t i = (row0 + u) * D + k;
+      const float dh = (t < Tb && u <= Ub) ? dz[i] * act_grad_f32<ACT>(e + pred[((size_t)b * U1 + u) * D + k]) : 0.f;
+      dz[i] = dh;
+      s += dh;
+    }
+    d_enc[((size_t)b * T + t) * D + k] = s;
+  }
+}
 // d_pred[b,u,:] = sum_t dH.  One CTA per (u, b_local).
 __global__ void dh_pred_kernel(const float* __restrict__ dh, float* __restrict__ d_pred, int b0, int T, int U1, int D) {
   int u = blockIdx.x, bl = blockIdx.y;
@@ -390,18 +417,18 @@ int joint_logits_f32(const float* enc, const float* pred, const float* w, const 
 
 int joint_fwd_f32(const float* enc, const float* pred, const float* w, const float* bias, const int32_t* targets,
                   const int32_t* t_len, const int32_t* u_len, float* lse, float* lp_blank, float* lp_label,
-                  int B, int T, int U1, int D, int V, int blank, cudaStream_t st) {
+                  int B, int T, int U1, int D, int V, int blank, int act, cudaStream_t st) {
   JointTileArgs a{};
   a.enc = enc; a.pred = pred; a.w = w; a.bias = bias; a.targets = targets; a.t_len = t_len; a.u_len = u_len;
   a.lse = lse; a.lp_blank = lp_blank; a.lp_label = lp_label;
   a.B = B; a.T = T; a.U1 = U1; a.D = D; a.V = V; a.blank = blank;
-  return launch_joint_tile<MODE_STATS>(a, B, st);
+  return launch_joint_tile<MODE_STATS>(a, B, st, act);
 }
 
 int joint_bwd_f32(const float* enc, const float* pred, const float* w, const float* bias, const int32_t* targets,
                   const int32_t* t_len, const int32_t* u_len, const float* lse, const float* alpha,
                   const float* beta, const float* costs, const float* grad_costs, float clamp, float* d_enc,
-                  float* d_pred, float* d_w, float* d_b, int B, int T, int U1, int D, int V, int blank,
+                  float* d_pred, float* d_w, float* d_b, int B, int T, int U1, int D, int V, int blank, int act,
                   void* ws, size_t ws_bytes, cudaStream_t st) {
   CTCVR_REQUIRE(ws_bytes >= joint_bwd_f32_ws_bytes(B, T, U1, D, V), "joint_rnnt_bwd fp32: workspace too small");
   const int nb_max = bwd_f32_chunk_utts(B, T, U1, D, V);
@@ -419,7 +446,7 @@ int joint_bwd_f32(const float* enc, const float* pred, const float* w, const flo
     a.B = B; a.T = T; a.U1 = U1; a.D = D; a.V = V; a.blank = blank; a.b0 = b0;
     a.lse_in = lse; a.alpha = alpha; a.beta = beta; a.costs = costs; a.grad_costs = grad_costs; a.clamp = clamp;
     a.g = g; a.z = z;
-    if (int rc = launch_joint_tile<MODE_GRAD>(a, nb, st)) return rc;
+    if (int rc = launch_joint_tile<MODE_GRAD>(a, nb, st, act)) return rc;
     // dZ[R,D] = g[R,V] . W[V,D]
     {
       dim3 grid(cdiv(D, 64), cdiv(R, 64), 1);
@@ -442,7 +469,12 @@ int joint_bwd_f32(const float* enc, const float* pred, const float* w, const flo
       colsum_kernel<<<grid, 128, 0, st>>>(g, d_b, R, V, rows_per);
       CTCVR_LAUNCH_CHECK();
     }
-    dh_enc_kernel<<<dim3(T, nb), 256, 0, st>>>(dz, z, d_enc, b0, T, U1, D);
+    if (act == ACT_RELU)
+      dh_enc_act_kernel<ACT_RELU><<<dim3(T, nb), 256, 0, st>>>(dz, enc, pred, t_len, u_len, d_enc, b0, T, U1, D);
+    else if (act == ACT_GELU)
+      dh_enc_act_kernel<ACT_GELU><<<dim3(T, nb), 256, 0, st>>>(dz, enc, pred, t_len, u_len, d_enc, b0, T, U1, D);
+    else
+      dh_enc_kernel<<<dim3(T, nb), 256, 0, st>>>(dz, z, d_enc, b0, T, U1, D);
     CTCVR_LAUNCH_CHECK();
     dh_pred_kernel<<<dim3(U1, nb), 256, 0, st>>>(dz, d_pred, b0, T, U1, D);
     CTCVR_LAUNCH_CHECK();

@@ -172,7 +172,7 @@ constexpr int DWR_A_STAGES = 3;
 constexpr int DWR_ACC_COLS = 416;
 
 // rows R0 .. R0+2*NP-1 of a tile: NP packed (row 2c, row 2c+1) pairs of tanh(e[tloc] + p[ul]), row = tloc*P + ul
-template <int P, int TT, int R0, int NP>
+template <int P, int TT, int R0, int NP, int ACT = ACT_TANH>
 __device__ __forceinline__ void dwr_rows(const uint32_t (&e)[TT], const uint32_t (&pr)[P], uint32_t (&w)[NP]) {
 #pragma unroll
   for (int c = 0; c < NP; ++c) {
@@ -181,18 +181,18 @@ __device__ __forceinline__ void dwr_rows(const uint32_t (&e)[TT], const uint32_t
     const int u0 = r0 % P, u1 = r1 % P;
     const uint32_t ep = __byte_perm(e[tl0], e[tl1], 0x5410);
     const uint32_t pp = __byte_perm(pr[u0], pr[u1], 0x5410);
-    w[c] = tanh_add_bf16x2_packed(ep, pp);
+    w[c] = act_add_bf16x2_packed<ACT>(ep, pp);
   }
 }
 
-// bf16x3: the same rows as hi / lo pairs of the fp32 tanh(e + p)
-template <int P, int TT, int R0, int NP>
+// bf16x3: the same rows as hi / lo pairs of the fp32 act(e + p)
+template <int P, int TT, int R0, int NP, int ACT = ACT_TANH>
 __device__ __forceinline__ void dwr_rows_x3(const float (&e)[TT], const float (&pr)[P], uint32_t (&hi)[NP], uint32_t (&lo)[NP]) {
 #pragma unroll
   for (int c = 0; c < NP; ++c) {
     const int r0 = R0 + 2 * c, r1 = r0 + 1;
     const int tl0 = (r0 / P < TT) ? r0 / P : TT - 1, tl1 = (r1 / P < TT) ? r1 / P : TT - 1;
-    const float z0 = tanhf(e[tl0] + pr[r0 % P]), z1 = tanhf(e[tl1] + pr[r1 % P]);
+    const float z0 = act_f32<ACT>(e[tl0] + pr[r0 % P]), z1 = act_f32<ACT>(e[tl1] + pr[r1 % P]);
     const __nv_bfloat162 h = __floats2bfloat162_rn(z0, z1);
     hi[c] = *reinterpret_cast<const uint32_t*>(&h);
     lo[c] = pack_bf16(z0 - __low2float(h), z1 - __high2float(h));
@@ -209,7 +209,8 @@ __host__ __device__ constexpr uint32_t dwr_slab_bytes() {          // [d half][p
 // SPLIT = true (precision bf16x3): dW^T = z_hi^T G_hi + z_hi^T G_lo + z_lo^T G_hi.  Per 64-row k-block the G loader
 // brings a G_hi and a G_lo stage (from the two spills), the producers write a z_hi and a z_lo A stage (z in fp32 from
 // the fp32 rows, read straight from global memory: no slab ring, warp 3 idles).
-template <int P, int TT, bool SPLIT>
+// ACT: the joint activation of the recomputed z (ACT_TANH / ACT_RELU / ACT_GELU).
+template <int P, int TT, bool SPLIT, int ACT = ACT_TANH>
 __device__ __forceinline__ void dw_gemm_rz_body(const CUtensorMap& tmap_e, const CUtensorMap& tmap_p,
                                                 const __nv_bfloat16* __restrict__ gr, const __nv_bfloat16* __restrict__ gr_lo,
                                                 const float* __restrict__ enc, const float* __restrict__ pred,
@@ -377,10 +378,10 @@ __device__ __forceinline__ void dw_gemm_rz_body(const CUtensorMap& tmap_e, const
           uint32_t wh[NP], wl[NP];
           auto rows = [&](auto HH) {
             constexpr int R = decltype(HH)::value * 64;
-            if (rh == 0) dwr_rows_x3<P, TT, R, NP>(e, pr, wh, wl);
-            else if (rh == 1) dwr_rows_x3<P, TT, R + 2 * NP, NP>(e, pr, wh, wl);
-            else if (rh == 2) dwr_rows_x3<P, TT, R + 4 * NP, NP>(e, pr, wh, wl);
-            else dwr_rows_x3<P, TT, R + 6 * NP, NP>(e, pr, wh, wl);
+            if (rh == 0) dwr_rows_x3<P, TT, R, NP, ACT>(e, pr, wh, wl);
+            else if (rh == 1) dwr_rows_x3<P, TT, R + 2 * NP, NP, ACT>(e, pr, wh, wl);
+            else if (rh == 2) dwr_rows_x3<P, TT, R + 4 * NP, NP, ACT>(e, pr, wh, wl);
+            else dwr_rows_x3<P, TT, R + 6 * NP, NP, ACT>(e, pr, wh, wl);
           };
           if (hh == 0) rows(std::integral_constant<int, 0>{}); else rows(std::integral_constant<int, 1>{});
           Pipe al2 = ap;
@@ -433,10 +434,10 @@ __device__ __forceinline__ void dw_gemm_rz_body(const CUtensorMap& tmap_e, const
         // rows hh*64 + rh*2*NP ..: one instantiation per (hh, rh) so that every (tloc, ul) is a compile-time constant
         auto rows = [&](auto HH) {
           constexpr int R = decltype(HH)::value * 64;
-          if (rh == 0) dwr_rows<P, TT, R, NP>(e, pr, w);
-          else if (rh == 1) dwr_rows<P, TT, R + 2 * NP, NP>(e, pr, w);
-          else if (rh == 2) dwr_rows<P, TT, R + 4 * NP, NP>(e, pr, w);
-          else dwr_rows<P, TT, R + 6 * NP, NP>(e, pr, w);
+          if (rh == 0) dwr_rows<P, TT, R, NP, ACT>(e, pr, w);
+          else if (rh == 1) dwr_rows<P, TT, R + 2 * NP, NP, ACT>(e, pr, w);
+          else if (rh == 2) dwr_rows<P, TT, R + 4 * NP, NP, ACT>(e, pr, w);
+          else dwr_rows<P, TT, R + 6 * NP, NP, ACT>(e, pr, w);
         };
         if (hh == 0) rows(std::integral_constant<int, 0>{}); else rows(std::integral_constant<int, 1>{});
         mbar_wait(a_empty(ap.stage), ap.phase ^ 1u, 54);
@@ -488,6 +489,32 @@ dw_gemm_rz_x3_kernel(const __grid_constant__ CUtensorMap tmap_e, const __grid_co
                      const int* __restrict__ ntiles_ptr, float* __restrict__ partials, int D, int Vp, int KBG, int KS) {
   dw_gemm_rz_body<P, TT, true>(tmap_e, tmap_p, gr, gr_lo, enc, pred, tile_rows, ntiles_ptr, partials, D, Vp, KBG, KS);
 }
+// relu / gelu joints, named apart for profiler traces
+#define CTCVR_DWR_ACT(name, act)                                                                                   \
+  template <int P, int TT>                                                                                          \
+  __global__ void __launch_bounds__(DWR_THREADS, 1)                                                                 \
+  name(const __grid_constant__ CUtensorMap tmap_e, const __grid_constant__ CUtensorMap tmap_p,                      \
+       const __nv_bfloat16* __restrict__ gr, const int4* __restrict__ tile_rows, const int* __restrict__ ntiles_ptr, \
+       float* __restrict__ partials, int D, int Vp, int KBG, int KS) {                                              \
+    dw_gemm_rz_body<P, TT, false, act>(tmap_e, tmap_p, gr, nullptr, nullptr, nullptr, tile_rows, ntiles_ptr,        \
+                                       partials, D, Vp, KBG, KS);                                                   \
+  }
+CTCVR_DWR_ACT(dw_gemm_rz_relu_kernel, ACT_RELU)
+CTCVR_DWR_ACT(dw_gemm_rz_gelu_kernel, ACT_GELU)
+#undef CTCVR_DWR_ACT
+#define CTCVR_DWR_X3_ACT(name, act)                                                                                \
+  template <int P, int TT>                                                                                          \
+  __global__ void __launch_bounds__(DWR_THREADS, 1)                                                                 \
+  name(const __grid_constant__ CUtensorMap tmap_e, const __grid_constant__ CUtensorMap tmap_p,                      \
+       const __nv_bfloat16* __restrict__ gr, const __nv_bfloat16* __restrict__ gr_lo,                               \
+       const float* __restrict__ enc, const float* __restrict__ pred, const int4* __restrict__ tile_rows,           \
+       const int* __restrict__ ntiles_ptr, float* __restrict__ partials, int D, int Vp, int KBG, int KS) {          \
+    dw_gemm_rz_body<P, TT, true, act>(tmap_e, tmap_p, gr, gr_lo, enc, pred, tile_rows, ntiles_ptr, partials, D, Vp, \
+                                      KBG, KS);                                                                     \
+  }
+CTCVR_DWR_X3_ACT(dw_gemm_rz_x3_relu_kernel, ACT_RELU)
+CTCVR_DWR_X3_ACT(dw_gemm_rz_x3_gelu_kernel, ACT_GELU)
+#undef CTCVR_DWR_X3_ACT
 
 // dW GEMM shared memory: G stages, slab ring (bf16 only), barriers
 template <int P>
@@ -810,8 +837,12 @@ static int sm_count() {
 int joint_fwd_f32(const float*, const float*, const float*, const float*, const int32_t*, const int32_t*,
                   const int32_t*, float*, float*, float*, int, int, int, int, int, int, cudaStream_t);
 
-// split = 1: precision bf16x3 (fp32 inputs, hi / lo operand split, joint_fwd2_x3_kernel)
-int joint_fwd_tc(const void* enc_v, const void* pred_v, int in_bf16, int split, const float* w, const float* bias,
+// the kernel of a family for the joint activation act (ACT_TANH / ACT_RELU / ACT_GELU)
+template <class K>
+static K pick_act(int act, K tanh_k, K relu_k, K gelu_k) { return act == ACT_RELU ? relu_k : act == ACT_GELU ? gelu_k : tanh_k; }
+
+// split = 1: precision bf16x3 (fp32 inputs, hi / lo operand split, joint_fwd2_x3_kernel); act: the joint activation
+int joint_fwd_tc(const void* enc_v, const void* pred_v, int in_bf16, int split, int act, const float* w, const float* bias,
                  const int32_t* targets, const int32_t* t_len, const int32_t* u_len, float* lse, float* lp_blank,
                  float* lp_label, int B, int T, int U1, int D, int V, int blank, void* ws, size_t ws_bytes, cudaStream_t st) {
   const float* enc = reinterpret_cast<const float*>(enc_v);
@@ -846,13 +877,15 @@ int joint_fwd_tc(const void* enc_v, const void* pred_v, int in_bf16, int split, 
     p.w_stages = ws_n;
     const size_t smem = fwd2_smem_bytes(NH, Vp, ws_n);
     CTCVR_REQUIRE(smem <= 232448, "joint_rnnt_fwd bf16x3: shared memory budget exceeded (%zu B)", smem);
-    CTCVR_CHECK_CUDA(cudaFuncSetAttribute(joint_fwd2_x3_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    const auto kern = pick_act(act, joint_fwd2_x3_kernel, joint_fwd2_x3_relu_kernel, joint_fwd2_x3_gelu_kernel);
+    CTCVR_CHECK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     const CUtensorMap unused{};             // the bf16x3 producers read the fp32 rows directly
-    joint_fwd2_x3_kernel<<<min(sm_count(), mt), F_THREADS, smem, st>>>(unused, unused, p);
+    kern<<<min(sm_count(), mt), F_THREADS, smem, st>>>(unused, unused, p);
     CTCVR_LAUNCH_CHECK();
     return 0;
   }
-  const bool use_pair = fwdp_smem_bytes(NH, D) <= 232448 && sm_count() >= 2 && !g_force_single_cta;
+  // the parked CTA-pair forward computes tanh only
+  const bool use_pair = fwdp_smem_bytes(NH, D) <= 232448 && sm_count() >= 2 && !g_force_single_cta && act == ACT_TANH;
   {
     PrepArgs q{};
     q.fwd_pair = use_pair ? 1 : 0;
@@ -905,9 +938,10 @@ int joint_fwd_tc(const void* enc_v, const void* pred_v, int in_bf16, int split, 
   p.w_stages = ws_n;
   const size_t smem = fwd2_smem_bytes(NH, Vp, ws_n);
   CTCVR_REQUIRE(smem <= 232448, "joint_rnnt_fwd bf16: shared memory budget exceeded (%zu B)", smem);
-  CTCVR_CHECK_CUDA(cudaFuncSetAttribute(joint_fwd2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  const auto kern = pick_act(act, joint_fwd2_kernel, joint_fwd2_relu_kernel, joint_fwd2_gelu_kernel);
+  CTCVR_CHECK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   const int grid = min(sm_count(), mt);
-  joint_fwd2_kernel<<<grid, F_THREADS, smem, st>>>(tmap_e, tmap_p, p);
+  kern<<<grid, F_THREADS, smem, st>>>(tmap_e, tmap_p, p);
   CTCVR_LAUNCH_CHECK();
   return 0;
 }
@@ -967,28 +1001,31 @@ size_t joint_bwd_tc_ws_bytes(int B, int T, int U1, int D, int V, int split) {
 // precision bf16x3: the single-CTA backward kernel and the dW GEMM in their split forms (fp32 inputs and gradients)
 template <int P, int TT>
 static int joint_bwd_x3(const float* enc, const float* pred, BwdParams& p, const BwdWs& W, const int32_t* t_len,
-                        const int32_t* u_len, float* d_enc, float* d_w, int B, int T, int U1, int D, int V, cudaStream_t st) {
+                        const int32_t* u_len, float* d_enc, float* d_w, int B, int T, int U1, int D, int V, int act,
+                        cudaStream_t st) {
   const int Vp = p.Vp, KBG = (Vp + 63) / 64, MB = D / 128;
   const CUtensorMap unused{};               // the split kernels read the fp32 rows directly
   const size_t smem = bwd3_smem_bytes(p.NH, Vp, D, true);
   CTCVR_REQUIRE(smem <= 232448 && p.r1_stages >= 2, "joint_rnnt_bwd bf16x3: shared memory budget exceeded (%zu B)", smem);
-  CTCVR_CHECK_CUDA(cudaFuncSetAttribute(joint_bwd3_x3_kernel<P, TT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  joint_bwd3_x3_kernel<P, TT><<<min(sm_count(), W.mt), NTHREADS, smem, st>>>(unused, unused, p);
+  const auto k1 = pick_act(act, joint_bwd3_x3_kernel<P, TT>, joint_bwd3_x3_relu_kernel<P, TT>, joint_bwd3_x3_gelu_kernel<P, TT>);
+  CTCVR_CHECK_CUDA(cudaFuncSetAttribute(k1, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  k1<<<min(sm_count(), W.mt), NTHREADS, smem, st>>>(unused, unused, p);
   CTCVR_LAUNCH_CHECK();
   reduce_denc_kernel<false><<<B * T, 128, 0, st>>>(W.d_enc_part, t_len, u_len, d_enc, B, T, U1, D, P, nullptr, nullptr);
   CTCVR_LAUNCH_CHECK();
   const size_t smem2 = dwr_smem_bytes<P>(KBG, true);
   CTCVR_REQUIRE(smem2 <= 232448, "dW GEMM bf16x3: shared memory budget exceeded (%zu B)", smem2);
-  CTCVR_CHECK_CUDA(cudaFuncSetAttribute(dw_gemm_rz_x3_kernel<P, TT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem2));
-  dw_gemm_rz_x3_kernel<P, TT><<<dim3(MB, W.KS), DWR_THREADS, smem2, st>>>(unused, unused, W.gt, W.gt_lo, enc, pred, W.tile_rows,
-                                                                        W.ntiles, W.partials, D, Vp, KBG, W.KS);
+  const auto k2 = pick_act(act, dw_gemm_rz_x3_kernel<P, TT>, dw_gemm_rz_x3_relu_kernel<P, TT>, dw_gemm_rz_x3_gelu_kernel<P, TT>);
+  CTCVR_CHECK_CUDA(cudaFuncSetAttribute(k2, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem2));
+  k2<<<dim3(MB, W.KS), DWR_THREADS, smem2, st>>>(unused, unused, W.gt, W.gt_lo, enc, pred, W.tile_rows, W.ntiles, W.partials, D,
+                                                 Vp, KBG, W.KS);
   CTCVR_LAUNCH_CHECK();
   reduce_dw_kernel<<<dim3(cdiv(D, 8), cdiv(Vp, 32)), 256, 0, st>>>(W.partials, d_w, D, V, Vp, W.KS);
   CTCVR_LAUNCH_CHECK();
   return 0;
 }
 
-int joint_bwd_tc(const void* enc_v, const void* pred_v, int in_bf16, int split, const float* w, const float* bias, const int32_t* targets,
+int joint_bwd_tc(const void* enc_v, const void* pred_v, int in_bf16, int split, int act, const float* w, const float* bias, const int32_t* targets,
                  const int32_t* t_len, const int32_t* u_len, const float* lse, const float* lp_blank, const float* lp_label,
                  const float* alpha, const float* beta,
                  const float* costs, const float* grad_costs, float clamp, float* d_enc, float* d_pred, float* d_w,
@@ -1026,8 +1063,8 @@ int joint_bwd_tc(const void* enc_v, const void* pred_v, int in_bf16, int split, 
     p.d_enc_part = W.d_enc_part; p.d_pred = d_pred; p.d_bias = d_b;
     p.prof = g_prof_buf;
     tc_error_host_word(&p.err_host);
-    return G.P == 21 ? joint_bwd_x3<21, 6>(enc, pred, p, W, t_len, u_len, d_enc, d_w, B, T, U1, D, V, st)
-                     : joint_bwd_x3<16, 8>(enc, pred, p, W, t_len, u_len, d_enc, d_w, B, T, U1, D, V, st);
+    return G.P == 21 ? joint_bwd_x3<21, 6>(enc, pred, p, W, t_len, u_len, d_enc, d_w, B, T, U1, D, V, act, st)
+                     : joint_bwd_x3<16, 8>(enc, pred, p, W, t_len, u_len, d_enc, d_w, B, T, U1, D, V, act, st);
   }
   // CTA-pair kernel (joint_tc_bwd_pair.cuh): D in 256-row blocks of dZ^T, tiles paired along the frame axis
   const size_t smem_pair = G.P == 21 ? bwd4_smem_bytes<21>(NH, Vp, D) : bwd4_smem_bytes<16>(NH, Vp, D);
@@ -1077,23 +1114,27 @@ int joint_bwd_tc(const void* enc_v, const void* pred_v, int in_bf16, int split, 
       p.r1_stages = bwd4_r1_stages(NH, Vp);
       const int gridp = std::max(2, std::min(sm_count() & ~1, mt & ~1));
       if (G.P == 21) {
-        CTCVR_CHECK_CUDA(cudaFuncSetAttribute(joint_bwd4_kernel<21, 6>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_pair));
-        joint_bwd4_kernel<21, 6><<<gridp, NTHREADS, smem_pair, st>>>(tmap_e, tmap_e2, tmap_p, p);
+        const auto k = pick_act(act, joint_bwd4_kernel<21, 6>, joint_bwd4_relu_kernel<21, 6>, joint_bwd4_gelu_kernel<21, 6>);
+        CTCVR_CHECK_CUDA(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_pair));
+        k<<<gridp, NTHREADS, smem_pair, st>>>(tmap_e, tmap_e2, tmap_p, p);
       } else {
-        CTCVR_CHECK_CUDA(cudaFuncSetAttribute(joint_bwd4_kernel<16, 8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_pair));
-        joint_bwd4_kernel<16, 8><<<gridp, NTHREADS, smem_pair, st>>>(tmap_e, tmap_e2, tmap_p, p);
+        const auto k = pick_act(act, joint_bwd4_kernel<16, 8>, joint_bwd4_relu_kernel<16, 8>, joint_bwd4_gelu_kernel<16, 8>);
+        CTCVR_CHECK_CUDA(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_pair));
+        k<<<gridp, NTHREADS, smem_pair, st>>>(tmap_e, tmap_e2, tmap_p, p);
       }
       CTCVR_LAUNCH_CHECK();
     } else {
     const size_t smem = bwd3_smem_bytes(NH, Vp, D);
     CTCVR_REQUIRE(smem <= 232448 && p.r1_stages >= 2, "joint_rnnt_bwd bf16: shared memory budget exceeded (%zu B)", smem);
     if (G.P == 21) {
-      CTCVR_CHECK_CUDA(cudaFuncSetAttribute(joint_bwd3_kernel<21, 6>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-      joint_bwd3_kernel<21, 6><<<grid, NTHREADS, smem, st>>>(tmap_e, tmap_p, p);
+      const auto k = pick_act(act, joint_bwd3_kernel<21, 6>, joint_bwd3_relu_kernel<21, 6>, joint_bwd3_gelu_kernel<21, 6>);
+      CTCVR_CHECK_CUDA(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+      k<<<grid, NTHREADS, smem, st>>>(tmap_e, tmap_p, p);
       CTCVR_LAUNCH_CHECK();
     } else {
-      CTCVR_CHECK_CUDA(cudaFuncSetAttribute(joint_bwd3_kernel<16, 8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-      joint_bwd3_kernel<16, 8><<<grid, NTHREADS, smem, st>>>(tmap_e, tmap_p, p);
+      const auto k = pick_act(act, joint_bwd3_kernel<16, 8>, joint_bwd3_relu_kernel<16, 8>, joint_bwd3_gelu_kernel<16, 8>);
+      CTCVR_CHECK_CUDA(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+      k<<<grid, NTHREADS, smem, st>>>(tmap_e, tmap_p, p);
       CTCVR_LAUNCH_CHECK();
     }
     }
@@ -1110,15 +1151,15 @@ int joint_bwd_tc(const void* enc_v, const void* pred_v, int in_bf16, int split, 
     if (G.P == 21) {
       const size_t smem = 1024 + (size_t)DW_STAGES * ((size_t)KBG * 8192) + DWR_S_STAGES * dwr_slab_bytes<21>() + 256;
       CTCVR_REQUIRE(smem <= 232448, "dW GEMM: shared memory budget exceeded (%zu B)", smem);
-      CTCVR_CHECK_CUDA(cudaFuncSetAttribute(dw_gemm_rz_kernel<21, 6>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-      dw_gemm_rz_kernel<21, 6><<<dim3(MB, W.KS), DWR_THREADS, smem, st>>>(tmap_e, tmap_p, W.gt, W.tile_rows, W.ntiles,
-                                                                         W.partials, D, Vp, KBG, W.KS);
+      const auto k = pick_act(act, dw_gemm_rz_kernel<21, 6>, dw_gemm_rz_relu_kernel<21, 6>, dw_gemm_rz_gelu_kernel<21, 6>);
+      CTCVR_CHECK_CUDA(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+      k<<<dim3(MB, W.KS), DWR_THREADS, smem, st>>>(tmap_e, tmap_p, W.gt, W.tile_rows, W.ntiles, W.partials, D, Vp, KBG, W.KS);
     } else {
       const size_t smem = 1024 + (size_t)DW_STAGES * ((size_t)KBG * 8192) + DWR_S_STAGES * dwr_slab_bytes<16>() + 256;
       CTCVR_REQUIRE(smem <= 232448, "dW GEMM: shared memory budget exceeded (%zu B)", smem);
-      CTCVR_CHECK_CUDA(cudaFuncSetAttribute(dw_gemm_rz_kernel<16, 8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-      dw_gemm_rz_kernel<16, 8><<<dim3(MB, W.KS), DWR_THREADS, smem, st>>>(tmap_e, tmap_p, W.gt, W.tile_rows, W.ntiles,
-                                                                         W.partials, D, Vp, KBG, W.KS);
+      const auto k = pick_act(act, dw_gemm_rz_kernel<16, 8>, dw_gemm_rz_relu_kernel<16, 8>, dw_gemm_rz_gelu_kernel<16, 8>);
+      CTCVR_CHECK_CUDA(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+      k<<<dim3(MB, W.KS), DWR_THREADS, smem, st>>>(tmap_e, tmap_p, W.gt, W.tile_rows, W.ntiles, W.partials, D, Vp, KBG, W.KS);
     }
     CTCVR_LAUNCH_CHECK();
   }

@@ -177,9 +177,31 @@ __device__ __forceinline__ void carve_bwd3(Bwd3Smem& L, uint8_t* raw, int NH, in
 
 // rows C0 .. C0+15 (= TMEM columns) of d block values w[]: dH = dZ * (1 - z^2), z = tanh(e[tloc] + p[ul]) recomputed
 // as packed bf16 pairs exactly as the P1 producers and the dW GEMM form it.  Every (tloc, ul) is a compile-time constant.
-template <int P, int TT, int C0>
+// Other activations (ACT): dH = dZ act'(h) with h the packed bf16 sum the producers form, act' in fp32.
+template <int P, int TT, int C0, int ACT = ACT_TANH>
 __device__ __forceinline__ void p4_chunk(const float (&w)[16], const uint32_t (&e)[TT], const uint32_t (&pr)[P],
                                          float (&es)[TT], float (&pa)[P]) {
+  if constexpr (ACT != ACT_TANH) {
+#pragma unroll
+    for (int j = 0; j < 16; j += 2) {
+      const int c = C0 + j;
+      if (c < TT * P) {
+        const int tl0 = c / P, u0 = c % P;
+        const int c1 = c + 1;
+        const int tl1 = (c1 / P < TT) ? c1 / P : TT - 1, u1 = c1 % P;
+        const uint32_t hh = add_bf16x2(__byte_perm(e[tl0], e[tl1], 0x5410), __byte_perm(pr[u0], pr[u1], 0x5410));
+        const float h0 = w[j] * act_grad_f32<ACT>(__uint_as_float(hh << 16));
+        es[tl0] += h0;
+        pa[u0] += h0;
+        if (c1 < TT * P) {
+          const float h1 = w[j + 1] * act_grad_f32<ACT>(__uint_as_float(hh & 0xffff0000u));
+          es[tl1] += h1;
+          pa[u1] += h1;
+        }
+      }
+    }
+    return;
+  }
 #pragma unroll
   for (int j = 0; j < 16; j += 2) {
     const int c = C0 + j;
@@ -203,8 +225,8 @@ __device__ __forceinline__ void p4_chunk(const float (&w)[16], const uint32_t (&
   }
 }
 
-// bf16x3 form of p4_chunk: z = tanh(e + p) in fp32 from the fp32 rows
-template <int P, int TT, int C0>
+// bf16x3 form of p4_chunk: z = tanh(e + p) in fp32 from the fp32 rows (other activations: act'(e + p) in fp32)
+template <int P, int TT, int C0, int ACT = ACT_TANH>
 __device__ __forceinline__ void p4_chunk(const float (&w)[16], const float (&e)[TT], const float (&pr)[P],
                                              float (&es)[TT], float (&pa)[P]) {
 #pragma unroll
@@ -212,8 +234,13 @@ __device__ __forceinline__ void p4_chunk(const float (&w)[16], const float (&e)[
     const int c = C0 + j;
     if (c < TT * P) {
       const int tl = c / P, u = c % P;
-      const float z = tanhf(e[tl] + pr[u]);
-      const float h = w[j] * fmaf(-z, z, 1.f);
+      float h;
+      if constexpr (ACT == ACT_TANH) {
+        const float z = tanhf(e[tl] + pr[u]);
+        h = w[j] * fmaf(-z, z, 1.f);
+      } else {
+        h = w[j] * act_grad_f32<ACT>(e[tl] + pr[u]);
+      }
       es[tl] += h;
       pa[u] += h;
     }
@@ -228,7 +255,8 @@ __device__ __forceinline__ void p4_chunk(const float (&w)[16], const float (&e)[
 //   P4  dH = dZ (1 - z^2) with z = tanh(e + p) in fp32 from the fp32 rows (global memory)
 //   d_bias = column sums of G_hi plus column sums of G_lo (after the reload)
 // Shared memory: the bf16 layout without the two slab regions (P1 ring / P4 slab).
-template <int P, int TT, bool SPLIT>
+// ACT: the joint activation of the P1 producers and the P4 derivative (ACT_TANH / ACT_RELU / ACT_GELU).
+template <int P, int TT, bool SPLIT, int ACT = ACT_TANH>
 __device__ __forceinline__ void joint_bwd3_body(const CUtensorMap& tmap_e, const CUtensorMap& tmap_p, const BwdParams& p) {
   extern __shared__ uint8_t smem_raw[];
   Bwd3Smem L;
@@ -576,8 +604,8 @@ __device__ __forceinline__ void joint_bwd3_body(const CUtensorMap& tmap_e, const
               const float4 e0 = __ldg(e4), e1 = __ldg(e4 + 1), e2 = __ldg(e4 + 2), e3 = __ldg(e4 + 3);
               const float4 q0 = __ldg(p4), q1 = __ldg(p4 + 1), q2 = __ldg(p4 + 2), q3 = __ldg(p4 + 3);
               uint32_t hi[8], lo[8];
-              tanh_split8(e0, e1, q0, q1, hi, lo);
-              tanh_split8(e2, e3, q2, q3, hi + 4, lo + 4);
+              tanh_split8<ACT>(e0, e1, q0, q1, hi, lo);
+              tanh_split8<ACT>(e2, e3, q2, q3, hi + 4, lo + 4);
               if (c == 0) {
                 mbar_wait(L.a_empty(s_hi), ph_hi ^ 1u, 42);
                 mbar_wait(L.a_empty(s_lo), ph_lo ^ 1u, 42);
@@ -607,10 +635,10 @@ __device__ __forceinline__ void joint_bwd3_body(const CUtensorMap& tmap_e, const
             const uint32_t c = (uint32_t)(kh * 4 + c4);
             const uint4 ev = lds128(sb + e_row + ((c ^ e_sw) << 4));
             const uint4 pv = lds128(sb + p_row + ((c ^ p_sw) << 4));
-            w[4 * c4 + 0] = tanh_add_bf16x2_packed(ev.x, pv.x);
-            w[4 * c4 + 1] = tanh_add_bf16x2_packed(ev.y, pv.y);
-            w[4 * c4 + 2] = tanh_add_bf16x2_packed(ev.z, pv.z);
-            w[4 * c4 + 3] = tanh_add_bf16x2_packed(ev.w, pv.w);
+            w[4 * c4 + 0] = act_add_bf16x2_packed<ACT>(ev.x, pv.x);
+            w[4 * c4 + 1] = act_add_bf16x2_packed<ACT>(ev.y, pv.y);
+            w[4 * c4 + 2] = act_add_bf16x2_packed<ACT>(ev.z, pv.z);
+            w[4 * c4 + 3] = act_add_bf16x2_packed<ACT>(ev.w, pv.w);
           }
           tmem_st16(tq + (uint32_t)(B_ACC_COLS + a_stg * 32 + kh * 16), w);
           tmem_st_wait();
@@ -832,27 +860,27 @@ __device__ __forceinline__ void joint_bwd3_body(const CUtensorMap& tmap_e, const
             tmem_ld16(tb, v0);
             tmem_ld_wait();
             tmem_ld16(tb + 16, v1);
-            p4_chunk<P, TT, 0>(v0, e, pr, es, pacc[mbl]);
+            p4_chunk<P, TT, 0, ACT>(v0, e, pr, es, pacc[mbl]);
             tmem_ld_wait();
             tmem_ld16(tb + 32, v0);
-            p4_chunk<P, TT, 16>(v1, e, pr, es, pacc[mbl]);
+            p4_chunk<P, TT, 16, ACT>(v1, e, pr, es, pacc[mbl]);
             tmem_ld_wait();
             tmem_ld16(tb + 48, v1);
-            p4_chunk<P, TT, 32>(v0, e, pr, es, pacc[mbl]);
+            p4_chunk<P, TT, 32, ACT>(v0, e, pr, es, pacc[mbl]);
             tmem_ld_wait();
             tmem_ld16(tb + 64, v0);
-            p4_chunk<P, TT, 48>(v1, e, pr, es, pacc[mbl]);
+            p4_chunk<P, TT, 48, ACT>(v1, e, pr, es, pacc[mbl]);
             tmem_ld_wait();
             tmem_ld16(tb + 80, v1);
-            p4_chunk<P, TT, 64>(v0, e, pr, es, pacc[mbl]);
+            p4_chunk<P, TT, 64, ACT>(v0, e, pr, es, pacc[mbl]);
             tmem_ld_wait();
             tmem_ld16(tb + 96, v0);
-            p4_chunk<P, TT, 80>(v1, e, pr, es, pacc[mbl]);
+            p4_chunk<P, TT, 80, ACT>(v1, e, pr, es, pacc[mbl]);
             tmem_ld_wait();
             tmem_ld16(tb + 112, v1);
-            p4_chunk<P, TT, 96>(v0, e, pr, es, pacc[mbl]);
+            p4_chunk<P, TT, 96, ACT>(v0, e, pr, es, pacc[mbl]);
             tmem_ld_wait();
-            p4_chunk<P, TT, 112>(v1, e, pr, es, pacc[mbl]);
+            p4_chunk<P, TT, 112, ACT>(v1, e, pr, es, pacc[mbl]);
 #pragma unroll
             for (int i = 0; i < TT; ++i) {
               const int tt = g.t0 + i;
@@ -892,6 +920,18 @@ joint_bwd3_x3_kernel(const __grid_constant__ CUtensorMap tmap_e, const __grid_co
                      const BwdParams p) {
   joint_bwd3_body<P, TT, true>(tmap_e, tmap_p, p);
 }
+// relu / gelu joints, named apart for profiler traces
+#define CTCVR_BWD3_ACT(name, split, act)                                                                           \
+  template <int P, int TT>                                                                                          \
+  __global__ void __launch_bounds__(NTHREADS, 1)                                                                    \
+  name(const __grid_constant__ CUtensorMap tmap_e, const __grid_constant__ CUtensorMap tmap_p, const BwdParams p) { \
+    joint_bwd3_body<P, TT, split, act>(tmap_e, tmap_p, p);                                                          \
+  }
+CTCVR_BWD3_ACT(joint_bwd3_relu_kernel, false, ACT_RELU)
+CTCVR_BWD3_ACT(joint_bwd3_gelu_kernel, false, ACT_GELU)
+CTCVR_BWD3_ACT(joint_bwd3_x3_relu_kernel, true, ACT_RELU)
+CTCVR_BWD3_ACT(joint_bwd3_x3_gelu_kernel, true, ACT_GELU)
+#undef CTCVR_BWD3_ACT
 
 }  // namespace tc
 }  // namespace ctcvr

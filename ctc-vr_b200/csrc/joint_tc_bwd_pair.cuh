@@ -87,10 +87,10 @@ __device__ __forceinline__ void carve_bwd4(Bwd4Smem& L, uint8_t* raw, int NH, in
   L.tmem_ptr = reinterpret_cast<uint32_t*>(raw + (a - base));
 }
 
-template <int P, int TT>
-__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NTHREADS, 1)
-joint_bwd4_kernel(const __grid_constant__ CUtensorMap tmap_e, const __grid_constant__ CUtensorMap tmap_e2,
-                  const __grid_constant__ CUtensorMap tmap_p, const BwdParams p) {
+// ACT: the joint activation of the P1 producers and the P4 derivative (ACT_TANH / ACT_RELU / ACT_GELU)
+template <int P, int TT, int ACT>
+__device__ __forceinline__ void joint_bwd4_body(const CUtensorMap& tmap_e, const CUtensorMap& tmap_e2,
+                                                const CUtensorMap& tmap_p, const BwdParams& p) {
   static_assert(2 * TT * 128 <= (int)BP_ENC_REGION, "the enc rows of both tiles share one 2 KB region");
   extern __shared__ uint8_t smem_raw[];
   Bwd4Smem L;
@@ -397,10 +397,10 @@ joint_bwd4_kernel(const __grid_constant__ CUtensorMap tmap_e, const __grid_const
             else { ev = lds128(sb + e_row + ((c ^ e_sw) << 4)); pv = lds128(sb + p_row + ((c ^ p_sw) << 4)); }
             if (CTCVR_EXP & 8) { w[4 * c4 + 0] = ev.x ^ pv.y; w[4 * c4 + 1] = ev.y; w[4 * c4 + 2] = ev.z; w[4 * c4 + 3] = ev.w; }
             else {
-            w[4 * c4 + 0] = tanh_add_bf16x2_packed(ev.x, pv.x);
-            w[4 * c4 + 1] = tanh_add_bf16x2_packed(ev.y, pv.y);
-            w[4 * c4 + 2] = tanh_add_bf16x2_packed(ev.z, pv.z);
-            w[4 * c4 + 3] = tanh_add_bf16x2_packed(ev.w, pv.w);
+            w[4 * c4 + 0] = act_add_bf16x2_packed<ACT>(ev.x, pv.x);
+            w[4 * c4 + 1] = act_add_bf16x2_packed<ACT>(ev.y, pv.y);
+            w[4 * c4 + 2] = act_add_bf16x2_packed<ACT>(ev.z, pv.z);
+            w[4 * c4 + 3] = act_add_bf16x2_packed<ACT>(ev.w, pv.w);
             }
           }
           tmem_st16(tq + (uint32_t)(B_ACC_COLS + a_stg * 32 + kh * 16), w);
@@ -579,27 +579,27 @@ joint_bwd4_kernel(const __grid_constant__ CUtensorMap tmap_e, const __grid_const
             tmem_ld16(tb, v0);
             tmem_ld_wait();
             tmem_ld16(tb + 16, v1);
-            p4_chunk<P, TT, 0>(v0, e, pr, es, pacc[mb2]);
+            p4_chunk<P, TT, 0, ACT>(v0, e, pr, es, pacc[mb2]);
             tmem_ld_wait();
             tmem_ld16(tb + 32, v0);
-            p4_chunk<P, TT, 16>(v1, e, pr, es, pacc[mb2]);
+            p4_chunk<P, TT, 16, ACT>(v1, e, pr, es, pacc[mb2]);
             tmem_ld_wait();
             tmem_ld16(tb + 48, v1);
-            p4_chunk<P, TT, 32>(v0, e, pr, es, pacc[mb2]);
+            p4_chunk<P, TT, 32, ACT>(v0, e, pr, es, pacc[mb2]);
             tmem_ld_wait();
             tmem_ld16(tb + 64, v0);
-            p4_chunk<P, TT, 48>(v1, e, pr, es, pacc[mb2]);
+            p4_chunk<P, TT, 48, ACT>(v1, e, pr, es, pacc[mb2]);
             tmem_ld_wait();
             tmem_ld16(tb + 80, v1);
-            p4_chunk<P, TT, 64>(v0, e, pr, es, pacc[mb2]);
+            p4_chunk<P, TT, 64, ACT>(v0, e, pr, es, pacc[mb2]);
             tmem_ld_wait();
             tmem_ld16(tb + 96, v0);
-            p4_chunk<P, TT, 80>(v1, e, pr, es, pacc[mb2]);
+            p4_chunk<P, TT, 80, ACT>(v1, e, pr, es, pacc[mb2]);
             tmem_ld_wait();
             tmem_ld16(tb + 112, v1);
-            p4_chunk<P, TT, 96>(v0, e, pr, es, pacc[mb2]);
+            p4_chunk<P, TT, 96, ACT>(v0, e, pr, es, pacc[mb2]);
             tmem_ld_wait();
-            p4_chunk<P, TT, 112>(v1, e, pr, es, pacc[mb2]);
+            p4_chunk<P, TT, 112, ACT>(v1, e, pr, es, pacc[mb2]);
 #pragma unroll
             for (int i = 0; i < TT; ++i) {
               const int tt = zt * TT + i;
@@ -626,6 +626,18 @@ joint_bwd4_kernel(const __grid_constant__ CUtensorMap tmap_e, const __grid_const
   cluster_sync_all();                       // no MMA / multicast commit / remote arrive may target a CTA that has left
   if (warp == 2) tmem_dealloc2(tmem_base, TMEM_COLS);
 }
+
+#define CTCVR_BWD4(name, act)                                                                                      \
+  template <int P, int TT>                                                                                          \
+  __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NTHREADS, 1)                                          \
+  name(const __grid_constant__ CUtensorMap tmap_e, const __grid_constant__ CUtensorMap tmap_e2,                     \
+       const __grid_constant__ CUtensorMap tmap_p, const BwdParams p) {                                             \
+    joint_bwd4_body<P, TT, act>(tmap_e, tmap_e2, tmap_p, p);                                                        \
+  }
+CTCVR_BWD4(joint_bwd4_kernel, ACT_TANH)
+CTCVR_BWD4(joint_bwd4_relu_kernel, ACT_RELU)     // relu / gelu joints, named apart for profiler traces
+CTCVR_BWD4(joint_bwd4_gelu_kernel, ACT_GELU)
+#undef CTCVR_BWD4
 
 }  // namespace tc
 }  // namespace ctcvr

@@ -99,12 +99,14 @@ __device__ __forceinline__ void carve_fwd2(FwdSmem& L, uint8_t* raw, int NH, int
 }
 
 
-// z = tanh(e + p) in fp32 (tanhf: accurate, the build does not use fast-math) for 8 consecutive k, split into
+// z = act(e + p) in fp32 (tanhf / erff: accurate, the build does not use fast-math) for 8 consecutive k, split into
 // hi = bf16_rn(z) and lo = bf16_rn(z - hi) as packed pairs (low half = even k, the TMEM operand layout)
+template <int ACT = ACT_TANH>
 __device__ __forceinline__ void tanh_split8(const float4& e0, const float4& e1, const float4& p0, const float4& p1,
                                             uint32_t* hi, uint32_t* lo) {
-  const float z[8] = {tanhf(e0.x + p0.x), tanhf(e0.y + p0.y), tanhf(e0.z + p0.z), tanhf(e0.w + p0.w),
-                      tanhf(e1.x + p1.x), tanhf(e1.y + p1.y), tanhf(e1.z + p1.z), tanhf(e1.w + p1.w)};
+  const float z[8] = {act_f32<ACT>(e0.x + p0.x), act_f32<ACT>(e0.y + p0.y), act_f32<ACT>(e0.z + p0.z),
+                      act_f32<ACT>(e0.w + p0.w), act_f32<ACT>(e1.x + p1.x), act_f32<ACT>(e1.y + p1.y),
+                      act_f32<ACT>(e1.z + p1.z), act_f32<ACT>(e1.w + p1.w)};
 #pragma unroll
   for (int j = 0; j < 4; ++j) {
     const __nv_bfloat162 h = __floats2bfloat162_rn(z[2 * j], z[2 * j + 1]);
@@ -118,7 +120,8 @@ __device__ __forceinline__ void tanh_split8(const float4& e0, const float4& e1, 
 //   W ring   : per k-block four stages (W_hi half 0, 1, W_lo half 0, 1) from w_t = [KB][hi, lo][2][NH][64]
 //   A stages : per k-block two TMEM stages (z_hi, z_lo of its 64 k): the same 3 x 32 columns as bf16
 //   producers: read the fp32 enc / pred rows straight from global memory (L2-resident), no slab ring (warp 3 idles)
-template <bool SPLIT>
+// ACT: the joint activation (ACT_TANH / ACT_RELU / ACT_GELU), applied by the A producers.
+template <bool SPLIT, int ACT = ACT_TANH>
 __device__ __forceinline__ void joint_fwd2_body(const CUtensorMap& tmap_e, const CUtensorMap& tmap_p, const FwdParams& p) {
   extern __shared__ uint8_t smem_raw[];
   FwdSmem L;
@@ -369,8 +372,8 @@ __device__ __forceinline__ void joint_fwd2_body(const CUtensorMap& tmap_e, const
           const float4 e0 = __ldg(e4), e1 = __ldg(e4 + 1), e2 = __ldg(e4 + 2), e3 = __ldg(e4 + 3);
           const float4 p0 = __ldg(p4), p1 = __ldg(p4 + 1), p2 = __ldg(p4 + 2), p3 = __ldg(p4 + 3);
           uint32_t hi[8], lo[8];
-          tanh_split8(e0, e1, p0, p1, hi, lo);
-          tanh_split8(e2, e3, p2, p3, hi + 4, lo + 4);
+          tanh_split8<ACT>(e0, e1, p0, p1, hi, lo);
+          tanh_split8<ACT>(e2, e3, p2, p3, hi + 4, lo + 4);
           if (c == 0) {
             mbar_wait(L.a_empty(ap.stage), ap.phase ^ 1u, 8);
             mbar_wait(L.a_empty(al.stage), al.phase ^ 1u, 8);
@@ -414,10 +417,10 @@ __device__ __forceinline__ void joint_fwd2_body(const CUtensorMap& tmap_e, const
           const uint32_t c = (uint32_t)(kh * 4 + c4);
           const uint4 ev = lds128(sb + e_row + ((c ^ e_sw) << 4));
           const uint4 pv = lds128(sb + p_row + ((c ^ p_sw) << 4));
-          w[4 * c4 + 0] = tanh_add_bf16x2_packed(ev.x, pv.x);
-          w[4 * c4 + 1] = tanh_add_bf16x2_packed(ev.y, pv.y);
-          w[4 * c4 + 2] = tanh_add_bf16x2_packed(ev.z, pv.z);
-          w[4 * c4 + 3] = tanh_add_bf16x2_packed(ev.w, pv.w);
+          w[4 * c4 + 0] = act_add_bf16x2_packed<ACT>(ev.x, pv.x);
+          w[4 * c4 + 1] = act_add_bf16x2_packed<ACT>(ev.y, pv.y);
+          w[4 * c4 + 2] = act_add_bf16x2_packed<ACT>(ev.z, pv.z);
+          w[4 * c4 + 3] = act_add_bf16x2_packed<ACT>(ev.w, pv.w);
         }
         tmem_st16(tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(F_ACC_COLS + ap.stage * 32 + kh * 16), w);
         tmem_st_wait();
@@ -447,6 +450,17 @@ joint_fwd2_x3_kernel(const __grid_constant__ CUtensorMap tmap_e, const __grid_co
                      const FwdParams p) {
   joint_fwd2_body<true>(tmap_e, tmap_p, p);
 }
+// relu / gelu joints: the same kernels with the activation of the A producers swapped, named apart for profiler traces
+#define CTCVR_FWD2_ACT(name, split, act)                                                                           \
+  __global__ void __launch_bounds__(F_THREADS, 1)                                                                   \
+  name(const __grid_constant__ CUtensorMap tmap_e, const __grid_constant__ CUtensorMap tmap_p, const FwdParams p) { \
+    joint_fwd2_body<split, act>(tmap_e, tmap_p, p);                                                                 \
+  }
+CTCVR_FWD2_ACT(joint_fwd2_relu_kernel, false, ACT_RELU)
+CTCVR_FWD2_ACT(joint_fwd2_gelu_kernel, false, ACT_GELU)
+CTCVR_FWD2_ACT(joint_fwd2_x3_relu_kernel, true, ACT_RELU)
+CTCVR_FWD2_ACT(joint_fwd2_x3_gelu_kernel, true, ACT_GELU)
+#undef CTCVR_FWD2_ACT
 
 // Tile table of the forward kernel: per utterance (W/4) groups of 4 label columns x 32-frame blocks, then a
 // 2-column group x 64-frame blocks if W & 2, then a 1-column group x 128-frame blocks if W & 1 (64-frame blocks for

@@ -368,6 +368,27 @@ __device__ __forceinline__ uint32_t tanh_add_bf16x2_packed(uint32_t a, uint32_t 
   return r;
 }
 
+// act(a + b) on packed bf16 pairs for every activation: the sum is the packed bf16 add of the tanh form; relu is a packed
+// max with 0 (exact); gelu is evaluated in fp32 (erff) from the bf16 sum and rounded to bf16.
+__device__ __forceinline__ uint32_t add_bf16x2(uint32_t a, uint32_t b) {
+  uint32_t s;
+  asm("add.rn.bf16x2 %0, %1, %2;" : "=r"(s) : "r"(a), "r"(b));
+  return s;
+}
+template <int ACT>
+__device__ __forceinline__ uint32_t act_add_bf16x2_packed(uint32_t a, uint32_t b) {
+  if constexpr (ACT == ACT_TANH) {
+    return tanh_add_bf16x2_packed(a, b);
+  } else if constexpr (ACT == ACT_RELU) {
+    uint32_t r;
+    asm("max.bf16x2 %0, %1, %2;" : "=r"(r) : "r"(add_bf16x2(a, b)), "r"(0u));
+    return r;
+  } else {
+    const uint32_t s = add_bf16x2(a, b);
+    return pack_bf16(gelu_f32(__uint_as_float(s << 16)), gelu_f32(__uint_as_float(s & 0xffff0000u)));
+  }
+}
+
 // Same, pinned in program order (volatile): the producers release a slab stage right behind these - the MUFU issue
 // waits for its operands, so every load of the stage has completed by the time the arrive that follows is issued.
 // (A plain `asm` may be scheduled below the arrive, which would then overtake the loads.)

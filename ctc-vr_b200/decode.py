@@ -19,6 +19,8 @@ import torch
 
 from . import _lib
 from ._lib import DecoderWeights, call, ptr, query, stream
+from .functional import _ACT
+from .joint import joint_activation
 
 
 class PreparedDecoder:
@@ -61,6 +63,10 @@ class PreparedDecoder:
         else:   # prejoin_linear=False: identity
             P = proj_t.shape[1]
             pf_t, pf_b = torch.eye(P, device=emb.device), torch.zeros(P, device=emb.device)
+        post = _post_ffn(j)
+        if post is not None:    # post(e + p) = post(e) + W_post p: the prediction side takes W_post without its bias
+            wp = f(post.weight)
+            pf_t, pf_b = (pf_t @ wp.t()).contiguous(), (wp @ pf_b).contiguous()
         out_t, out_b = f(j.ffn_out.weight).t().contiguous(), f(j.ffn_out.bias)
         self._keep = (gate_tok, w_hh_t, w_ih_t, b_gate, proj_t, proj_b, pf_t, pf_b, out_t, out_b)
         s = DecoderWeights()
@@ -68,6 +74,7 @@ class PreparedDecoder:
                             "pred_ffn_b", "out_t", "out_b"), self._keep):
             setattr(s, name, None if t is None else t.data_ptr())
         s.V, s.H, s.L, s.P, s.D = out_t.shape[1], H, L, proj_t.shape[1], out_t.shape[0]
+        s.activation = _ACT[joint_activation(j)]
         self.struct, self._key = s, key
         return s
 
@@ -87,11 +94,20 @@ def _blank_of(model) -> int:
     return int(model.blank if hasattr(model, "blank") else model.blank_id)
 
 
+def _post_ffn(joint):
+    """The post-join linear of a joint that applies one (joint.py:64-65), else None."""
+    return joint.post_ffn if getattr(joint, "postjoin_linear", False) and getattr(joint, "post_ffn", None) is not None \
+        else None
+
+
 def _enc_proj(model, encoder_out):
     j = model.joint
     x = encoder_out.float()
     if getattr(j, "enc_ffn", None) is not None:
         x = torch.nn.functional.linear(x, j.enc_ffn.weight, j.enc_ffn.bias)
+    post = _post_ffn(j)
+    if post is not None:    # the encoder side of the folded post-join linear keeps its bias
+        x = torch.nn.functional.linear(x, post.weight.float(), post.bias.float())
     return x.contiguous()
 
 

@@ -21,6 +21,9 @@ from ._lib import call, ptr, query, stream
 F32, BF16, BF16X3 = 0, 1, 2
 _PREC = {"fp32": F32, "f32": F32, "bf16": BF16, "bf16x3": BF16X3, F32: F32, BF16: BF16, BF16X3: BF16X3}
 _PREC_NAME = {F32: "fp32", BF16: "bf16", BF16X3: "bf16x3"}
+# joint activation bits OR'ed into the precision argument (CTCVR_ACT_* of include/ctcvr.h)
+ACT_TANH, ACT_RELU, ACT_GELU = 0x000, 0x100, 0x200
+_ACT = {"tanh": ACT_TANH, "relu": ACT_RELU, "gelu": ACT_GELU}
 
 
 def _f32c(t):
@@ -37,15 +40,18 @@ def _ws(nbytes, device):
 
 class _FusedJointRnnt(torch.autograd.Function):
     @staticmethod
-    def forward(ctx, enc_proj, pred_proj, w_out, b_out, targets, t_len, u_len, blank, clamp, precision):
+    def forward(ctx, enc_proj, pred_proj, w_out, b_out, targets, t_len, u_len, blank, clamp, precision, act):
         _lib.require_cuda(enc_proj, pred_proj, w_out, b_out)
         dev = enc_proj.device
         w, b = _f32c(w_out), _f32c(b_out)
         B, T, D = enc_proj.shape
         U1 = pred_proj.shape[1]
         V = w.shape[0]
-        # bf16 activations (autocast) are consumed in place by the tensor-core path: no fp32 round trip
-        bf16_in = precision == BF16 and enc_proj.dtype == torch.bfloat16 and pred_proj.dtype == torch.bfloat16
+        # bf16 activations (autocast) are consumed in place by the tensor-core path: no fp32 round trip.  The bf16-input
+        # entry points are tanh only; other joints pass bf16 inputs through the fp32-input entry point, whose bf16 path
+        # rounds them to bf16 again (exact), so the arithmetic is the same.
+        bf16_in = precision == BF16 and act == ACT_TANH and enc_proj.dtype == torch.bfloat16 and \
+            pred_proj.dtype == torch.bfloat16
         if bf16_in:
             e, p = enc_proj.detach().contiguous(), pred_proj.detach().contiguous()
         else:
@@ -70,23 +76,23 @@ class _FusedJointRnnt(torch.autograd.Function):
         alpha, beta = torch.empty_like(lse), torch.empty_like(lse)
         costs = torch.empty((B,), dtype=torch.float32, device=dev)
         with torch.cuda.device(dev):
-            ws = _ws(query("ctcvr_joint_rnnt_fwd_ws_bytes", B, T, U1, D, V, precision), dev)
+            ws = _ws(query("ctcvr_joint_rnnt_fwd_ws_bytes", B, T, U1, D, V, precision | act), dev)
             if bf16_in:
                 call("ctcvr_joint_rnnt_fwd_bf16in", ptr(e), ptr(p), ptr(w), ptr(b), ptr(tg), ptr(tl), ptr(ul), ptr(lse),
                      ptr(lpb), ptr(lpl), B, T, U1, D, V, blank, ptr(ws), ws.numel(), stream())
             else:
                 call("ctcvr_joint_rnnt_fwd", ptr(e), ptr(p), ptr(w), ptr(b), ptr(tg), ptr(tl), ptr(ul), ptr(lse),
-                     ptr(lpb), ptr(lpl), B, T, U1, D, V, blank, precision, ptr(ws), ws.numel(), stream())
+                     ptr(lpb), ptr(lpl), B, T, U1, D, V, blank, precision | act, ptr(ws), ws.numel(), stream())
             call("ctcvr_rnnt_lattice", ptr(lpb), ptr(lpl), ptr(tl), ptr(ul), ptr(alpha), ptr(beta), ptr(costs),
                  B, T, U1, stream())
         ctx.save_for_backward(e, p, w, b, tg, tl, ul, lse, lpb, lpl, alpha, beta, costs)
-        ctx.cfg = (blank, float(clamp), precision, bf16_in)
+        ctx.cfg = (blank, float(clamp), precision, bf16_in, act, enc_proj.dtype, pred_proj.dtype)
         return costs
 
     @staticmethod
     def backward(ctx, grad_costs):
         e, p, w, b, tg, tl, ul, lse, lpb, lpl, alpha, beta, costs = ctx.saved_tensors
-        blank, clamp, precision, bf16_in = ctx.cfg
+        blank, clamp, precision, bf16_in, act, e_dtype, p_dtype = ctx.cfg
         B, T, D = e.shape
         U1, V = p.shape[1], w.shape[0]
         dev = e.device
@@ -97,7 +103,7 @@ class _FusedJointRnnt(torch.autograd.Function):
         d_p = torch.empty(p.shape, dtype=gdt, device=dev)
         d_w, d_b = torch.empty_like(w), torch.empty_like(b)
         with torch.cuda.device(dev):
-            ws = _ws(query("ctcvr_joint_rnnt_bwd_ws_bytes", B, T, U1, D, V, precision), dev)
+            ws = _ws(query("ctcvr_joint_rnnt_bwd_ws_bytes", B, T, U1, D, V, precision | act), dev)
             if bf16_in:
                 call("ctcvr_joint_rnnt_bwd_bf16in", ptr(e), ptr(p), ptr(w), ptr(b), ptr(tg), ptr(tl), ptr(ul), ptr(lse),
                      ptr(lpb), ptr(lpl), ptr(alpha), ptr(beta), ptr(costs), ptr(gc), clamp, ptr(d_e), ptr(d_p), ptr(d_w), ptr(d_b),
@@ -105,15 +111,26 @@ class _FusedJointRnnt(torch.autograd.Function):
             else:
                 call("ctcvr_joint_rnnt_bwd", ptr(e), ptr(p), ptr(w), ptr(b), ptr(tg), ptr(tl), ptr(ul), ptr(lse),
                      ptr(lpb), ptr(lpl), ptr(alpha), ptr(beta), ptr(costs), ptr(gc), clamp, ptr(d_e), ptr(d_p), ptr(d_w), ptr(d_b),
-                     B, T, U1, D, V, blank, precision, ptr(ws), ws.numel(), stream())
-        return d_e, d_p, d_w, d_b, None, None, None, None, None, None
+                     B, T, U1, D, V, blank, precision | act, ptr(ws), ws.numel(), stream())
+        if not bf16_in:                                   # gradients in the dtype of the inputs
+            d_e, d_p = d_e.to(e_dtype), d_p.to(p_dtype)
+        return d_e, d_p, d_w, d_b, None, None, None, None, None, None, None
 
 
 def fused_joint_rnnt_loss(enc_proj, pred_proj, w_out, b_out, targets, logit_lengths, target_lengths,
-                          blank: int, clamp: float = -1.0, reduction: str = "mean", precision="fp32"):
+                          blank: int, clamp: float = -1.0, reduction: str = "mean", precision="fp32",
+                          activation: str = "tanh"):
     """costs_b = RNN-T negative log-likelihood of utterance b for
-    logits = ffn_out(tanh(enc_proj[:, :, None] + pred_proj[:, None])) without materialising them.
+    logits = ffn_out(act(enc_proj[:, :, None] + pred_proj[:, None])) without materialising them.
     enc_proj [B,T,D] / pred_proj [B,U+1,D] are the enc_ffn / pred_ffn outputs (joint.py:54-55).
+    activation: 'tanh' (default), 'relu' (nn.ReLU, derivative 0 at 0) or 'gelu' (nn.GELU(), exact erf form).  A post-join
+    linear folds into the two inputs: post(e + p) = (W_post e + b_post) + W_post p.  Every precision below holds for every
+    activation; in 'bf16' the sum e + p is rounded to bf16 before the activation (gelu is then evaluated in fp32).  One
+    exception, from relu's kink: in 'bf16' on fp32 inputs, every element whose e + p lies within the bf16 rounding error
+    of 0 can land on the other side of the kink, and its derivative flips between 0 and 1.  That adds about
+    sqrt(flipped fraction) to the relative error of the gradients (measured 4.6e-2 on d_enc with 0.5-scale Gaussian
+    inputs at D = 384, where 4.6e-4 of the elements flip), on top of the 3e-2 below; a relu joint on bf16 inputs is within
+    the 3e-2 of those inputs.
 
     precision='fp32' (default) is the reference's arithmetic (loss and gradients within 1e-4 of torchaudio's);
     precision='bf16' is the explicit opt-in to the tcgen05 path (bf16 operands, fp32 accumulation, softmax and
@@ -124,8 +141,10 @@ def fused_joint_rnnt_loss(enc_proj, pred_proj, w_out, b_out, targets, logit_leng
     hi = bf16(x) and lo = bf16(x - hi) and each product is hi*hi + hi*lo + lo*hi, with tanh, d cost / d logits and the
     reductions in fp32.  Loss and gradients are within 1e-4 of the reference, like fp32; inputs are taken as fp32, and
     the shape limits and the error on other shapes are those of 'bf16'."""
+    if activation not in _ACT:
+        raise ValueError(f"fused_joint_rnnt_loss: activation must be one of {sorted(_ACT)}, got {activation!r}")
     costs = _FusedJointRnnt.apply(enc_proj, pred_proj, w_out, b_out, targets, logit_lengths, target_lengths,
-                                  int(blank), float(clamp), _PREC[precision])
+                                  int(blank), float(clamp), _PREC[precision], _ACT[activation])
     return _reduce(costs, reduction)
 
 

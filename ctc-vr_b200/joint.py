@@ -5,6 +5,7 @@ from typing import Optional
 
 import torch
 from torch import nn
+from torch.nn import functional as F
 
 from . import functional as CF
 
@@ -31,7 +32,7 @@ class _Bf16Linear(torch.autograd.Function):
     def forward(ctx, x, weight, bias):
         xb = x.reshape(-1, x.shape[-1]).to(torch.bfloat16)
         wb = weight.to(torch.bfloat16)
-        y = torch.addmm(bias.to(torch.bfloat16), xb, wb.t())
+        y = torch.addmm(bias.to(torch.bfloat16), xb, wb.t()) if bias is not None else torch.mm(xb, wb.t())
         ctx.save_for_backward(xb, wb)
         ctx.x_shape, ctx.x_dtype, ctx.w_dtype = x.shape, x.dtype, weight.dtype
         return y.reshape(*x.shape[:-1], weight.shape[0])
@@ -51,6 +52,37 @@ class _Bf16Linear(torch.autograd.Function):
         if ctx.needs_input_grad[2]:
             db = torch.mm(_ones_row(dy2.shape[0], dy2.device), dy2, out_dtype=torch.float32).reshape(-1).to(ctx.w_dtype)
         return dx, dw, db
+
+
+def joint_activation(joint) -> str:
+    """'tanh', 'relu' or 'gelu': the activation module of a TransducerJoint or of the reference's joint
+    (model/component/joint.py:20-27).  Anything else (e.g. the tanh approximation of GELU) raises: the fused kernels
+    would otherwise compute a different function."""
+    act = getattr(joint, "activation", None)
+    if isinstance(act, nn.Tanh):
+        return "tanh"
+    if isinstance(act, nn.ReLU):
+        return "relu"
+    if isinstance(act, nn.GELU) and getattr(act, "approximate", "none") == "none":
+        return "gelu"
+    raise RuntimeError(f"ctcvr_b200: the fused joint kernels compute tanh, relu or exact gelu, not {act!r}")
+
+
+def fused_joint_inputs(joint, enc_out, pred_out, linear=F.linear, pre_project: bool = True):
+    """(enc_proj, pred_proj) for the fused loss of a joint_mode='add' joint: the pre-join linears (when the joint has
+    them), then the post-join linear folded into both sides - it is linear, so
+    post(e + p) = (W_post e + b_post) + W_post p.  `linear(x, weight, bias)` runs each product (bias may be None)."""
+    if getattr(joint, "joint_mode", "add") != "add":
+        raise RuntimeError("ctcvr_b200: the fused RNN-T loss needs joint_mode='add'")
+    e, p = enc_out, pred_out
+    if pre_project and getattr(joint, "prejoin_linear", True) and joint.enc_ffn is not None and joint.pred_ffn is not None:
+        e = linear(e, joint.enc_ffn.weight, joint.enc_ffn.bias)
+        p = linear(p, joint.pred_ffn.weight, joint.pred_ffn.bias)
+    post = getattr(joint, "post_ffn", None)
+    if getattr(joint, "postjoin_linear", False) and post is not None:
+        e = linear(e, post.weight, post.bias)
+        p = linear(p, post.weight, None)
+    return e, p
 
 
 class TransducerJoint(nn.Module):
@@ -110,9 +142,17 @@ class TransducerJoint(nn.Module):
                         pre_project: bool = True):
         """joint + log-softmax + RNN-T lattice loss in one op (the seam of transducer.py:172-187).
         precision='fp32' keeps the reference's arithmetic; 'bf16' opts into the tcgen05 tensor-core path; 'bf16x3'
-        runs the tensor-core path at fp32 accuracy (the pre-projections then stay fp32, as with 'fp32')."""
+        runs the tensor-core path at fp32 accuracy (the pre-projections then stay fp32, as with 'fp32').
+        Every activation ('tanh', 'relu', 'gelu') with or without pre-join and post-join linears is fused; the post-join
+        linear folds into the two inputs (`fused_joint_inputs`).  joint_mode must be 'add'."""
+        if self.joint_mode != "add":
+            raise RuntimeError("rnnt_loss_fused: only joint_mode='add'")
         if not self.fusable:
-            raise RuntimeError("rnnt_loss_fused: only joint_mode='add', activation='tanh', postjoin_linear=False")
+            lin = _Bf16Linear.apply if precision in ("bf16", CF.BF16) and enc_out.is_cuda else F.linear
+            e, p = fused_joint_inputs(self, enc_out, pred_out, lin, pre_project)
+            return CF.fused_joint_rnnt_loss(e, p, self.ffn_out.weight, self.ffn_out.bias, targets, logit_lengths,
+                                            target_lengths, blank, clamp, reduction, precision,
+                                            activation=self.activation_name)
         if precision in ("bf16", CF.BF16) and enc_out.is_cuda:
             # bf16 path: the two pre-projections are plain library GEMMs; run them on the tensor cores too
             if pre_project and self.prejoin_linear and self.enc_ffn is not None and self.pred_ffn is not None:

@@ -93,14 +93,13 @@ def compute_rnnt_loss(self, encoder_out, encoder_out_lens, text, text_lengths, c
     joint = self.joint
     precision = getattr(self, "precision", "fp32")      # reference arithmetic unless the model opts into bf16
     from . import functional as CF
-    j_ok = getattr(joint, "prejoin_linear", True) and not getattr(joint, "postjoin_linear", False) and \
-        isinstance(getattr(joint, "activation", None), nn.Tanh)
-    if not j_ok:
-        raise RuntimeError("ctcvr_b200: fused RNN-T loss needs the add/tanh joint both reference models build")
+    from .joint import fused_joint_inputs, joint_activation
+    act = joint_activation(joint)                       # tanh / relu / exact gelu, anything else raises
+    # pre-join linears (if any), then the post-join linear folded into both sides (joint.fused_joint_inputs)
     if precision == "bf16" and encoder_out.is_cuda:
         with torch.autocast("cuda", dtype=torch.bfloat16):
-            e, p = joint.enc_ffn(encoder_out), joint.pred_ffn(predictor_out)
+            e, p = fused_joint_inputs(joint, encoder_out, predictor_out)
     else:
-        e, p = joint.enc_ffn(encoder_out), joint.pred_ffn(predictor_out)
+        e, p = fused_joint_inputs(joint, encoder_out, predictor_out)
     return CF.fused_joint_rnnt_loss(e, p, joint.ffn_out.weight, joint.ffn_out.bias, rnnt_text, t_len32, u_len32,
-                                    self.blank, clamp, "mean", precision)
+                                    self.blank, clamp, "mean", precision, activation=act)

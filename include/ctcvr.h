@@ -23,6 +23,12 @@
  *     hi = bf16(x), lo = bf16(x - hi) and each product is hi*hi + hi*lo + lo*hi (three MMAs into one
  *     fp32 accumulator); tanh, G = d cost / d logits and the reductions stay fp32.  Loss and gradients
  *     within 1e-4 of the reference, like CTCVR_F32; same shape limits and alignment as CTCVR_BF16.
+ *   - joint activation: `precision` of the fused joint entry points (and their _ws_bytes queries) carries one
+ *     CTCVR_ACT_* value OR'ed into it: z = tanh / relu / gelu(enc_proj + pred_proj) (joint.py `activation`).  0 is
+ *     tanh, so CTCVR_F32 / CTCVR_BF16 / CTCVR_BF16X3 alone keep their meaning; any other bit is an error return.  fp32
+ *     and bf16x3 form act and act' in fp32; bf16 forms h as a packed bf16 add (relu: packed max with 0; gelu: erff in
+ *     fp32 from the bf16 h).  The post-join linear of joint.py folds into enc_proj / pred_proj (it is linear):
+ *     post(e + p) = (W_post e + b_post) + W_post p.  The _bf16in entry points and ctcvr_joint_logits are tanh only.
  */
 #ifndef CTCVR_H_
 #define CTCVR_H_
@@ -37,6 +43,12 @@ extern "C" {
 #define CTCVR_F32 0
 #define CTCVR_BF16 1
 #define CTCVR_BF16X3 2
+/* joint activation z = act(enc_proj + pred_proj), OR'ed into `precision` of ctcvr_joint_rnnt_fwd / _bwd and their
+ * _ws_bytes queries (0 = tanh, so the plain precision values keep their meaning) and set in
+ * ctcvr_decoder_weights.activation */
+#define CTCVR_ACT_TANH 0x000
+#define CTCVR_ACT_RELU 0x100 /* nn.ReLU: derivative h > 0 (0 at h = 0, as torch) */
+#define CTCVR_ACT_GELU 0x200 /* nn.GELU(), exact erf form: h Phi(h), derivative Phi(h) + h phi(h) */
 
 const char* ctcvr_last_error(void);
 int ctcvr_version(void);
@@ -218,6 +230,9 @@ typedef struct {
   const float* out_t;      /* [D,V]      joint.ffn_out.weight^T */
   const float* out_b;      /* [V] */
   int V, H, L, P, D;
+  int activation;          /* joint activation: CTCVR_ACT_TANH (0) / CTCVR_ACT_RELU / CTCVR_ACT_GELU.  A post-join
+                              linear is folded in by the caller: pred_ffn_t <- pred_ffn_t W_post^T, pred_ffn_b <-
+                              W_post pred_ffn_b, and enc_proj = post_ffn(enc_ffn(encoder_out)) */
 } ctcvr_decoder_weights;
 
 /* ---- A5/A6/A6' greedy — model/component/transducer.py:22-70 (n_steps=64, fresh state),

@@ -44,7 +44,8 @@ __global__ void ctc_loss_kernel(const float* __restrict__ lp, const int64_t* __r
                                 int Sp, int blank, int zero_infinity) {
   extern __shared__ float sm[];
   const int b = blockIdx.x, s = threadIdx.x, nthr = blockDim.x;
-  const int Tb = min(in_lens[b], T), Ub = max(min(tgt_lens[b], Umax), 0);    // lengths beyond the tensors cannot index outside them
+  // lengths beyond the tensors cannot index outside them; a negative length behaves exactly like 0
+  const int Tb = max(min(in_lens[b], T), 0), Ub = max(min(tgt_lens[b], Umax), 0);
   const int S = 2 * Ub + 1;
   float* cur = sm;                  // [Sp] alpha_{t} / beta_{t} exchange
   float* ab = cur + Sp;             // [Sp] alpha+beta at time t
@@ -56,21 +57,24 @@ __global__ void ctc_loss_kernel(const float* __restrict__ lp, const int64_t* __r
   float* ga = alpha_ws + (size_t)b * T * Sp;
   float* gb = grad ? grad + (size_t)b * T * V : nullptr;
 
-  int lab = blank;
-  if (s < S && (s & 1)) lab = (int)targets[(size_t)b * Umax + (s >> 1)];
-  if ((unsigned)lab >= (unsigned)V) lab = blank;    // out-of-range label (undefined in the reference): no stray index
+  // label of odd state q; an out-of-range label (undefined in the reference) is blank: no stray index, and every
+  // rule below (skips, label chains) sees the same label the split form does
+  auto label = [&](int q) {
+    const int l = (int)targets[(size_t)b * Umax + (q >> 1)];
+    return (unsigned)l < (unsigned)V ? l : blank;
+  };
+  const int lab = (s < S && (s & 1)) ? label(s) : blank;
   bool skip_ok = false;             // may take the s-2 transition
-  if (s < S && (s & 1) && s >= 2) skip_ok = (lab != (int)targets[(size_t)b * Umax + (s >> 1) - 1]);
+  if (s < S && (s & 1) && s >= 2) skip_ok = (lab != label(s - 2));
 
   // label -> leader map, same-label chains (leader = lowest state carrying the label)
   for (int v = s; v < V; v += nthr) slot[v] = -1;
   if (s < Sp) nxt[s] = -1;
   __syncthreads();
   if (s == 0) {
-    slot[blank] = 0;                // all even states: handled by a block reduction, leader 0
+    slot[blank] = 0;                // all even states: handled by a block reduction, leader 0; odd blank states chain from 0
     for (int q = 1; q < S; q += 2) {
-      int l = (int)targets[(size_t)b * Umax + (q >> 1)];
-      if ((unsigned)l >= (unsigned)V) continue;     // out-of-range label: not tracked (its state keeps lab = blank)
+      const int l = label(q);
       if (slot[l] < 0) slot[l] = q;
       else { int p = slot[l]; while (nxt[p] >= 0) p = nxt[p]; nxt[p] = q; }
     }
@@ -116,7 +120,7 @@ __global__ void ctc_loss_kernel(const float* __restrict__ lp, const int64_t* __r
   }
   // ---- beta + gradient, t descending
   bool skip_fwd = false;           // may take the s+2 transition
-  if (s < S && (s & 1) && s + 2 < S) skip_fwd = (lab != (int)targets[(size_t)b * Umax + (s >> 1) + 1]);
+  if (s < S && (s & 1) && s + 2 < S) skip_fwd = (lab != label(s + 2));
   __syncthreads();
   float bprev = kNegInf;
   for (int t = Tb - 1; t >= 0; --t) {
@@ -144,7 +148,7 @@ __global__ void ctc_loss_kernel(const float* __restrict__ lp, const int64_t* __r
       for (int q = nxt[s]; q >= 0; q = nxt[q]) acc = log_add_exp(acc, ab[q]);
       lc[s] = acc;
     }
-    {   // blank: block log-sum-exp over even states
+    {   // blank: block log-sum-exp over even states, then the odd states labelled blank
       float m = (s < S && !(s & 1)) ? ab[s] : kNegInf;
       float wm = warp_max(m);
       if ((s & 31) == 0) red[s >> 5] = wm;
@@ -159,7 +163,9 @@ __global__ void ctc_loss_kernel(const float* __restrict__ lp, const int64_t* __r
       if (s == 0) {
         float tot = 0.f;
         for (int w = 0; w < (nthr >> 5); ++w) tot += red[w];
-        lc[0] = (bm == kNegInf) ? kNegInf : bm + logf(tot);
+        float acc = (bm == kNegInf) ? kNegInf : bm + logf(tot);
+        for (int q = nxt[0]; q >= 0; q = nxt[q]) acc = log_add_exp(acc, ab[q]);
+        lc[0] = acc;
       }
       __syncthreads();
     }
@@ -224,7 +230,8 @@ __global__ void ctc_alpha_beta_kernel(const float* __restrict__ lp, const int64_
                                       int T, int V, int Umax, int Sp, int blank, int zero_infinity) {
   extern __shared__ float sm[];
   const int b = blockIdx.x, tid = threadIdx.x, nthr = blockDim.x;
-  const int Tb = min(in_lens[b], T), Ub = max(min(tgt_lens[b], Umax), 0);    // lengths beyond the tensors cannot index outside them
+  // lengths beyond the tensors cannot index outside them; a negative length behaves exactly like 0
+  const int Tb = max(min(in_lens[b], T), 0), Ub = max(min(tgt_lens[b], Umax), 0);
   const int S = 2 * Ub + 1;
   float* sel = sm;                               // [Tb][S]  lp[t][label(s)]
   float* ca = sel + (size_t)T * S;               // [2][Sp + 4] alpha exchange, two guard cells on each side
@@ -427,7 +434,7 @@ __global__ void __launch_bounds__(128) ctc_grad_kernel(const float* __restrict__
                                                        float* __restrict__ grad, int T, int V, int Sp, int blank) {
   extern __shared__ float sm[];
   const int b = blockIdx.y, warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int Tb = min(in_lens[b], T), S = min(2 * max(tgt_lens[b], 0) + 1, Sp);
+  const int Tb = max(min(in_lens[b], T), 0), S = min(2 * max(tgt_lens[b], 0) + 1, Sp);
   int* mlab = reinterpret_cast<int*>(sm);        // [3][Sp]
   float* abw = sm + 3 * Sp + warp * Sp;          // [4][Sp] alpha + beta of the warp's row
   float* acc = sm + 7 * Sp + warp * V;           // [4][V] per-label log-sum
@@ -472,11 +479,13 @@ __global__ void __launch_bounds__(128) ctc_grad_kernel(const float* __restrict__
       }
     }
     __syncwarp();
+    // blank also labels the odd states whose target is blank (or out of range): their chain sum is acc[blank]
+    const float lc_blank_all = ctc_lse3(lc_blank, acc[blank], kCtcNeg);
     const float* lrow = lp + ((size_t)b * T + t) * V;
     for (int v = lane; v < V; v += 32) {
       const float l = lrow[v];
       float g = expf(l);
-      const float c = (v == blank) ? lc_blank : acc[v];
+      const float c = (v == blank) ? lc_blank_all : acc[v];
       if (c > -1.0e29f) g -= expf(c - l + nllb);
       grow[v] = g * scale;
     }
@@ -552,7 +561,7 @@ __global__ void __launch_bounds__(256) ctc_argmax_kernel(const float* __restrict
                                                          int32_t* __restrict__ ids, int T, int V) {
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int b = blockIdx.y, t = blockIdx.x * GREEDY_FRAMES_PER_CTA + warp;
-  if (t >= min(lens[b], T)) return;
+  if (t >= max(min(lens[b], T), 0)) return;
   const float* x = scores + ((size_t)b * T + t) * V;
   float best = kNegInf;
   int bi = V;
@@ -584,7 +593,7 @@ __global__ void __launch_bounds__(128) ctc_collapse_kernel(const int32_t* __rest
   const int lane = threadIdx.x & 31;
   const int b = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
   if (b >= B) return;
-  const int Tb = min(lens[b], T);
+  const int Tb = max(min(lens[b], T), 0);
   int32_t* row = tokens + (size_t)b * T;
   int count = 0, carry = -1;                      // carry = id of the frame in front of the group
   for (int t0 = 0; t0 < Tb; t0 += 32) {

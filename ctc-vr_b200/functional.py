@@ -260,8 +260,11 @@ class _CtcFromLogits(torch.autograd.Function):
         dev = x.device
         lp = torch.empty_like(x)
         nll = torch.empty((B,), dtype=torch.float32, device=dev)
+        if targets.dim() != 2 or targets.shape[0] != B:
+            raise ValueError(f"ctc_loss_from_logits: targets must be [B, Umax] = [{B}, Umax] (padded), got "
+                             f"{list(targets.shape)}; concatenated 1-D targets are not supported")
         tg = targets.detach().to(device=dev, dtype=torch.int64).contiguous()
-        Umax = tg.shape[1] if tg.dim() == 2 else 0
+        Umax = tg.shape[1]
         il, tl = _i32c(in_lens, dev), _i32c(tgt_lens, dev)
         grad = torch.empty_like(x) if logits.requires_grad else None
         with torch.cuda.device(dev):
@@ -283,7 +286,11 @@ def ctc_loss_from_logits(logits, targets, input_lengths, target_lengths, blank: 
                          zero_infinity: bool = True):
     """F.log_softmax(logits, -1) followed by nn.CTCLoss(blank, reduction, zero_infinity) on [B,T,V] logits.
     Returns (loss, log_probs [B,T,V]).  reduction semantics are ATen's: 'mean' divides each nll by
-    clamp_min(target_length, 1) and averages over the batch."""
+    clamp_min(target_length, 1) and averages over the batch.
+    targets are padded [B, Umax] (ValueError otherwise); Umax <= 511.  Values the reference leaves undefined are
+    defined here and cannot index outside the tensors: lengths are clamped to [0, T] and [0, Umax], so a negative
+    input length behaves exactly like 0 (cost inf, 0 under zero_infinity, when the target is not empty; zero
+    gradient), and a label outside [0, V) behaves exactly like `blank`."""
     _lib.require_cuda(logits)
     nll, lp = _CtcFromLogits.apply(logits, targets, input_lengths, target_lengths, int(blank), bool(zero_infinity))
     if reduction == "sum":

@@ -198,7 +198,9 @@ int ctcvr_rnnt_loss_dense(const float* logits, const int32_t* targets, const int
  * ctcvr_log_softmax: y[r,:] = log_softmax(x[r,:]) over rows x V.
  * ctcvr_ctc_loss: log_probs [B,T,V]; targets [B,Umax] int64 (as the reference passes them);
  * nll [B] (inf -> 0 when zero_infinity); grad_logits [B,T,V] (may be NULL) = d nll_b/d logits
- * scaled by grad_scale[b]; ws: ctcvr_ctc_loss_ws_bytes. */
+ * scaled by grad_scale[b]; ws: ctcvr_ctc_loss_ws_bytes.  Umax <= 511.  in_lens are clamped to
+ * [0, T] and tgt_lens to [0, Umax]: a negative length behaves exactly like 0.  A label outside
+ * [0, V) behaves exactly like blank, in the cost and the gradient, whichever kernel runs. */
 int ctcvr_log_softmax(const float* x, float* y, long rows, int V, void* stream);
 size_t ctcvr_ctc_loss_ws_bytes(int B, int T, int Umax);
 int ctcvr_ctc_loss(const float* log_probs, const int64_t* targets, const int32_t* in_lens,

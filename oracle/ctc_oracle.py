@@ -68,7 +68,7 @@ def ctc_loss_restated(log_probs: np.ndarray, targets: np.ndarray, in_lens, tgt_l
                     a = al[t - 1, s]
                     if s >= 1:
                         a = lae(a, al[t - 1, s - 1])
-                    if s >= 2 and lab[s] != blank and lab[s] != lab[s - 2]:
+                    if s >= 2 and lab[s] != lab[s - 2]:
                         a = lae(a, al[t - 1, s - 2])
                     al[t, s] = a + lp[t, lab[s]] if a != ninf else ninf
             be[Tb - 1, S - 1] = lp[Tb - 1, lab[S - 1]]
@@ -79,7 +79,7 @@ def ctc_loss_restated(log_probs: np.ndarray, targets: np.ndarray, in_lens, tgt_l
                     a = be[t + 1, s]
                     if s + 1 < S:
                         a = lae(a, be[t + 1, s + 1])
-                    if s + 2 < S and lab[s] != blank and lab[s] != lab[s + 2]:
+                    if s + 2 < S and lab[s] != lab[s + 2]:
                         a = lae(a, be[t + 1, s + 2])
                     be[t, s] = a + lp[t, lab[s]] if a != ninf else ninf
             ll = al[Tb - 1, S - 1]

@@ -91,6 +91,39 @@ def test_ctc_restated_matches_reference_heads():
         assert nll[2] == 0.0 and np.all(g[2] == 0)            # infeasible -> zero_infinity
 
 
+def test_ctc_restated_matches_aten_with_blank_targets():
+    """The restatement against torch's ctc_loss in fp64 on targets equal to blank, where l' has odd states labelled
+    blank: ATen allows the skip into such a state from the label two states back (and out of it two states on), and
+    the gradient's blank column gathers them with the even states.  Also repeats, an empty target, an infeasible one.
+
+    One exception: on the last frame ATen sets, rather than adds, the entry of the last target ("a blank and a
+    non-blank"), so when that target is blank its gradient drops the final blank state.  There the restatement is held
+    to central differences of ATen's cost instead."""
+    g = torch.Generator().manual_seed(8)
+    B, Tm, V, blank = 5, 9, 6, 2
+    logits = 2.0 * torch.randn(B, Tm, V, generator=g, dtype=torch.float64)
+    ys = torch.tensor([[2, 4, 1, 2], [4, 2, 2, 1], [2, 2, 2, 2], [3, 3, 0, 0], [1, 5, 1, 4]])
+    hl, yl = torch.tensor([9, 7, 9, 9, 3]), torch.tensor([4, 4, 4, 0, 4])
+
+    def aten(x):
+        return torch.nn.functional.ctc_loss(x.log_softmax(2).transpose(0, 1), ys, hl, yl, blank=blank,
+                                            reduction="none", zero_infinity=True)
+    x = logits.clone().requires_grad_(True)
+    want = aten(x)
+    want.sum().backward()
+    nll, grad = CO.ctc_loss_restated(logits.log_softmax(2).numpy(), ys.numpy(), hl.numpy(), yl.numpy(), blank)
+    assert want[4].item() == 0.0 and nll[4] == 0.0 and np.all(grad[4] == 0)      # 3 frames for 4 labels
+    np.testing.assert_allclose(nll, want.detach().numpy(), rtol=1e-12)
+    ag = x.grad.numpy().copy()
+    for b in (0, 2):                                  # last target blank: central differences on the last frame
+        t = int(hl[b]) - 1
+        for v in range(V):
+            e = torch.zeros_like(logits)
+            e[b, t, v] = 1e-6
+            ag[b, t, v] = float(aten(logits + e)[b] - aten(logits - e)[b]) / 2e-6
+    np.testing.assert_allclose(grad, ag, rtol=1e-6, atol=1e-9)
+
+
 def test_example2_known_answers():
     """3.ipynb:87,159 and 3_v2.ipynb:150 record the frame argmax / collapsed ids of utts 0,1."""
     fx = load_golden("example2.npz")

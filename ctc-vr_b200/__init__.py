@@ -11,12 +11,12 @@ from .ctc import CTC, OnlineCTC  # noqa: F401
 from .evaluate import calculate_cer, calculate_cer_batch  # noqa: F401
 from .decode import (BeamHypothesis, OnlineBeamState, basic_greedy_search, beam_chunk_online, beam_search_batch,  # noqa: F401
                      greedy_batch, greedy_chunk, prefix_beam_search, prefix_beam_search_batch)
-from .functional import (ctc_greedy_search as ctc_greedy_hyps, ctc_loss_from_logits, fused_joint_rnnt_loss,  # noqa: F401
-                         joint_logits, rnnt_loss)
+from .functional import (ctc_forced_align, ctc_greedy_search as ctc_greedy_hyps, ctc_loss_from_logits,  # noqa: F401
+                         fused_joint_rnnt_loss, joint_logits, rnnt_forced_align, rnnt_loss, rnnt_viterbi)
 from .graph import BucketedJointRnntStep, GraphedJointRnntStep  # noqa: F401
 from .joint import TransducerJoint  # noqa: F401
 from .predictor import RNNPredictor  # noqa: F401
 from .search import DecodeResult, ctc_greedy_search, ctc_prefix_beam_search  # noqa: F401
-from .transducer import Transducer, add_blank  # noqa: F401
+from .transducer import Transducer, add_blank, compute_rnnt_alignment  # noqa: F401
 
 __version__ = "0.1.0"

@@ -58,6 +58,10 @@ _SIGS = {
     "ctcvr_ctc_loss_ws_bytes": (Z, [I, I, I]),
     "ctcvr_ctc_loss": (I, [P, P, P, P, P, P, P, I, I, I, I, I, I, P, Z, P]),
     "ctcvr_ctc_greedy": (I, [P, P, P, P, I, I, I, I, P]),
+    "ctcvr_rnnt_viterbi_ws_bytes": (Z, [I, I, I]),
+    "ctcvr_rnnt_viterbi": (I, [P, P, P, P, P, P, P, I, I, I, P, Z, P]),
+    "ctcvr_ctc_viterbi_ws_bytes": (Z, [I, I, I]),
+    "ctcvr_ctc_viterbi": (I, [P, P, P, P, P, P, P, P, I, I, I, I, I, P, Z, P]),
     "ctcvr_rnnt_greedy_ws_bytes": (Z, [P, I]),
     "ctcvr_rnnt_greedy": (I, [P, P, P, P, P, P, P, P, I, I, I, I, I, P, Z, P]),
     "ctcvr_rnnt_beam_state_bytes": (Z, [P, I, I, I]),

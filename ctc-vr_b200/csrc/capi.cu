@@ -44,6 +44,12 @@ size_t ctc_loss_ws_bytes(int, int, int);
 int ctc_loss(const float*, const int64_t*, const int32_t*, const int32_t*, const float*, float*, float*, int, int, int,
              int, int, int, void*, size_t, cudaStream_t);
 int ctc_greedy(const float*, const int32_t*, int32_t*, int32_t*, int, int, int, int, cudaStream_t);
+size_t rnnt_viterbi_ws_bytes(int, int, int);
+int rnnt_viterbi(const float*, const float*, const int32_t*, const int32_t*, int32_t*, float*, float*, int, int, int, void*,
+                 size_t, cudaStream_t);
+size_t ctc_viterbi_ws_bytes(int, int, int);
+int ctc_viterbi(const float*, const int64_t*, const int32_t*, const int32_t*, int32_t*, float*, float*, int32_t*, int, int,
+                int, int, int, void*, size_t, cudaStream_t);
 int rnnt_greedy(const ctcvr_decoder_weights&, const float*, const int32_t*, float*, float*, int32_t*, int32_t*,
                 int32_t*, int, int, int, int, int, cudaStream_t);
 size_t rnnt_beam_state_bytes(const ctcvr_decoder_weights&, int, int, int);
@@ -321,6 +327,35 @@ int ctcvr_ctc_greedy(const float* scores, const int32_t* lens, int32_t* out_toke
                      int V, int blank, void* stream) {
   CTCVR_REQUIRE(B >= 0 && T > 0 && V > 0 && scores && lens && out_tokens && out_lens, "ctc_greedy: bad arguments");
   return ctc_greedy(scores, lens, out_tokens, out_lens, B, T, V, blank, ST(stream));
+}
+
+size_t ctcvr_rnnt_viterbi_ws_bytes(int B, int T, int U1) {
+  return (B > 0 && T > 0 && U1 > 0) ? rnnt_viterbi_ws_bytes(B, T, U1) : 0;
+}
+
+int ctcvr_rnnt_viterbi(const float* lp_blank, const float* lp_label, const int32_t* t_len, const int32_t* u_len,
+                       int32_t* frames, float* token_logprobs, float* scores, int B, int T, int U1, void* ws,
+                       size_t ws_bytes, void* stream) {
+  CTCVR_REQUIRE(B > 0 && T > 0 && U1 > 0, "rnnt_viterbi: bad dims B=%d T=%d U1=%d", B, T, U1);
+  CTCVR_REQUIRE(lp_blank && lp_label && t_len && u_len && scores && (U1 == 1 || (frames && token_logprobs)),
+                "rnnt_viterbi: NULL pointer");
+  return rnnt_viterbi(lp_blank, lp_label, t_len, u_len, frames, token_logprobs, scores, B, T, U1, ws, ws_bytes,
+                      ST(stream));
+}
+
+size_t ctcvr_ctc_viterbi_ws_bytes(int B, int T, int Umax) {
+  return (B > 0 && T > 0 && Umax >= 0) ? ctc_viterbi_ws_bytes(B, T, Umax) : 0;
+}
+
+int ctcvr_ctc_viterbi(const float* log_probs, const int64_t* targets, const int32_t* in_lens, const int32_t* tgt_lens,
+                      int32_t* labels, float* frame_logprobs, float* scores, int32_t* spans, int B, int T, int V,
+                      int Umax, int blank, void* ws, size_t ws_bytes, void* stream) {
+  CTCVR_REQUIRE(B > 0 && T > 0 && V > 0 && Umax >= 0, "ctc_viterbi: bad dims B=%d T=%d V=%d Umax=%d", B, T, V, Umax);
+  CTCVR_REQUIRE(log_probs && in_lens && tgt_lens && labels && frame_logprobs && scores && (Umax == 0 || (targets && spans)),
+                "ctc_viterbi: NULL pointer");
+  CTCVR_REQUIRE(blank >= 0 && blank < V, "ctc_viterbi: blank %d must be within [0, %d)", blank, V);
+  return ctc_viterbi(log_probs, targets, in_lens, tgt_lens, labels, frame_logprobs, scores, spans, B, T, V, Umax, blank,
+                     ws, ws_bytes, ST(stream));
 }
 
 size_t ctcvr_rnnt_greedy_ws_bytes(const ctcvr_decoder_weights* w, int N) { (void)w; (void)N; return 256; }

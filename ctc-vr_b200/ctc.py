@@ -30,6 +30,12 @@ class CTC(torch.nn.Module):
     def log_softmax(self, hs_pad):
         return CF.log_softmax_rows(self.ctc_lo(hs_pad))
 
+    @torch.no_grad()
+    def forced_align(self, hs_pad, hlens, ys_pad, ys_lens):
+        """Best CTC alignment of ys_pad [B,Umax] on log_softmax(ctc_lo(hs_pad)) (no dropout):
+        functional.ctc_forced_align -> (labels [B,T], frame_logprobs [B,T], scores [B], spans [B,Umax,2])."""
+        return CF.ctc_forced_align(self.log_softmax(hs_pad), ys_pad, hlens, ys_lens, self.blank_id)
+
     def argmax(self, hs_pad):
         return torch.argmax(self.ctc_lo(hs_pad), dim=2)
 
@@ -47,6 +53,12 @@ class OnlineCTC(torch.nn.Module):
 
     def log_softmax(self, hs_pad):
         return CF.log_softmax_rows(self.ctc_lo(hs_pad))
+
+    @torch.no_grad()
+    def forced_align(self, hs_pad, hlens, ys_pad, ys_lens):
+        """Best CTC alignment of ys_pad [B,Umax] on log_softmax(ctc_lo(hs_pad)) (no dropout):
+        functional.ctc_forced_align -> (labels [B,T], frame_logprobs [B,T], scores [B], spans [B,Umax,2])."""
+        return CF.ctc_forced_align(self.log_softmax(hs_pad), ys_pad, hlens, ys_lens, self.blank_id)
 
     def argmax(self, hs_pad):
         return torch.argmax(self.ctc_lo(hs_pad), dim=2)

@@ -10,6 +10,9 @@
   joint_logits           — dense TransducerJoint tail (model/component/joint.py:57-68).
   lstm_sequence          — one layer of the predictor's nn.LSTM over a whole label sequence, forward and backward
                            (model/component/predictor.py:58, SURVEY.md §8f row 2).
+  rnnt_viterbi / rnnt_forced_align / ctc_forced_align
+                         — batched forced alignment: the best path of a known transcript through the RNN-T lattice
+                           (on the fused joint's log-probs) or the CTC trellis, with per-token frames / spans.
 """
 from __future__ import annotations
 
@@ -38,51 +41,63 @@ def _ws(nbytes, device):
     return torch.empty(max(int(nbytes), 256), dtype=torch.uint8, device=device)
 
 
+def _joint_fwd(enc_proj, pred_proj, w_out, b_out, targets, t_len, u_len, blank, precision, act,
+               op="fused_joint_rnnt_loss"):
+    """The fused joint forward (`ctcvr_joint_rnnt_fwd` / `_bf16in`) with the fused loss's input handling and errors.
+    Returns the kernel inputs (e, p, w, b, tg, tl, ul), whether the bf16-input entry point ran, and lse / lp_blank /
+    lp_label [B,T,U1]."""
+    _lib.require_cuda(enc_proj, pred_proj, w_out, b_out)
+    dev = enc_proj.device
+    w, b = _f32c(w_out), _f32c(b_out)
+    B, T, D = enc_proj.shape
+    U1 = pred_proj.shape[1]
+    V = w.shape[0]
+    # bf16 activations (autocast) are consumed in place by the tensor-core path: no fp32 round trip.  The bf16-input
+    # entry points are tanh only; other joints pass bf16 inputs through the fp32-input entry point, whose bf16 path
+    # rounds them to bf16 again (exact), so the arithmetic is the same.
+    bf16_in = precision == BF16 and act == ACT_TANH and enc_proj.dtype == torch.bfloat16 and \
+        pred_proj.dtype == torch.bfloat16
+    if bf16_in:
+        e, p = enc_proj.detach().contiguous(), pred_proj.detach().contiguous()
+    else:
+        e, p = _f32c(enc_proj), _f32c(pred_proj)
+    if p.shape[0] != B or p.shape[2] != D or w.shape[1] != D or b.shape[0] != V:
+        raise RuntimeError(f"{op}: inconsistent shapes")
+    tg = _i32c(targets, dev)
+    if tg.dim() != 2 or tg.shape[0] != B or tg.shape[1] != U1 - 1:
+        raise RuntimeError(f"{op}: targets must be [B, U] with U == pred_out.size(1) - 1")
+    tl, ul = _i32c(t_len, dev), _i32c(u_len, dev)
+    if tl.dim() != 1 or ul.dim() != 1 or tl.shape[0] != B or ul.shape[0] != B:
+        raise RuntimeError(f"{op}: logit_lengths / target_lengths must be [B]")
+    if not (0 <= blank < V):
+        raise RuntimeError(f"{op}: blank must be within [0, vocab)")
+    # Length / label VALUES are not read back (that would be a host sync in the training step): the kernels clamp
+    # lengths to the tensor extents and treat a label outside [0, V) as blank, so bad values cannot fault the GPU.
+    if precision in (BF16, BF16X3) and not bool(query("ctcvr_joint_tc_supported", U1, D, V)):
+        raise RuntimeError(f"{op}: precision='{_PREC_NAME[precision]}' needs D % 128 == 0, D <= 512, "
+                           f"V <= 416 and U+1 <= 128 (got D={D}, V={V}, U+1={U1}); use precision='fp32' for this shape")
+    lse = torch.empty((B, T, U1), dtype=torch.float32, device=dev)
+    lpb, lpl = torch.empty_like(lse), torch.empty_like(lse)
+    with torch.cuda.device(dev):
+        ws = _ws(query("ctcvr_joint_rnnt_fwd_ws_bytes", B, T, U1, D, V, precision | act), dev)
+        if bf16_in:
+            call("ctcvr_joint_rnnt_fwd_bf16in", ptr(e), ptr(p), ptr(w), ptr(b), ptr(tg), ptr(tl), ptr(ul), ptr(lse),
+                 ptr(lpb), ptr(lpl), B, T, U1, D, V, blank, ptr(ws), ws.numel(), stream())
+        else:
+            call("ctcvr_joint_rnnt_fwd", ptr(e), ptr(p), ptr(w), ptr(b), ptr(tg), ptr(tl), ptr(ul), ptr(lse),
+                 ptr(lpb), ptr(lpl), B, T, U1, D, V, blank, precision | act, ptr(ws), ws.numel(), stream())
+    return (e, p, w, b, tg, tl, ul), bf16_in, lse, lpb, lpl
+
+
 class _FusedJointRnnt(torch.autograd.Function):
     @staticmethod
     def forward(ctx, enc_proj, pred_proj, w_out, b_out, targets, t_len, u_len, blank, clamp, precision, act):
-        _lib.require_cuda(enc_proj, pred_proj, w_out, b_out)
-        dev = enc_proj.device
-        w, b = _f32c(w_out), _f32c(b_out)
-        B, T, D = enc_proj.shape
-        U1 = pred_proj.shape[1]
-        V = w.shape[0]
-        # bf16 activations (autocast) are consumed in place by the tensor-core path: no fp32 round trip.  The bf16-input
-        # entry points are tanh only; other joints pass bf16 inputs through the fp32-input entry point, whose bf16 path
-        # rounds them to bf16 again (exact), so the arithmetic is the same.
-        bf16_in = precision == BF16 and act == ACT_TANH and enc_proj.dtype == torch.bfloat16 and \
-            pred_proj.dtype == torch.bfloat16
-        if bf16_in:
-            e, p = enc_proj.detach().contiguous(), pred_proj.detach().contiguous()
-        else:
-            e, p = _f32c(enc_proj), _f32c(pred_proj)
-        if p.shape[0] != B or p.shape[2] != D or w.shape[1] != D or b.shape[0] != V:
-            raise RuntimeError("fused_joint_rnnt_loss: inconsistent shapes")
-        tg = _i32c(targets, dev)
-        if tg.dim() != 2 or tg.shape[0] != B or tg.shape[1] != U1 - 1:
-            raise RuntimeError("fused_joint_rnnt_loss: targets must be [B, U] with U == pred_out.size(1) - 1")
-        tl, ul = _i32c(t_len, dev), _i32c(u_len, dev)
-        if tl.dim() != 1 or ul.dim() != 1 or tl.shape[0] != B or ul.shape[0] != B:
-            raise RuntimeError("fused_joint_rnnt_loss: logit_lengths / target_lengths must be [B]")
-        if not (0 <= blank < V):
-            raise RuntimeError("fused_joint_rnnt_loss: blank must be within [0, vocab)")
-        # Length / label VALUES are not read back (that would be a host sync in the training step): the kernels clamp
-        # lengths to the tensor extents and treat a label outside [0, V) as blank, so bad values cannot fault the GPU.
-        if precision in (BF16, BF16X3) and not bool(query("ctcvr_joint_tc_supported", U1, D, V)):
-            raise RuntimeError(f"fused_joint_rnnt_loss: precision='{_PREC_NAME[precision]}' needs D % 128 == 0, D <= 512, "
-                               f"V <= 416 and U+1 <= 128 (got D={D}, V={V}, U+1={U1}); use precision='fp32' for this shape")
-        lse = torch.empty((B, T, U1), dtype=torch.float32, device=dev)
-        lpb, lpl = torch.empty_like(lse), torch.empty_like(lse)
+        (e, p, w, b, tg, tl, ul), bf16_in, lse, lpb, lpl = _joint_fwd(enc_proj, pred_proj, w_out, b_out, targets, t_len,
+                                                                      u_len, blank, precision, act)
+        B, T, U1 = lse.shape
         alpha, beta = torch.empty_like(lse), torch.empty_like(lse)
-        costs = torch.empty((B,), dtype=torch.float32, device=dev)
-        with torch.cuda.device(dev):
-            ws = _ws(query("ctcvr_joint_rnnt_fwd_ws_bytes", B, T, U1, D, V, precision | act), dev)
-            if bf16_in:
-                call("ctcvr_joint_rnnt_fwd_bf16in", ptr(e), ptr(p), ptr(w), ptr(b), ptr(tg), ptr(tl), ptr(ul), ptr(lse),
-                     ptr(lpb), ptr(lpl), B, T, U1, D, V, blank, ptr(ws), ws.numel(), stream())
-            else:
-                call("ctcvr_joint_rnnt_fwd", ptr(e), ptr(p), ptr(w), ptr(b), ptr(tg), ptr(tl), ptr(ul), ptr(lse),
-                     ptr(lpb), ptr(lpl), B, T, U1, D, V, blank, precision | act, ptr(ws), ws.numel(), stream())
+        costs = torch.empty((B,), dtype=torch.float32, device=lse.device)
+        with torch.cuda.device(lse.device):
             call("ctcvr_rnnt_lattice", ptr(lpb), ptr(lpl), ptr(tl), ptr(ul), ptr(alpha), ptr(beta), ptr(costs),
                  B, T, U1, stream())
         ctx.save_for_backward(e, p, w, b, tg, tl, ul, lse, lpb, lpl, alpha, beta, costs)
@@ -458,6 +473,88 @@ def lstm_sequence(x, w_ih, w_hh, b_ih, b_hh, h0, c0):
     biases [4H] (or both None), h0 / c0 [B,H].  Returns (out [B,U1,H], h_n [B,H], c_n [B,H]) in fp32, differentiable
     in every argument.  This is the reference predictor's recurrence (model/component/predictor.py:58)."""
     return _LstmSeq.apply(x, w_ih, w_hh, b_ih, b_hh, h0, c0)
+
+
+def _len_check(op, B, *lens):
+    for t in lens:
+        if t.dim() != 1 or t.shape[0] != B:
+            raise RuntimeError(f"{op}: lengths must be [B] = [{B}]")
+
+
+@torch.no_grad()
+def rnnt_viterbi(lp_blank, lp_label, logit_lengths, target_lengths):
+    """Best path through the RNN-T lattice of lp_blank / lp_label [B,T,U+1] (fp32, the layout the fused forward writes):
+    delta(0,0) = 0, delta(t,u) = max(delta(t-1,u) + lp_blank(t-1,u), delta(t,u-1) + lp_label(t,u-1)).
+    Returns (frames [B,U] int32: the frame at which label u is emitted, non-decreasing, -1 beyond U_b;
+    token_logprobs [B,U] fp32: lp_label at that cell, 0 beyond U_b; scores [B] fp32: the path's log-probability).
+    An exact tie takes the blank predecessor, so a label goes to the earliest frame among equal paths.  Lengths are
+    clamped to [0, T] / [0, U]; an utterance without frames (or whose best path crosses a -inf log-prob) gets score
+    -inf and frames -1.  No host sync: capturable in a CUDA graph."""
+    _lib.require_cuda(lp_blank, lp_label)
+    lpb, lpl = _f32c(lp_blank), _f32c(lp_label)
+    if lpb.dim() != 3 or lpl.shape != lpb.shape:
+        raise RuntimeError("rnnt_viterbi: lp_blank and lp_label must both be [B, T, U+1]")
+    B, T, U1 = lpb.shape
+    dev = lpb.device
+    tl, ul = _i32c(logit_lengths, dev), _i32c(target_lengths, dev)
+    _len_check("rnnt_viterbi", B, tl, ul)
+    frames = torch.empty((B, U1 - 1), dtype=torch.int32, device=dev)
+    tok = torch.empty((B, U1 - 1), dtype=torch.float32, device=dev)
+    scores = torch.empty((B,), dtype=torch.float32, device=dev)
+    with torch.cuda.device(dev):
+        ws = _ws(query("ctcvr_rnnt_viterbi_ws_bytes", B, T, U1), dev)
+        call("ctcvr_rnnt_viterbi", ptr(lpb), ptr(lpl), ptr(tl), ptr(ul), ptr(frames), ptr(tok), ptr(scores), B, T, U1,
+             ptr(ws), ws.numel(), stream())
+    return frames, tok, scores
+
+
+@torch.no_grad()
+def rnnt_forced_align(enc_proj, pred_proj, w_out, b_out, targets, logit_lengths, target_lengths, blank: int,
+                      precision="fp32", activation: str = "tanh"):
+    """Forced alignment of `targets` [B,U] through the fused joint: the forward of `fused_joint_rnnt_loss` (same inputs,
+    precisions, activations and errors; the logits never reach HBM) followed by `rnnt_viterbi` on its log-probs.
+    Returns (frames [B,U] int32, token_logprobs [B,U] fp32, scores [B] fp32) as `rnnt_viterbi`; scores <= -cost of the
+    loss on the same inputs (one path against the sum over all of them)."""
+    if activation not in _ACT:
+        raise ValueError(f"rnnt_forced_align: activation must be one of {sorted(_ACT)}, got {activation!r}")
+    (_, _, _, _, _, tl, ul), _, _, lpb, lpl = _joint_fwd(enc_proj, pred_proj, w_out, b_out, targets, logit_lengths,
+                                                         target_lengths, int(blank), _PREC[precision],
+                                                         _ACT[activation], op="rnnt_forced_align")
+    return rnnt_viterbi(lpb, lpl, tl, ul)
+
+
+@torch.no_grad()
+def ctc_forced_align(log_probs, targets, input_lengths, target_lengths, blank: int):
+    """Batched CTC forced alignment (torchaudio.functional.forced_align + merge_tokens for a whole padded batch).
+    log_probs [B,T,V] fp32, targets [B,Umax] padded (Umax <= 511).  Returns (labels [B,T] int32: per frame the blank or
+    the label of the best path, -1 for t >= T_b; frame_logprobs [B,T] fp32: its log-prob, 0 for t >= T_b; scores [B];
+    spans [B,Umax,2] int32: first frame and last frame + 1 of each target token, -1 beyond U_b).  An exact tie takes
+    the smaller jump, and between the two end states the final blank.  Lengths are clamped to [0, T] / [0, Umax] and a
+    label outside [0, V) acts as blank, as in `ctc_loss_from_logits`.  An utterance without a path (T_b = 0, or fewer
+    frames than labels plus repeated neighbours) gets score -inf and -1 everywhere.  No host sync."""
+    _lib.require_cuda(log_probs)
+    lp = _f32c(log_probs)
+    if lp.dim() != 3:
+        raise RuntimeError("ctc_forced_align: log_probs must be [B, T, V]")
+    B, T, V = lp.shape
+    dev = lp.device
+    if targets.dim() != 2 or targets.shape[0] != B:
+        raise ValueError(f"ctc_forced_align: targets must be [B, Umax] = [{B}, Umax] (padded), got {list(targets.shape)}")
+    if not (0 <= blank < V):
+        raise RuntimeError("ctc_forced_align: blank must be within [0, vocab)")
+    tg = targets.detach().to(device=dev, dtype=torch.int64).contiguous()
+    Umax = tg.shape[1]
+    il, tl = _i32c(input_lengths, dev), _i32c(target_lengths, dev)
+    _len_check("ctc_forced_align", B, il, tl)
+    labels = torch.empty((B, T), dtype=torch.int32, device=dev)
+    frame_lp = torch.empty((B, T), dtype=torch.float32, device=dev)
+    scores = torch.empty((B,), dtype=torch.float32, device=dev)
+    spans = torch.empty((B, Umax, 2), dtype=torch.int32, device=dev)
+    with torch.cuda.device(dev):
+        ws = _ws(query("ctcvr_ctc_viterbi_ws_bytes", B, T, Umax), dev)
+        call("ctcvr_ctc_viterbi", ptr(lp), ptr(tg), ptr(il), ptr(tl), ptr(labels), ptr(frame_lp), ptr(scores), ptr(spans),
+             B, T, V, Umax, int(blank), ptr(ws), ws.numel(), stream())
+    return labels, frame_lp, scores, spans
 
 
 def ctc_greedy_search(scores, lens, blank: int):

@@ -164,3 +164,14 @@ class TransducerJoint(nn.Module):
             e, p = self.project(enc_out, pred_out, pre_project)
         return CF.fused_joint_rnnt_loss(e, p, self.ffn_out.weight, self.ffn_out.bias, targets, logit_lengths,
                                         target_lengths, blank, clamp, reduction, precision)
+
+    @torch.no_grad()
+    def forced_align(self, enc_out, pred_out, targets, logit_lengths, target_lengths, blank: int,
+                     precision: str = "fp32", pre_project: bool = True):
+        """Forced alignment of `targets` [B,U] through this joint (functional.rnnt_forced_align): the inputs go through
+        the same pre-join / post-join handling as `rnnt_loss_fused` (every activation, joint_mode='add').  Returns
+        (frames [B,U] int32, token_logprobs [B,U], scores [B])."""
+        lin = _Bf16Linear.apply if precision in ("bf16", CF.BF16) and enc_out.is_cuda else F.linear
+        e, p = fused_joint_inputs(self, enc_out, pred_out, lin, pre_project)
+        return CF.rnnt_forced_align(e, p, self.ffn_out.weight, self.ffn_out.bias, targets, logit_lengths, target_lengths,
+                                    blank, precision, activation=self.activation_name)

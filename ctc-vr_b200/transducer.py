@@ -103,3 +103,26 @@ def compute_rnnt_loss(self, encoder_out, encoder_out_lens, text, text_lengths, c
         e, p = fused_joint_inputs(joint, encoder_out, predictor_out)
     return CF.fused_joint_rnnt_loss(e, p, joint.ffn_out.weight, joint.ffn_out.bias, rnnt_text, t_len32, u_len32,
                                     self.blank, clamp, "mean", precision, activation=act)
+
+
+@torch.no_grad()
+def compute_rnnt_alignment(self, encoder_out, encoder_out_lens, text, text_lengths):
+    """Forced alignment of `text` with the same prologue, predictor and joint as `compute_rnnt_loss` (works on the
+    reference's own Transducer instance too).  Returns (frames [B,U] int32: the encoder frame of each token, -1 beyond
+    its length; token_logprobs [B,U]; scores [B]: the best path's log-probability)."""
+    if not text.is_cuda:
+        raise RuntimeError("ctcvr_b200 ops run on CUDA (B200) tensors only; there is no CPU path")
+    ys_in_pad, rnnt_text, t_len32, u_len32 = rnnt_prologue(text, text_lengths, encoder_out_lens, self.blank, self.ignore_id)
+    predictor_out = self.predictor(ys_in_pad)
+    joint = self.joint
+    precision = getattr(self, "precision", "fp32")
+    from . import functional as CF
+    from .joint import fused_joint_inputs, joint_activation
+    act = joint_activation(joint)
+    if precision == "bf16" and encoder_out.is_cuda:
+        with torch.autocast("cuda", dtype=torch.bfloat16):
+            e, p = fused_joint_inputs(joint, encoder_out, predictor_out)
+    else:
+        e, p = fused_joint_inputs(joint, encoder_out, predictor_out)
+    return CF.rnnt_forced_align(e, p, joint.ffn_out.weight, joint.ffn_out.bias, rnnt_text, t_len32, u_len32,
+                                self.blank, precision, activation=act)

@@ -214,6 +214,33 @@ int ctcvr_ctc_loss(const float* log_probs, const int64_t* targets, const int32_t
 int ctcvr_ctc_greedy(const float* scores, const int32_t* lens, int32_t* out_tokens,
                      int32_t* out_lens, int B, int T, int V, int blank, void* stream);
 
+/* ---- Forced alignment: the best (Viterbi) path of a known transcript, batched, one CTA per utterance
+ * (csrc/align.cu).  Lengths are clamped to the tensor extents (a negative length acts as 0) and a CTC label outside
+ * [0, V) acts as blank, as in the loss entry points.  An utterance without a path of finite log-probability (T_b = 0;
+ * CTC: T_b < U_b + repeated neighbours; or every path crossing a -inf log-prob) gets score -inf and -1 in every frame,
+ * label and span entry; no error is raised.  ws: the _ws_bytes query (0 when the shapes take the shared-memory form;
+ * ws may then be NULL).
+ *
+ * ctcvr_rnnt_viterbi: lp_blank / lp_label [B,T,U1] as ctcvr_joint_rnnt_fwd writes them.  delta(0,0) = 0,
+ * delta(t,u) = max(delta(t-1,u) + lp_blank(t-1,u), delta(t,u-1) + lp_label(t,u-1)); scores [B] = delta(T_b-1,U_b) +
+ * lp_blank(T_b-1,U_b).  frames [B,U1-1] int32 = the frame at which label u is emitted (non-decreasing; -1 beyond U_b),
+ * token_logprobs [B,U1-1] = lp_label at that cell (0 beyond U_b).  An exact tie takes the blank predecessor (t-1,u):
+ * the label is emitted at the earlier frame.
+ * ctcvr_ctc_viterbi: log_probs [B,T,V], targets [B,Umax] int64 (padded, as ctcvr_ctc_loss takes them), Umax <= 511.
+ * labels [B,T] int32 = per frame the blank or the label of the best path's state (-1 for t >= T_b), frame_logprobs
+ * [B,T] = its log-prob (0 for t >= T_b), scores [B], spans [B,Umax,2] int32 = first frame and last frame + 1 of each
+ * target token (torchaudio.functional.merge_tokens' convention; -1 beyond U_b).  State s-2 is a predecessor of s only
+ * when label(s) != blank and label(s) != label(s-2); an exact tie takes the smaller jump, and between the two end
+ * states the final blank. */
+size_t ctcvr_rnnt_viterbi_ws_bytes(int B, int T, int U1);
+int ctcvr_rnnt_viterbi(const float* lp_blank, const float* lp_label, const int32_t* t_len, const int32_t* u_len,
+                       int32_t* frames, float* token_logprobs, float* scores, int B, int T, int U1, void* ws,
+                       size_t ws_bytes, void* stream);
+size_t ctcvr_ctc_viterbi_ws_bytes(int B, int T, int Umax);
+int ctcvr_ctc_viterbi(const float* log_probs, const int64_t* targets, const int32_t* in_lens, const int32_t* tgt_lens,
+                      int32_t* labels, float* frame_logprobs, float* scores, int32_t* spans, int B, int T, int V,
+                      int Umax, int blank, void* ws, size_t ws_bytes, void* stream);
+
 /* Predictor + joint weights for the on-device decoders, in the layouts the kernels stream
  * (all fp32, device).  Source parameters: model/component/predictor.py:27-38 /
  * wenet/transducer/predictor.py:60-89 (embed, rnn.weight_ih_l*, rnn.weight_hh_l*, rnn.bias_*,

@@ -37,6 +37,11 @@ _SIGS = {
     "ctcvr_joint_tc_supported": (I, [I, I, I]),
     "ctcvr_joint_rnnt_fwd_bf16in": (I, [P, P, P, P, P, P, P, P, P, P, I, I, I, I, I, I, P, Z, P]),
     "ctcvr_joint_rnnt_bwd_bf16in": (I, [P] * 14 + [F] + [P] * 4 + [I] * 6 + [P, Z, P]),
+    "ctcvr_joint_tc_vt_supported": (I, [I, I, I]),
+    "ctcvr_joint_rnnt_fwd_vt_ws_bytes": (Z, [I, I, I, I, I, I]),
+    "ctcvr_joint_rnnt_fwd_vt": (I, [P, P, P, P, P, P, P, P, P, P, I, I, I, I, I, I, I, P, Z, P]),
+    "ctcvr_joint_rnnt_bwd_vt_ws_bytes": (Z, [I, I, I, I, I, I]),
+    "ctcvr_joint_rnnt_bwd_vt": (I, [P] * 14 + [F] + [P] * 4 + [I] * 7 + [P, Z, P]),
     "ctcvr_rnnt_prologue": (I, [P, P, I, P, I, I, I, I, P, P, P, P, P]),
     "ctcvr_loss_combine": (I, [P, I, P, F, F, P, P]),
     "ctcvr_cer_ws_bytes": (Z, [I, I, I]),

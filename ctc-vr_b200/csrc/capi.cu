@@ -35,6 +35,15 @@ int joint_bwd_tc(const void*, const void*, int, int, int, const float*, const fl
                  const int32_t*, const float*, const float*, const float*, const float*, const float*, const float*,
                  const float*, float, float*,
                  float*, float*, float*, int, int, int, int, int, int, void*, size_t, cudaStream_t);
+bool joint_tc_vt_supported(int, int, int);
+size_t joint_fwd_vt_ws_bytes(int, int, int, int, int, int);
+int joint_fwd_vt(const float*, const float*, int, int, const float*, const float*, const int32_t*, const int32_t*,
+                 const int32_t*, float*, float*, float*, int, int, int, int, int, int, void*, size_t, cudaStream_t);
+size_t joint_bwd_vt_ws_bytes(int, int, int, int, int, int);
+int joint_bwd_vt(const float*, const float*, int, int, const float*, const float*, const int32_t*, const int32_t*,
+                 const int32_t*, const float*, const float*, const float*, const float*, const float*, const float*,
+                 const float*, float, float*, float*, float*, float*, int, int, int, int, int, int, void*, size_t,
+                 cudaStream_t);
 int rnnt_lattice(const float*, const float*, const int32_t*, const int32_t*, float*, float*, float*, int, int, int,
                  cudaStream_t);
 int rnnt_loss_dense(const float*, const int32_t*, const int32_t*, const int32_t*, float*, float*, int, int, int, int,
@@ -207,6 +216,56 @@ int ctcvr_joint_rnnt_bwd(const float* enc_proj, const float* pred_proj, const fl
 }
 
 int ctcvr_joint_tc_supported(int U1, int D, int V) { return joint_tc_bwd_supported(U1, D, V) ? 1 : 0; }
+
+int ctcvr_joint_tc_vt_supported(int U1, int D, int V) { return joint_tc_vt_supported(U1, D, V) ? 1 : 0; }
+
+size_t ctcvr_joint_rnnt_fwd_vt_ws_bytes(int B, int T, int U1, int D, int V, int precision) {
+  precision &= 0xff;                        // the activation bits do not change the workspace
+  if (precision == CTCVR_BF16 || precision == CTCVR_BF16X3)
+    return joint_fwd_vt_ws_bytes(B, T, U1, D, V, precision == CTCVR_BF16X3);
+  return 256;
+}
+
+int ctcvr_joint_rnnt_fwd_vt(const float* enc_proj, const float* pred_proj, const float* w_out, const float* b_out,
+                            const int32_t* targets, const int32_t* t_len, const int32_t* u_len, float* lse,
+                            float* lp_blank, float* lp_label, int B, int T, int U1, int D, int V, int blank,
+                            int precision, void* ws, size_t ws_bytes, void* stream) {
+  if (int rc = check_dims("joint_rnnt_fwd_vt", B, T, U1, D, V)) return rc;
+  CTCVR_REQUIRE(enc_proj && pred_proj && w_out && b_out && t_len && u_len && lse && lp_blank && lp_label &&
+                    (targets || U1 == 1), "joint_rnnt_fwd_vt: NULL pointer");
+  CTCVR_REQUIRE(blank >= 0 && blank < V, "joint_rnnt_fwd_vt: blank %d must be within [0, %d)", blank, V);
+  int prec = 0, act = 0;
+  CTCVR_SPLIT_PRECISION("joint_rnnt_fwd_vt", precision, prec, act);
+  CTCVR_REQUIRE(prec != CTCVR_F32, "joint_rnnt_fwd_vt: precision CTCVR_F32 takes every vocabulary in ctcvr_joint_rnnt_fwd");
+  return joint_fwd_vt(enc_proj, pred_proj, prec == CTCVR_BF16X3, act, w_out, b_out, targets, t_len, u_len, lse, lp_blank,
+                      lp_label, B, T, U1, D, V, blank, ws, ws_bytes, ST(stream));
+}
+
+size_t ctcvr_joint_rnnt_bwd_vt_ws_bytes(int B, int T, int U1, int D, int V, int precision) {
+  precision &= 0xff;                        // the activation bits do not change the workspace
+  if (precision == CTCVR_BF16 || precision == CTCVR_BF16X3)
+    return joint_bwd_vt_ws_bytes(B, T, U1, D, V, precision == CTCVR_BF16X3);
+  return 256;
+}
+
+int ctcvr_joint_rnnt_bwd_vt(const float* enc_proj, const float* pred_proj, const float* w_out, const float* b_out,
+                            const int32_t* targets, const int32_t* t_len, const int32_t* u_len, const float* lse,
+                            const float* lp_blank, const float* lp_label, const float* alpha, const float* beta,
+                            const float* costs, const float* grad_costs, float clamp, float* d_enc_proj,
+                            float* d_pred_proj, float* d_w_out, float* d_b_out, int B, int T, int U1, int D, int V,
+                            int blank, int precision, void* ws, size_t ws_bytes, void* stream) {
+  if (int rc = check_dims("joint_rnnt_bwd_vt", B, T, U1, D, V)) return rc;
+  CTCVR_REQUIRE(enc_proj && pred_proj && w_out && b_out && t_len && u_len && lse && lp_blank && lp_label && alpha &&
+                    beta && costs && grad_costs && d_enc_proj && d_pred_proj && d_w_out && d_b_out && ws,
+                "joint_rnnt_bwd_vt: NULL pointer");
+  CTCVR_REQUIRE(blank >= 0 && blank < V, "joint_rnnt_bwd_vt: blank %d must be within [0, %d)", blank, V);
+  int prec = 0, act = 0;
+  CTCVR_SPLIT_PRECISION("joint_rnnt_bwd_vt", precision, prec, act);
+  CTCVR_REQUIRE(prec != CTCVR_F32, "joint_rnnt_bwd_vt: precision CTCVR_F32 takes every vocabulary in ctcvr_joint_rnnt_bwd");
+  return joint_bwd_vt(enc_proj, pred_proj, prec == CTCVR_BF16X3, act, w_out, b_out, targets, t_len, u_len, lse, lp_blank,
+                      lp_label, alpha, beta, costs, grad_costs, clamp, d_enc_proj, d_pred_proj, d_w_out, d_b_out, B, T,
+                      U1, D, V, blank, ws, ws_bytes, ST(stream));
+}
 
 int ctcvr_joint_rnnt_fwd_bf16in(const void* enc_proj_bf16, const void* pred_proj_bf16, const float* w_out,
                                 const float* b_out, const int32_t* targets, const int32_t* t_len, const int32_t* u_len,

@@ -704,6 +704,46 @@ __global__ void __launch_bounds__(256) prep_kernel(const PrepArgs q) {
     if (q.na4 + q.nb4 > 0) to_bf16_part(first, stride, q.a, q.ab, q.na4, q.b4, q.bb, q.nb4);
   }
 }
+// Vocabulary tiles: the same launch with the weights of nvt tiles of Vp = Vc columns each (q.V = the full vocabulary,
+// q.nW = weight blocks per tile).  Tile c holds rows [c Vc, c Vc + Vc) of W_out; its w_t / wt_t / bias_l2 follow those of
+// tile c - 1 without a gap.
+template <bool SPLIT>
+__global__ void __launch_bounds__(256) prep_vt_kernel(const PrepArgs q, int nvt) {
+  const int blk = blockIdx.x;
+  if (blk < q.nW * nvt) {
+    const int c = blk / q.nW, v0 = c * q.Vp;
+    const size_t ws = (size_t)q.Vp * q.D * (SPLIT ? 2 : 1), wts = (size_t)((q.Vp + 63) / 64) * 64 * q.D * (SPLIT ? 2 : 1);
+    prep_weights3_part<SPLIT>((blk - c * q.nW) * 256 + threadIdx.x, q.w + (size_t)v0 * q.D, q.bias + v0, q.w_t + c * ws,
+                              q.wt_t ? q.wt_t + c * wts : nullptr, nullptr, q.bias_l2 + (size_t)c * q.Vp,
+                              min(q.V - v0, q.Vp), q.Vp, q.D);
+  } else {                                // the blocks behind the weights: as in prep_kernel
+    const int nW = q.nW * nvt;
+    if (blk < nW + q.B) {
+      if (q.geom) build_tiles_block(blk - nW, q.t_len, q.u_len, q.B, q.T, q.U1, q.geom, q.tiles, q.tile_rows, q.ntiles, q.max_tiles);
+      else build_tiles_fwd_block(blk - nW, q.t_len, q.u_len, q.B, q.T, q.U1, q.tiles, q.ntiles, q.max_tiles, q.fwd_pair);
+    } else {
+      const long nb = gridDim.x - nW - q.B, first = (long)(blk - nW - q.B) * 256 + threadIdx.x, stride = nb * 256;
+      for (long i = first; i < q.n0; i += stride) q.zero0[i] = 0.f;
+      for (long i = first; i < q.n1; i += stride) q.zero1[i] = 0.f;
+      if (q.na4 + q.nb4 > 0) to_bf16_part(first, stride, q.a, q.ab, q.na4, q.b4, q.bb, q.nb4);
+    }
+  }
+}
+
+// Vocabulary tiles, after the last tile's forward: lp_blank / lp_label hold raw logit + bias, lse the merged log-sum-exp
+// of the whole vocabulary.  One thread per lattice cell; the cells the untiled forward writes, written the same way.
+__global__ void __launch_bounds__(256) vt_finalize_kernel(const float* __restrict__ lse, float* __restrict__ lp_blank,
+                                                          float* __restrict__ lp_label, const int32_t* __restrict__ t_len,
+                                                          const int32_t* __restrict__ u_len, int B, int T, int U1) {
+  const long i = (long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= (long)B * T * U1) return;
+  const int b = (int)(i / ((long)T * U1)), r = (int)(i - (long)b * T * U1), t = r / U1, u = r - t * U1;
+  const int Tb = max(min(t_len[b], T), 0), Ub = max(min(u_len[b], U1 - 1), 0);
+  if (t >= Tb || u > Ub) return;
+  const float l = lse[i];
+  lp_blank[i] -= l;
+  lp_label[i] = (u < Ub) ? lp_label[i] - l : kNegInf;
+}
 
 int make_tmap_bf16_2d(CUtensorMap* map, const void* base, uint64_t rows, uint64_t cols, uint64_t pitch_elems,
                       uint32_t box_rows, bool swizzle) {
@@ -788,6 +828,19 @@ bool joint_tc_supported(int U1, int D, int V) { return D % 64 == 0 && D >= 64 &&
 // the predicate of the bf16 path, both directions (the backward tiles D in 128-lane blocks of dZ^T, at most four)
 bool joint_tc_bwd_supported(int U1, int D, int V) { return joint_tc_supported(U1, D, V) && D % 128 == 0 && D <= 512; }
 
+// Vocabulary tiles (ctcvr_joint_rnnt_*_vt): n = ceil(pad32(V) / 416) tiles of Vc = pad32(ceil(V / n)) columns; tile c
+// covers [c Vc, min(V, c Vc + Vc)).  Every tile is a vocabulary the untiled kernels take (Vc <= 416), and the last one
+// is non-empty for every V up to the cap.
+constexpr int VT_MAX_V = 32768;
+struct VocabTiles { int n, Vc; };
+static VocabTiles vocab_tiles(int V) {
+  const int n = cdiv(pad_v(V), 416);
+  return {n, pad_v(cdiv(V, n))};
+}
+bool joint_tc_vt_supported(int U1, int D, int V) {
+  return D % 128 == 0 && D >= 128 && D <= 512 && U1 >= 1 && U1 <= 128 && V >= 1 && V <= VT_MAX_V;
+}
+
 static int max_tiles_fwd2(int B, int T, int U1) {
   return B * ((U1 >> 2) * ((T + 31) / 32) + (T + 63) / 64 + (T + 63) / 64);
 }
@@ -800,17 +853,18 @@ struct FwdWs {
   size_t bytes;
 };
 // split (bf16x3): hi and lo copies of W_out; the fp32 activations are read in place (no bf16 copies)
-static FwdWs carve_fwd_ws(void* ws, int B, int T, int U1, int D, int V, bool split = false) {
+// nvt > 1: vocabulary tiles of V = Vc columns each, their weights back to back
+static FwdWs carve_fwd_ws(void* ws, int B, int T, int U1, int D, int V, bool split = false, int nvt = 1) {
   int Vp = pad_v(V);
   uint8_t* p = reinterpret_cast<uint8_t*>(ws);
   size_t off = 0;
   FwdWs w;
   auto take = [&](size_t n) { void* r = p + off; off = align_up(off + n, 1024); return r; };
-  w.wb = reinterpret_cast<__nv_bfloat16*>(take((size_t)Vp * D * 2 * (split ? 2 : 1)));
+  w.wb = reinterpret_cast<__nv_bfloat16*>(take((size_t)nvt * Vp * D * 2 * (split ? 2 : 1)));
   w.eb = split ? nullptr : reinterpret_cast<__nv_bfloat16*>(take((size_t)B * T * D * 2));
   w.pb = split ? nullptr : reinterpret_cast<__nv_bfloat16*>(take((size_t)B * U1 * D * 2));
   w.bias_pad = reinterpret_cast<float*>(take((size_t)Vp * 4));
-  w.bias_l2 = reinterpret_cast<float*>(take((size_t)Vp * 4));
+  w.bias_l2 = reinterpret_cast<float*>(take((size_t)nvt * Vp * 4));
   const int mt = max_tiles_flat(B, T, U1) > max_tiles_fwd2(B, T, U1) ? max_tiles_flat(B, T, U1) : max_tiles_fwd2(B, T, U1);
   w.tiles = reinterpret_cast<int4*>(take((size_t)mt * 16));
   w.ntiles = reinterpret_cast<int*>(take(4));
@@ -841,6 +895,39 @@ int joint_fwd_f32(const float*, const float*, const float*, const float*, const 
 template <class K>
 static K pick_act(int act, K tanh_k, K relu_k, K gelu_k) { return act == ACT_RELU ? relu_k : act == ACT_GELU ? gelu_k : tanh_k; }
 
+// the fields of FwdParams every single-CTA forward launch shares
+static FwdParams fwd_params(const FwdWs& W, const float* bias, const int32_t* targets, const int32_t* t_len,
+                            const int32_t* u_len, float* lse, float* lp_blank, float* lp_label, int B, int T, int U1,
+                            int D, int V, int blank) {
+  FwdParams p{};
+  p.w_t = W.wb;
+  p.bias = bias; p.bias_l2 = W.bias_l2; p.targets = targets; p.t_len = t_len; p.u_len = u_len;
+  p.tiles = W.tiles; p.ntiles = W.ntiles;
+  p.B = B; p.T = T; p.U1 = U1; p.D = D; p.V = V; p.Vp = pad_v(V); p.NH = p.Vp / 2; p.blank = blank;
+  p.lse = lse; p.lp_blank = lp_blank; p.lp_label = lp_label;
+  p.prof = g_prof_buf;
+  tc_error_host_word(&p.err_host);
+  return p;
+}
+
+// one launch of the single-CTA forward kernel (joint_fwd2_*): the untiled call, or one vocabulary tile (vt)
+static int launch_fwd2(FwdParams& p, const CUtensorMap& tmap_e, const CUtensorMap& tmap_p, bool split, int act, bool vt,
+                       int mt, cudaStream_t st) {
+  int ws_n = F_MAX_W_STAGES;
+  while (ws_n > 2 && fwd2_smem_bytes(p.NH, p.Vp, ws_n) > 232448) --ws_n;
+  p.w_stages = ws_n;
+  const size_t smem = fwd2_smem_bytes(p.NH, p.Vp, ws_n);
+  CTCVR_REQUIRE(smem <= 232448, "joint_rnnt_fwd %s: shared memory budget exceeded (%zu B)", split ? "bf16x3" : "bf16", smem);
+  const auto kern = split ? (vt ? pick_act(act, joint_fwd2_x3_vt_kernel, joint_fwd2_x3_vt_relu_kernel, joint_fwd2_x3_vt_gelu_kernel)
+                                : pick_act(act, joint_fwd2_x3_kernel, joint_fwd2_x3_relu_kernel, joint_fwd2_x3_gelu_kernel))
+                          : (vt ? pick_act(act, joint_fwd2_vt_kernel, joint_fwd2_vt_relu_kernel, joint_fwd2_vt_gelu_kernel)
+                                : pick_act(act, joint_fwd2_kernel, joint_fwd2_relu_kernel, joint_fwd2_gelu_kernel));
+  CTCVR_CHECK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  kern<<<min(sm_count(), mt), F_THREADS, smem, st>>>(tmap_e, tmap_p, p);
+  CTCVR_LAUNCH_CHECK();
+  return 0;
+}
+
 // split = 1: precision bf16x3 (fp32 inputs, hi / lo operand split, joint_fwd2_x3_kernel); act: the joint activation
 int joint_fwd_tc(const void* enc_v, const void* pred_v, int in_bf16, int split, int act, const float* w, const float* bias,
                  const int32_t* targets, const int32_t* t_len, const int32_t* u_len, float* lse, float* lp_blank,
@@ -864,25 +951,10 @@ int joint_fwd_tc(const void* enc_v, const void* pred_v, int in_bf16, int split, 
     q.tiles = W.tiles; q.ntiles = W.ntiles;
     prep_kernel<true><<<q.nW + B, 256, 0, st>>>(q);
     CTCVR_LAUNCH_CHECK();
-    FwdParams p{};
-    p.w_t = W.wb; p.enc = enc; p.pred = pred;
-    p.bias = bias; p.bias_l2 = W.bias_l2; p.targets = targets; p.t_len = t_len; p.u_len = u_len;
-    p.tiles = W.tiles; p.ntiles = W.ntiles;
-    p.B = B; p.T = T; p.U1 = U1; p.D = D; p.V = V; p.Vp = Vp; p.NH = NH; p.blank = blank;
-    p.lse = lse; p.lp_blank = lp_blank; p.lp_label = lp_label;
-    p.prof = g_prof_buf;
-    tc_error_host_word(&p.err_host);
-    int ws_n = F_MAX_W_STAGES;
-    while (ws_n > 2 && fwd2_smem_bytes(NH, Vp, ws_n) > 232448) --ws_n;
-    p.w_stages = ws_n;
-    const size_t smem = fwd2_smem_bytes(NH, Vp, ws_n);
-    CTCVR_REQUIRE(smem <= 232448, "joint_rnnt_fwd bf16x3: shared memory budget exceeded (%zu B)", smem);
-    const auto kern = pick_act(act, joint_fwd2_x3_kernel, joint_fwd2_x3_relu_kernel, joint_fwd2_x3_gelu_kernel);
-    CTCVR_CHECK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    FwdParams p = fwd_params(W, bias, targets, t_len, u_len, lse, lp_blank, lp_label, B, T, U1, D, V, blank);
+    p.enc = enc; p.pred = pred;
     const CUtensorMap unused{};             // the bf16x3 producers read the fp32 rows directly
-    kern<<<min(sm_count(), mt), F_THREADS, smem, st>>>(unused, unused, p);
-    CTCVR_LAUNCH_CHECK();
-    return 0;
+    return launch_fwd2(p, unused, unused, true, act, false, mt, st);
   }
   // the parked CTA-pair forward computes tanh only
   const bool use_pair = fwdp_smem_bytes(NH, D) <= 232448 && sm_count() >= 2 && !g_force_single_cta && act == ACT_TANH;
@@ -925,23 +997,68 @@ int joint_fwd_tc(const void* enc_v, const void* pred_v, int in_bf16, int split, 
   CUtensorMap tmap_e, tmap_p;
   if (make_tmap_bf16_2d(&tmap_e, W.eb, (uint64_t)B * T, D, D, 32)) return 1;
   if (make_tmap_bf16_2d(&tmap_p, W.pb, (uint64_t)B * U1, D, D, 4)) return 1;
-  FwdParams p{};
-  p.w_t = W.wb;
-  p.bias = bias; p.bias_l2 = W.bias_l2; p.targets = targets; p.t_len = t_len; p.u_len = u_len;
-  p.tiles = W.tiles; p.ntiles = W.ntiles;
-  p.B = B; p.T = T; p.U1 = U1; p.D = D; p.V = V; p.Vp = Vp; p.NH = NH; p.blank = blank;
-  p.lse = lse; p.lp_blank = lp_blank; p.lp_label = lp_label;
-  p.prof = g_prof_buf;
-  tc_error_host_word(&p.err_host);
-  int ws_n = F_MAX_W_STAGES;
-  while (ws_n > 2 && fwd2_smem_bytes(NH, Vp, ws_n) > 232448) --ws_n;
-  p.w_stages = ws_n;
-  const size_t smem = fwd2_smem_bytes(NH, Vp, ws_n);
-  CTCVR_REQUIRE(smem <= 232448, "joint_rnnt_fwd bf16: shared memory budget exceeded (%zu B)", smem);
-  const auto kern = pick_act(act, joint_fwd2_kernel, joint_fwd2_relu_kernel, joint_fwd2_gelu_kernel);
-  CTCVR_CHECK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  const int grid = min(sm_count(), mt);
-  kern<<<grid, F_THREADS, smem, st>>>(tmap_e, tmap_p, p);
+  FwdParams p = fwd_params(W, bias, targets, t_len, u_len, lse, lp_blank, lp_label, B, T, U1, D, V, blank);
+  return launch_fwd2(p, tmap_e, tmap_p, false, act, false, mt, st);
+}
+
+size_t joint_fwd_vt_ws_bytes(int B, int T, int U1, int D, int V, int split) {
+  if (!joint_tc_vt_supported(U1, D, V)) return 256;       // the call itself fails with the reason
+  const VocabTiles vt = vocab_tiles(V);
+  if (vt.n == 1) return joint_fwd_tc_ws_bytes(B, T, U1, D, V, split);
+  return carve_fwd_ws(nullptr, B, T, U1, D, vt.Vc, split != 0, vt.n).bytes;
+}
+
+// Vocabulary tiles (ctcvr_joint_rnnt_fwd_vt): one prep launch for the weights of every tile, one forward launch per
+// tile merging its log-sum-exp into lse, and vt_finalize_kernel.  One tile (pad32(V) <= 416) is the untiled call.
+int joint_fwd_vt(const float* enc, const float* pred, int split, int act, const float* w, const float* bias,
+                 const int32_t* targets, const int32_t* t_len, const int32_t* u_len, float* lse, float* lp_blank,
+                 float* lp_label, int B, int T, int U1, int D, int V, int blank, void* ws, size_t ws_bytes, cudaStream_t st) {
+  const char* prec = split ? "bf16x3" : "bf16";
+  CTCVR_REQUIRE(joint_tc_vt_supported(U1, D, V), "joint_rnnt_fwd_vt: precision = %s needs D %% 128 == 0, D <= 512, V <= %d and U+1 <= 128 (got D=%d V=%d U+1=%d); use precision = fp32 for this shape", prec, VT_MAX_V, D, V, U1);
+  const VocabTiles vt = vocab_tiles(V);
+  if (vt.n == 1)
+    return joint_fwd_tc(enc, pred, 0, split, act, w, bias, targets, t_len, u_len, lse, lp_blank, lp_label, B, T, U1, D, V,
+                        blank, ws, ws_bytes, st);
+  if (check_tc_error("joint_rnnt_fwd_vt")) return 1;
+  CTCVR_REQUIRE(ws && ws_bytes >= joint_fwd_vt_ws_bytes(B, T, U1, D, V, split), "joint_rnnt_fwd_vt %s: workspace too small", prec);
+  CTCVR_REQUIRE(((uintptr_t)enc & 15) == 0 && ((uintptr_t)pred & 15) == 0, "joint_rnnt_fwd_vt %s: enc_proj / pred_proj must be 16-byte aligned", prec);
+  const int Vc = vt.Vc;
+  FwdWs W = carve_fwd_ws(ws, B, T, U1, D, Vc, split != 0, vt.n);
+  const int mt = max_tiles_fwd2(B, T, U1);
+  {
+    PrepArgs q{};
+    q.w = w; q.bias = bias; q.w_t = W.wb; q.bias_l2 = W.bias_l2; q.V = V; q.Vp = Vc; q.D = D;
+    q.nW = cdiv((long)((Vc + 63) / 64) * 64 * D, 256);
+    q.t_len = t_len; q.u_len = u_len; q.B = B; q.T = T; q.U1 = U1; q.geom = 0; q.max_tiles = mt;
+    q.tiles = W.tiles; q.ntiles = W.ntiles;
+    int extra = 0;
+    if (!split) {
+      q.a = reinterpret_cast<const float4*>(enc); q.ab = reinterpret_cast<uint2*>(W.eb); q.na4 = (long)B * T * D / 4;
+      q.b4 = reinterpret_cast<const float4*>(pred); q.bb = reinterpret_cast<uint2*>(W.pb); q.nb4 = (long)B * U1 * D / 4;
+      extra = (int)std::min<long>((q.na4 + q.nb4 + 255) / 256, 148L * 8);
+    }
+    if (split) prep_vt_kernel<true><<<q.nW * vt.n + B, 256, 0, st>>>(q, vt.n);
+    else prep_vt_kernel<false><<<q.nW * vt.n + B + extra, 256, 0, st>>>(q, vt.n);
+    CTCVR_LAUNCH_CHECK();
+  }
+  CUtensorMap tmap_e{}, tmap_p{};           // bf16x3: unused (the producers read the fp32 rows directly)
+  if (!split) {
+    if (make_tmap_bf16_2d(&tmap_e, W.eb, (uint64_t)B * T, D, D, 32)) return 1;
+    if (make_tmap_bf16_2d(&tmap_p, W.pb, (uint64_t)B * U1, D, D, 4)) return 1;
+  }
+  const size_t wstride = (size_t)Vc * D * (split ? 2 : 1);
+  for (int c = 0; c < vt.n; ++c) {
+    const int v0 = c * Vc, Vr = std::min(V - v0, Vc);
+    FwdParams p = fwd_params(W, bias + v0, targets, t_len, u_len, lse, lp_blank, lp_label, B, T, U1, D, Vr,
+                             (blank >= v0 && blank < v0 + Vr) ? blank - v0 : -1);
+    p.w_t = W.wb + c * wstride; p.bias_l2 = W.bias_l2 + (size_t)c * Vc;
+    p.Vp = Vc; p.NH = Vc / 2;                 // the tile's padded width (pad_v(Vr) may be smaller in the last tile)
+    if (split) { p.enc = enc; p.pred = pred; }
+    p.v0 = v0; p.Vg = V; p.blank_g = blank; p.merge = c > 0;
+    if (launch_fwd2(p, tmap_e, tmap_p, split != 0, act, true, mt, st)) return 1;
+  }
+  const long cells = (long)B * T * U1;
+  vt_finalize_kernel<<<cdiv(cells, 256), 256, 0, st>>>(lse, lp_blank, lp_label, t_len, u_len, B, T, U1);
   CTCVR_LAUNCH_CHECK();
   return 0;
 }
@@ -962,7 +1079,8 @@ struct BwdWs {
   size_t bytes;
 };
 // split (bf16x3): hi / lo copies of W_out and W_out^T and a second G spill (G_lo); no bf16 activation copies
-static BwdWs carve_bwd_ws(void* ws, int B, int T, int U1, int D, int V, bool split = false) {
+// nvt > 1: vocabulary tiles of V = Vc columns each: their weights back to back, one tile's G spill and dW partials
+static BwdWs carve_bwd_ws(void* ws, int B, int T, int U1, int D, int V, bool split = false, int nvt = 1) {
   const int Vp = pad_v(V);
   uint8_t* p = reinterpret_cast<uint8_t*>(ws);
   size_t off = 0;
@@ -975,12 +1093,12 @@ static BwdWs carve_bwd_ws(void* ws, int B, int T, int U1, int D, int V, bool spl
   if (w.KS < 1) w.KS = 1;
   auto take = [&](size_t n) { void* r = p + off; off = align_up(off + n, 1024); return r; };
   const size_t nw = split ? 2 : 1;
-  w.wb = reinterpret_cast<__nv_bfloat16*>(take((size_t)Vp * D * 2 * nw));
-  w.wtb = reinterpret_cast<__nv_bfloat16*>(take((size_t)((Vp + 63) / 64) * 64 * D * 2 * nw));
+  w.wb = reinterpret_cast<__nv_bfloat16*>(take((size_t)nvt * Vp * D * 2 * nw));
+  w.wtb = reinterpret_cast<__nv_bfloat16*>(take((size_t)nvt * ((Vp + 63) / 64) * 64 * D * 2 * nw));
   w.eb = split ? nullptr : reinterpret_cast<__nv_bfloat16*>(take((size_t)B * T * D * 2));
   w.pb = split ? nullptr : reinterpret_cast<__nv_bfloat16*>(take((size_t)B * U1 * D * 2));
   w.bias_pad = reinterpret_cast<float*>(take((size_t)Vp * 4));
-  w.bias_l2 = reinterpret_cast<float*>(take((size_t)Vp * 4));
+  w.bias_l2 = reinterpret_cast<float*>(take((size_t)nvt * Vp * 4));
   w.tiles = reinterpret_cast<int4*>(take((size_t)w.mt * 16));
   w.tile_rows = reinterpret_cast<int4*>(take((size_t)w.mt * 16));
   w.ntiles = reinterpret_cast<int*>(take(4));
@@ -988,7 +1106,7 @@ static BwdWs carve_bwd_ws(void* ws, int B, int T, int U1, int D, int V, bool spl
   w.gt_lo = split ? reinterpret_cast<__nv_bfloat16*>(take((size_t)((Vp + 63) / 64) * 64 * w.Rpad * 2)) : nullptr;
   w.d_enc_part = reinterpret_cast<float*>(take((size_t)w.S_max * B * T * D * 4));
   w.partials = reinterpret_cast<float*>(take((size_t)w.KS * D * Vp * 4));
-  w.d_pred_acc = reinterpret_cast<float*>(take((size_t)B * U1 * D * 4));
+  w.d_pred_acc = nvt > 1 ? nullptr : reinterpret_cast<float*>(take((size_t)B * U1 * D * 4));   // bf16 inputs only
   w.bytes = off;
   return w;
 }
@@ -998,31 +1116,96 @@ size_t joint_bwd_tc_ws_bytes(int B, int T, int U1, int D, int V, int split) {
   return carve_bwd_ws(nullptr, B, T, U1, D, V, split != 0).bytes;
 }
 
-// precision bf16x3: the single-CTA backward kernel and the dW GEMM in their split forms (fp32 inputs and gradients)
+// Kernel 1 of the backward for tile geometry (P, TT): the CTA-pair kernel (bf16, use_pair), the single-CTA kernel or its
+// bf16x3 form; the untiled call, or one vocabulary tile (vt).  The tensor maps are unused by the bf16x3 form.
 template <int P, int TT>
-static int joint_bwd_x3(const float* enc, const float* pred, BwdParams& p, const BwdWs& W, const int32_t* t_len,
-                        const int32_t* u_len, float* d_enc, float* d_w, int B, int T, int U1, int D, int V, int act,
-                        cudaStream_t st) {
-  const int Vp = p.Vp, KBG = (Vp + 63) / 64, MB = D / 128;
-  const CUtensorMap unused{};               // the split kernels read the fp32 rows directly
-  const size_t smem = bwd3_smem_bytes(p.NH, Vp, D, true);
-  CTCVR_REQUIRE(smem <= 232448 && p.r1_stages >= 2, "joint_rnnt_bwd bf16x3: shared memory budget exceeded (%zu B)", smem);
-  const auto k1 = pick_act(act, joint_bwd3_x3_kernel<P, TT>, joint_bwd3_x3_relu_kernel<P, TT>, joint_bwd3_x3_gelu_kernel<P, TT>);
-  CTCVR_CHECK_CUDA(cudaFuncSetAttribute(k1, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  k1<<<min(sm_count(), W.mt), NTHREADS, smem, st>>>(unused, unused, p);
+static int launch_bwd_main(BwdParams& p, const BwdWs& W, bool use_pair, bool split, int act, bool vt, cudaStream_t st) {
+  const int B = p.B, T = p.T, U1 = p.U1, D = p.D;
+  CUtensorMap tmap_e{}, tmap_p{};
+  if (!split) {
+    if (make_tmap_bf16_2d(&tmap_e, W.eb, (uint64_t)B * T, D, D, TT)) return 1;
+    if (make_tmap_bf16_2d(&tmap_p, W.pb, (uint64_t)B * U1, D, D, P)) return 1;
+  }
+  if (use_pair) {
+    CUtensorMap tmap_e2;                 // both tiles' frames in one box (P4 slab)
+    if (make_tmap_bf16_2d(&tmap_e2, W.eb, (uint64_t)B * T, D, D, 2 * TT)) return 1;
+    p.r1_stages = bwd4_r1_stages(p.NH, p.Vp);
+    const size_t smem = bwd4_smem_bytes<P>(p.NH, p.Vp, D);
+    const int gridp = std::max(2, std::min(sm_count() & ~1, W.mt & ~1));
+    const auto k = vt ? pick_act(act, joint_bwd4_vt_kernel<P, TT>, joint_bwd4_vt_relu_kernel<P, TT>, joint_bwd4_vt_gelu_kernel<P, TT>)
+                      : pick_act(act, joint_bwd4_kernel<P, TT>, joint_bwd4_relu_kernel<P, TT>, joint_bwd4_gelu_kernel<P, TT>);
+    CTCVR_CHECK_CUDA(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    k<<<gridp, NTHREADS, smem, st>>>(tmap_e, tmap_e2, tmap_p, p);
+    CTCVR_LAUNCH_CHECK();
+    return 0;
+  }
+  p.r1_stages = bwd3_r1_stages(p.NH, p.Vp);
+  const size_t smem = bwd3_smem_bytes(p.NH, p.Vp, D, split);
+  CTCVR_REQUIRE(smem <= 232448 && p.r1_stages >= 2, "joint_rnnt_bwd %s: shared memory budget exceeded (%zu B)", split ? "bf16x3" : "bf16", smem);
+  const auto k = split ? (vt ? pick_act(act, joint_bwd3_x3_vt_kernel<P, TT>, joint_bwd3_x3_vt_relu_kernel<P, TT>, joint_bwd3_x3_vt_gelu_kernel<P, TT>)
+                             : pick_act(act, joint_bwd3_x3_kernel<P, TT>, joint_bwd3_x3_relu_kernel<P, TT>, joint_bwd3_x3_gelu_kernel<P, TT>))
+                       : (vt ? pick_act(act, joint_bwd3_vt_kernel<P, TT>, joint_bwd3_vt_relu_kernel<P, TT>, joint_bwd3_vt_gelu_kernel<P, TT>)
+                             : pick_act(act, joint_bwd3_kernel<P, TT>, joint_bwd3_relu_kernel<P, TT>, joint_bwd3_gelu_kernel<P, TT>));
+  CTCVR_CHECK_CUDA(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  k<<<min(sm_count(), W.mt), NTHREADS, smem, st>>>(tmap_e, tmap_p, p);
   CTCVR_LAUNCH_CHECK();
-  reduce_denc_kernel<false><<<B * T, 128, 0, st>>>(W.d_enc_part, t_len, u_len, d_enc, B, T, U1, D, P, nullptr, nullptr);
-  CTCVR_LAUNCH_CHECK();
-  const size_t smem2 = dwr_smem_bytes<P>(KBG, true);
-  CTCVR_REQUIRE(smem2 <= 232448, "dW GEMM bf16x3: shared memory budget exceeded (%zu B)", smem2);
-  const auto k2 = pick_act(act, dw_gemm_rz_x3_kernel<P, TT>, dw_gemm_rz_x3_relu_kernel<P, TT>, dw_gemm_rz_x3_gelu_kernel<P, TT>);
-  CTCVR_CHECK_CUDA(cudaFuncSetAttribute(k2, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem2));
-  k2<<<dim3(MB, W.KS), DWR_THREADS, smem2, st>>>(unused, unused, W.gt, W.gt_lo, enc, pred, W.tile_rows, W.ntiles, W.partials, D,
-                                                 Vp, KBG, W.KS);
+  return 0;
+}
+
+// Kernel 2 of the backward and its split-K reduction: d_w[v][:] for the V real rows of the Vp-column G spill in gt
+// (/ gt_lo), for tile geometry (P, TT).  d_w points at the first row of the vocabulary tile.
+template <int P, int TT>
+static int launch_bwd_dw(const BwdWs& W, const float* enc, const float* pred, const __nv_bfloat16* gt,
+                         const __nv_bfloat16* gt_lo, float* d_w, int B, int T, int U1, int D, int V, int Vp, bool split,
+                         int act, cudaStream_t st) {
+  const int KBG = (Vp + 63) / 64, MB = D / 128;
+  const size_t smem = dwr_smem_bytes<P>(KBG, split);
+  CTCVR_REQUIRE(smem <= 232448, "dW GEMM%s: shared memory budget exceeded (%zu B)", split ? " bf16x3" : "", smem);
+  if (split) {
+    const CUtensorMap unused{};             // the split kernels read the fp32 rows directly
+    const auto k = pick_act(act, dw_gemm_rz_x3_kernel<P, TT>, dw_gemm_rz_x3_relu_kernel<P, TT>, dw_gemm_rz_x3_gelu_kernel<P, TT>);
+    CTCVR_CHECK_CUDA(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    k<<<dim3(MB, W.KS), DWR_THREADS, smem, st>>>(unused, unused, gt, gt_lo, enc, pred, W.tile_rows, W.ntiles, W.partials, D,
+                                                Vp, KBG, W.KS);
+  } else {
+    CUtensorMap tmap_e, tmap_p;          // the same 64-wide SW128 boxes as kernel 1: TT enc rows / P pred rows
+    if (make_tmap_bf16_2d(&tmap_e, W.eb, (uint64_t)B * T, D, D, TT)) return 1;
+    if (make_tmap_bf16_2d(&tmap_p, W.pb, (uint64_t)B * U1, D, D, P)) return 1;
+    const auto k = pick_act(act, dw_gemm_rz_kernel<P, TT>, dw_gemm_rz_relu_kernel<P, TT>, dw_gemm_rz_gelu_kernel<P, TT>);
+    CTCVR_CHECK_CUDA(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    k<<<dim3(MB, W.KS), DWR_THREADS, smem, st>>>(tmap_e, tmap_p, gt, W.tile_rows, W.ntiles, W.partials, D, Vp, KBG, W.KS);
+  }
   CTCVR_LAUNCH_CHECK();
   reduce_dw_kernel<<<dim3(cdiv(D, 8), cdiv(Vp, 32)), 256, 0, st>>>(W.partials, d_w, D, V, Vp, W.KS);
   CTCVR_LAUNCH_CHECK();
   return 0;
+}
+
+// the fields of BwdParams every kernel-1 launch shares
+static BwdParams bwd_params(const BwdWs& W, const float* enc, const float* pred, const int32_t* targets,
+                            const int32_t* t_len, const int32_t* u_len, const float* lse, const float* lp_blank,
+                            const float* lp_label, const float* alpha, const float* beta, const float* costs,
+                            const float* grad_costs, float clamp, float* d_pred, float* d_b, int B, int T, int U1, int D,
+                            int V, int blank, bool split) {
+  BwdParams p{};
+  p.w_t = W.wb; p.wt_t = W.wtb;
+  if (split) { p.enc = enc; p.pred = pred; p.gt_lo = W.gt_lo; }
+  p.bias_l2 = W.bias_l2; p.targets = targets; p.t_len = t_len; p.u_len = u_len;
+  p.tiles = W.tiles; p.ntiles = W.ntiles;
+  p.B = B; p.T = T; p.U1 = U1; p.D = D; p.V = V; p.Vp = pad_v(V); p.NH = p.Vp / 2; p.blank = blank;
+  p.lse = lse; p.lp_blank = lp_blank; p.lp_label = lp_label;
+  p.alpha = alpha; p.beta = beta; p.costs = costs; p.grad_costs = grad_costs; p.clamp = clamp;
+  p.gt = W.gt;
+  p.d_enc_part = W.d_enc_part; p.d_pred = d_pred; p.d_bias = d_b;
+  p.prof = g_prof_buf;
+  tc_error_host_word(&p.err_host);
+  return p;
+}
+
+// the CTA-pair backward kernel takes D % 256 == 0 when its shared memory and ring fit (bf16 only)
+static bool bwd_use_pair(const RectGeom& G, int NH, int Vp, int D) {
+  const size_t smem_pair = G.P == 21 ? bwd4_smem_bytes<21>(NH, Vp, D) : bwd4_smem_bytes<16>(NH, Vp, D);
+  return D % 256 == 0 && smem_pair <= 232448 && sm_count() >= 2 && bwd4_r1_stages(NH, Vp) >= 4 && !g_bwd_single_cta;
 }
 
 int joint_bwd_tc(const void* enc_v, const void* pred_v, int in_bf16, int split, int act, const float* w, const float* bias, const int32_t* targets,
@@ -1036,40 +1219,13 @@ int joint_bwd_tc(const void* enc_v, const void* pred_v, int in_bf16, int split, 
   if (check_tc_error("joint_rnnt_bwd")) return 1;
   CTCVR_REQUIRE(ws && ws_bytes >= joint_bwd_tc_ws_bytes(B, T, U1, D, V, split), "joint_rnnt_bwd %s: workspace too small", split ? "bf16x3" : "bf16");
   CTCVR_REQUIRE(((uintptr_t)enc & 15) == 0 && ((uintptr_t)pred & 15) == 0, "joint_rnnt_bwd %s: enc_proj / pred_proj must be 16-byte aligned", split ? "bf16x3" : "bf16");
-  const int Vp = pad_v(V), NH = Vp / 2, MB = D / 128;
+  const int Vp = pad_v(V), NH = Vp / 2;
   BwdWs W = carve_bwd_ws(ws, B, T, U1, D, V, split != 0);
   const int KBG = (Vp + 63) / 64;
   const int mt = W.mt;
   RectGeom G = pick_rect_geom(T, U1);
-  if (split) {
-    PrepArgs q{};
-    q.w = w; q.bias = bias; q.w_t = W.wb; q.wt_t = W.wtb; q.bias_pad = W.bias_pad; q.bias_l2 = W.bias_l2;
-    q.V = V; q.Vp = Vp; q.D = D; q.nW = cdiv((long)KBG * 64 * D, 256);
-    q.t_len = t_len; q.u_len = u_len; q.B = B; q.T = T; q.U1 = U1; q.geom = G.P | (G.TT << 8);
-    q.max_tiles = mt; q.tiles = W.tiles; q.tile_rows = W.tile_rows; q.ntiles = W.ntiles;
-    q.zero0 = d_pred; q.n0 = (long)B * U1 * D; q.zero1 = d_b; q.n1 = V;
-    const int extra = (int)std::min<long>((q.n0 + 1023) / 1024, 148L * 8);
-    prep_kernel<true><<<q.nW + B + extra, 256, 0, st>>>(q);
-    CTCVR_LAUNCH_CHECK();
-    BwdParams p{};
-    p.w_t = W.wb; p.wt_t = W.wtb; p.enc = enc; p.pred = pred; p.gt_lo = W.gt_lo;
-    p.bias_l2 = W.bias_l2; p.targets = targets; p.t_len = t_len; p.u_len = u_len;
-    p.tiles = W.tiles; p.ntiles = W.ntiles;
-    p.B = B; p.T = T; p.U1 = U1; p.D = D; p.V = V; p.Vp = Vp; p.NH = NH; p.blank = blank;
-    p.r1_stages = bwd3_r1_stages(NH, Vp);
-    p.lse = lse; p.lp_blank = lp_blank; p.lp_label = lp_label;
-    p.alpha = alpha; p.beta = beta; p.costs = costs; p.grad_costs = grad_costs; p.clamp = clamp;
-    p.gt = W.gt;
-    p.d_enc_part = W.d_enc_part; p.d_pred = d_pred; p.d_bias = d_b;
-    p.prof = g_prof_buf;
-    tc_error_host_word(&p.err_host);
-    return G.P == 21 ? joint_bwd_x3<21, 6>(enc, pred, p, W, t_len, u_len, d_enc, d_w, B, T, U1, D, V, act, st)
-                     : joint_bwd_x3<16, 8>(enc, pred, p, W, t_len, u_len, d_enc, d_w, B, T, U1, D, V, act, st);
-  }
   // CTA-pair kernel (joint_tc_bwd_pair.cuh): D in 256-row blocks of dZ^T, tiles paired along the frame axis
-  const size_t smem_pair = G.P == 21 ? bwd4_smem_bytes<21>(NH, Vp, D) : bwd4_smem_bytes<16>(NH, Vp, D);
-  const bool use_pair = D % 256 == 0 && smem_pair <= 232448 && sm_count() >= 2 && bwd4_r1_stages(NH, Vp) >= 4 &&
-                        !g_bwd_single_cta;
+  const bool use_pair = !split && bwd_use_pair(G, NH, Vp, D);
   G.even = use_pair ? 1 : 0;
   // bf16 inputs -> bf16 gradients: d_pred is accumulated in fp32 in the workspace and converted by the d_enc reduction
   float* d_pred_acc = in_bf16 ? W.d_pred_acc : d_pred;
@@ -1080,90 +1236,97 @@ int joint_bwd_tc(const void* enc_v, const void* pred_v, int in_bf16, int split, 
     q.t_len = t_len; q.u_len = u_len; q.B = B; q.T = T; q.U1 = U1; q.geom = G.P | (G.TT << 8) | (G.even << 16);
     q.max_tiles = mt; q.tiles = W.tiles; q.tile_rows = W.tile_rows; q.ntiles = W.ntiles;
     q.zero0 = d_pred_acc; q.n0 = (long)B * U1 * D; q.zero1 = d_b; q.n1 = V;
-    if (in_bf16) {
-      W.eb = const_cast<__nv_bfloat16*>(reinterpret_cast<const __nv_bfloat16*>(enc_v));
-      W.pb = const_cast<__nv_bfloat16*>(reinterpret_cast<const __nv_bfloat16*>(pred_v));
+    if (split) {
+      const int extra = (int)std::min<long>((q.n0 + 1023) / 1024, 148L * 8);
+      prep_kernel<true><<<q.nW + B + extra, 256, 0, st>>>(q);
     } else {
-      q.a = reinterpret_cast<const float4*>(enc); q.ab = reinterpret_cast<uint2*>(W.eb); q.na4 = (long)B * T * D / 4;
-      q.b4 = reinterpret_cast<const float4*>(pred); q.bb = reinterpret_cast<uint2*>(W.pb); q.nb4 = (long)B * U1 * D / 4;
+      if (in_bf16) {
+        W.eb = const_cast<__nv_bfloat16*>(reinterpret_cast<const __nv_bfloat16*>(enc_v));
+        W.pb = const_cast<__nv_bfloat16*>(reinterpret_cast<const __nv_bfloat16*>(pred_v));
+      } else {
+        q.a = reinterpret_cast<const float4*>(enc); q.ab = reinterpret_cast<uint2*>(W.eb); q.na4 = (long)B * T * D / 4;
+        q.b4 = reinterpret_cast<const float4*>(pred); q.bb = reinterpret_cast<uint2*>(W.pb); q.nb4 = (long)B * U1 * D / 4;
+      }
+      const int extra = (int)std::min<long>((q.n0 + q.na4 * 4 + q.nb4 * 4 + 1023) / 1024, 148L * 8);
+      prep_kernel<false><<<q.nW + B + extra, 256, 0, st>>>(q);
     }
-    const int extra = (int)std::min<long>((q.n0 + q.na4 * 4 + q.nb4 * 4 + 1023) / 1024, 148L * 8);
-    prep_kernel<false><<<q.nW + B + extra, 256, 0, st>>>(q);
     CTCVR_LAUNCH_CHECK();
   }
-  {
-    const int grid = min(sm_count(), mt);
-    CUtensorMap tmap_e, tmap_p;
-    if (make_tmap_bf16_2d(&tmap_e, W.eb, (uint64_t)B * T, D, D, G.TT)) return 1;
-    if (make_tmap_bf16_2d(&tmap_p, W.pb, (uint64_t)B * U1, D, D, G.P)) return 1;
-    BwdParams p{};
-    p.w_t = W.wb; p.wt_t = W.wtb;
-    p.bias_l2 = W.bias_l2; p.targets = targets; p.t_len = t_len; p.u_len = u_len;
-    p.tiles = W.tiles; p.ntiles = W.ntiles;
-    p.B = B; p.T = T; p.U1 = U1; p.D = D; p.V = V; p.Vp = Vp; p.NH = NH; p.blank = blank;
-    p.r1_stages = bwd3_r1_stages(NH, Vp);
-    p.lse = lse; p.lp_blank = lp_blank; p.lp_label = lp_label;
-    p.alpha = alpha; p.beta = beta; p.costs = costs; p.grad_costs = grad_costs; p.clamp = clamp;
-    p.gt = W.gt;
-    p.d_enc_part = W.d_enc_part; p.d_pred = d_pred_acc; p.d_bias = d_b;
-    p.prof = g_prof_buf;
-    tc_error_host_word(&p.err_host);
-    if (use_pair) {
-      CUtensorMap tmap_e2;                 // both tiles' frames in one box (P4 slab)
-      if (make_tmap_bf16_2d(&tmap_e2, W.eb, (uint64_t)B * T, D, D, 2 * G.TT)) return 1;
-      p.r1_stages = bwd4_r1_stages(NH, Vp);
-      const int gridp = std::max(2, std::min(sm_count() & ~1, mt & ~1));
-      if (G.P == 21) {
-        const auto k = pick_act(act, joint_bwd4_kernel<21, 6>, joint_bwd4_relu_kernel<21, 6>, joint_bwd4_gelu_kernel<21, 6>);
-        CTCVR_CHECK_CUDA(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_pair));
-        k<<<gridp, NTHREADS, smem_pair, st>>>(tmap_e, tmap_e2, tmap_p, p);
-      } else {
-        const auto k = pick_act(act, joint_bwd4_kernel<16, 8>, joint_bwd4_relu_kernel<16, 8>, joint_bwd4_gelu_kernel<16, 8>);
-        CTCVR_CHECK_CUDA(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_pair));
-        k<<<gridp, NTHREADS, smem_pair, st>>>(tmap_e, tmap_e2, tmap_p, p);
-      }
-      CTCVR_LAUNCH_CHECK();
-    } else {
-    const size_t smem = bwd3_smem_bytes(NH, Vp, D);
-    CTCVR_REQUIRE(smem <= 232448 && p.r1_stages >= 2, "joint_rnnt_bwd bf16: shared memory budget exceeded (%zu B)", smem);
-    if (G.P == 21) {
-      const auto k = pick_act(act, joint_bwd3_kernel<21, 6>, joint_bwd3_relu_kernel<21, 6>, joint_bwd3_gelu_kernel<21, 6>);
-      CTCVR_CHECK_CUDA(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-      k<<<grid, NTHREADS, smem, st>>>(tmap_e, tmap_p, p);
-      CTCVR_LAUNCH_CHECK();
-    } else {
-      const auto k = pick_act(act, joint_bwd3_kernel<16, 8>, joint_bwd3_relu_kernel<16, 8>, joint_bwd3_gelu_kernel<16, 8>);
-      CTCVR_CHECK_CUDA(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-      k<<<grid, NTHREADS, smem, st>>>(tmap_e, tmap_p, p);
-      CTCVR_LAUNCH_CHECK();
-    }
-    }
-  }
+  BwdParams p = bwd_params(W, enc, pred, targets, t_len, u_len, lse, lp_blank, lp_label, alpha, beta, costs, grad_costs,
+                           clamp, d_pred_acc, d_b, B, T, U1, D, V, blank, split != 0);
+  if (G.P == 21 ? launch_bwd_main<21, 6>(p, W, use_pair, split != 0, act, false, st)
+                : launch_bwd_main<16, 8>(p, W, use_pair, split != 0, act, false, st)) return 1;
   if (in_bf16)
     reduce_denc_kernel<true><<<B * T + B * U1, 128, 0, st>>>(W.d_enc_part, t_len, u_len, d_enc, B, T, U1, D, G.P, d_pred_acc, d_pred);
   else
     reduce_denc_kernel<false><<<B * T, 128, 0, st>>>(W.d_enc_part, t_len, u_len, d_enc, B, T, U1, D, G.P, nullptr, nullptr);
   CTCVR_LAUNCH_CHECK();
+  return G.P == 21 ? launch_bwd_dw<21, 6>(W, enc, pred, W.gt, W.gt_lo, d_w, B, T, U1, D, V, Vp, split != 0, act, st)
+                   : launch_bwd_dw<16, 8>(W, enc, pred, W.gt, W.gt_lo, d_w, B, T, U1, D, V, Vp, split != 0, act, st);
+}
+
+size_t joint_bwd_vt_ws_bytes(int B, int T, int U1, int D, int V, int split) {
+  if (!joint_tc_vt_supported(U1, D, V)) return 256;       // the call itself fails with the reason
+  const VocabTiles vt = vocab_tiles(V);
+  if (vt.n == 1) return joint_bwd_tc_ws_bytes(B, T, U1, D, V, split);
+  return carve_bwd_ws(nullptr, B, T, U1, D, vt.Vc, split != 0, vt.n).bytes;
+}
+
+// Vocabulary tiles (ctcvr_joint_rnnt_bwd_vt): one prep launch (every tile's weights, the tile table, the zero fills of
+// d_pred and d_bias), then per tile kernel 1 (d_pred / d_bias accumulate; d_enc partials stored by tile 0, added by the
+// others), kernel 2 and its reduction into the tile's rows of d_w; the d_enc reduction once at the end.  The G spill
+// and the dW partials are one tile's, reused by the next in stream order.  One tile is the untiled call.
+int joint_bwd_vt(const float* enc, const float* pred, int split, int act, const float* w, const float* bias,
+                 const int32_t* targets, const int32_t* t_len, const int32_t* u_len, const float* lse,
+                 const float* lp_blank, const float* lp_label, const float* alpha, const float* beta, const float* costs,
+                 const float* grad_costs, float clamp, float* d_enc, float* d_pred, float* d_w, float* d_b, int B, int T,
+                 int U1, int D, int V, int blank, void* ws, size_t ws_bytes, cudaStream_t st) {
+  const char* prec = split ? "bf16x3" : "bf16";
+  CTCVR_REQUIRE(joint_tc_vt_supported(U1, D, V), "joint_rnnt_bwd_vt: precision = %s needs D %% 128 == 0, D <= 512, V <= %d and U+1 <= 128 (got D=%d V=%d U+1=%d); use precision = fp32 for this shape", prec, VT_MAX_V, D, V, U1);
+  const VocabTiles vt = vocab_tiles(V);
+  if (vt.n == 1)
+    return joint_bwd_tc(enc, pred, 0, split, act, w, bias, targets, t_len, u_len, lse, lp_blank, lp_label, alpha, beta,
+                        costs, grad_costs, clamp, d_enc, d_pred, d_w, d_b, B, T, U1, D, V, blank, ws, ws_bytes, st);
+  if (check_tc_error("joint_rnnt_bwd_vt")) return 1;
+  CTCVR_REQUIRE(ws && ws_bytes >= joint_bwd_vt_ws_bytes(B, T, U1, D, V, split), "joint_rnnt_bwd_vt %s: workspace too small", prec);
+  CTCVR_REQUIRE(((uintptr_t)enc & 15) == 0 && ((uintptr_t)pred & 15) == 0, "joint_rnnt_bwd_vt %s: enc_proj / pred_proj must be 16-byte aligned", prec);
+  const int Vc = vt.Vc, KBG = (Vc + 63) / 64;
+  BwdWs W = carve_bwd_ws(ws, B, T, U1, D, Vc, split != 0, vt.n);
+  RectGeom G = pick_rect_geom(T, U1);
+  const bool use_pair = !split && bwd_use_pair(G, Vc / 2, Vc, D);
+  G.even = use_pair ? 1 : 0;
   {
-    CUtensorMap tmap_e, tmap_p;          // the same 64-wide SW128 boxes as kernel 1: TT enc rows / P pred rows
-    if (make_tmap_bf16_2d(&tmap_e, W.eb, (uint64_t)B * T, D, D, G.TT)) return 1;
-    if (make_tmap_bf16_2d(&tmap_p, W.pb, (uint64_t)B * U1, D, D, G.P)) return 1;
-    if (G.P == 21) {
-      const size_t smem = 1024 + (size_t)DW_STAGES * ((size_t)KBG * 8192) + DWR_S_STAGES * dwr_slab_bytes<21>() + 256;
-      CTCVR_REQUIRE(smem <= 232448, "dW GEMM: shared memory budget exceeded (%zu B)", smem);
-      const auto k = pick_act(act, dw_gemm_rz_kernel<21, 6>, dw_gemm_rz_relu_kernel<21, 6>, dw_gemm_rz_gelu_kernel<21, 6>);
-      CTCVR_CHECK_CUDA(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-      k<<<dim3(MB, W.KS), DWR_THREADS, smem, st>>>(tmap_e, tmap_p, W.gt, W.tile_rows, W.ntiles, W.partials, D, Vp, KBG, W.KS);
-    } else {
-      const size_t smem = 1024 + (size_t)DW_STAGES * ((size_t)KBG * 8192) + DWR_S_STAGES * dwr_slab_bytes<16>() + 256;
-      CTCVR_REQUIRE(smem <= 232448, "dW GEMM: shared memory budget exceeded (%zu B)", smem);
-      const auto k = pick_act(act, dw_gemm_rz_kernel<16, 8>, dw_gemm_rz_relu_kernel<16, 8>, dw_gemm_rz_gelu_kernel<16, 8>);
-      CTCVR_CHECK_CUDA(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-      k<<<dim3(MB, W.KS), DWR_THREADS, smem, st>>>(tmap_e, tmap_p, W.gt, W.tile_rows, W.ntiles, W.partials, D, Vp, KBG, W.KS);
+    PrepArgs q{};
+    q.w = w; q.bias = bias; q.w_t = W.wb; q.wt_t = W.wtb; q.bias_l2 = W.bias_l2;
+    q.V = V; q.Vp = Vc; q.D = D; q.nW = cdiv((long)KBG * 64 * D, 256);
+    q.t_len = t_len; q.u_len = u_len; q.B = B; q.T = T; q.U1 = U1; q.geom = G.P | (G.TT << 8) | (G.even << 16);
+    q.max_tiles = W.mt; q.tiles = W.tiles; q.tile_rows = W.tile_rows; q.ntiles = W.ntiles;
+    q.zero0 = d_pred; q.n0 = (long)B * U1 * D; q.zero1 = d_b; q.n1 = V;
+    if (!split) {
+      q.a = reinterpret_cast<const float4*>(enc); q.ab = reinterpret_cast<uint2*>(W.eb); q.na4 = (long)B * T * D / 4;
+      q.b4 = reinterpret_cast<const float4*>(pred); q.bb = reinterpret_cast<uint2*>(W.pb); q.nb4 = (long)B * U1 * D / 4;
     }
+    const int extra = (int)std::min<long>((q.n0 + q.na4 * 4 + q.nb4 * 4 + 1023) / 1024, 148L * 8);
+    if (split) prep_vt_kernel<true><<<q.nW * vt.n + B + extra, 256, 0, st>>>(q, vt.n);
+    else prep_vt_kernel<false><<<q.nW * vt.n + B + extra, 256, 0, st>>>(q, vt.n);
     CTCVR_LAUNCH_CHECK();
   }
-  reduce_dw_kernel<<<dim3(cdiv(D, 8), cdiv(Vp, 32)), 256, 0, st>>>(W.partials, d_w, D, V, Vp, W.KS);
+  const size_t wstride = (size_t)Vc * D * (split ? 2 : 1), wtstride = (size_t)KBG * 64 * D * (split ? 2 : 1);
+  for (int c = 0; c < vt.n; ++c) {
+    const int v0 = c * Vc, Vr = std::min(V - v0, Vc);
+    BwdParams p = bwd_params(W, enc, pred, targets, t_len, u_len, lse, lp_blank, lp_label, alpha, beta, costs, grad_costs,
+                             clamp, d_pred, d_b + v0, B, T, U1, D, Vr, (blank >= v0 && blank < v0 + Vr) ? blank - v0 : -1,
+                             split != 0);
+    p.w_t = W.wb + c * wstride; p.wt_t = W.wtb + c * wtstride; p.bias_l2 = W.bias_l2 + (size_t)c * Vc;
+    p.Vp = Vc; p.NH = Vc / 2;                 // the tile's padded width (pad_v(Vr) may be smaller in the last tile)
+    p.v0 = v0; p.Vg = V; p.blank_g = blank; p.accum = c > 0;
+    if (G.P == 21 ? launch_bwd_main<21, 6>(p, W, use_pair, split != 0, act, true, st)
+                  : launch_bwd_main<16, 8>(p, W, use_pair, split != 0, act, true, st)) return 1;
+    float* dw = d_w + (size_t)v0 * D;
+    if (G.P == 21 ? launch_bwd_dw<21, 6>(W, enc, pred, W.gt, W.gt_lo, dw, B, T, U1, D, Vr, Vc, split != 0, act, st)
+                  : launch_bwd_dw<16, 8>(W, enc, pred, W.gt, W.gt_lo, dw, B, T, U1, D, Vr, Vc, split != 0, act, st)) return 1;
+  }
+  reduce_denc_kernel<false><<<B * T, 128, 0, st>>>(W.d_enc_part, t_len, u_len, d_enc, B, T, U1, D, G.P, nullptr, nullptr);
   CTCVR_LAUNCH_CHECK();
   return 0;
 }

@@ -102,6 +102,10 @@ struct BwdParams {
   const float* enc;
   const float* pred;
   __nv_bfloat16* gt_lo;
+  // vocabulary tiles (VT kernels only): this launch covers columns [v0, v0 + V) of a vocabulary of Vg entries whose
+  // blank is blank_g; w_t / wt_t / bias_l2 / gt / d_bias are the tile's, blank is the tile's blank column or -1, and
+  // lse is the full vocabulary's.  accum: add to d_enc_part (an earlier tile stored it) instead of storing.
+  int v0, Vg, blank_g, accum;
 };
 
 // Shared memory: [weight ring: 4 W^T stages][G tile (P2/P3)]  -- P1 views both as one W ring --
@@ -256,7 +260,9 @@ __device__ __forceinline__ void p4_chunk(const float (&w)[16], const float (&e)[
 //   d_bias = column sums of G_hi plus column sums of G_lo (after the reload)
 // Shared memory: the bf16 layout without the two slab regions (P1 ring / P4 slab).
 // ACT: the joint activation of the P1 producers and the P4 derivative (ACT_TANH / ACT_RELU / ACT_GELU).
-template <int P, int TT, bool SPLIT, int ACT = ACT_TANH>
+// VT: one vocabulary tile of a larger vocabulary (BwdParams v0 ..): labels are mapped to the tile's columns, and only
+// the columns it holds are patched.
+template <int P, int TT, bool SPLIT, int ACT = ACT_TANH, bool VT = false>
 __device__ __forceinline__ void joint_bwd3_body(const CUtensorMap& tmap_e, const CUtensorMap& tmap_p, const BwdParams& p) {
   extern __shared__ uint8_t smem_raw[];
   Bwd3Smem L;
@@ -669,7 +675,8 @@ __device__ __forceinline__ void joint_bwd3_body(const CUtensorMap& tmap_e, const
           bl1 = p.beta[cell + 1];
           lpl = p.lp_label[cell];
           lab = p.targets[(size_t)g.b * (p.U1 - 1) + u];
-          if ((unsigned)lab >= (unsigned)p.V) lab = p.blank;      // out-of-range ids cannot index outside the tile
+          if (VT) lab = vt_column(lab, p.Vg, p.blank_g, p.v0, p.V);
+          else if ((unsigned)lab >= (unsigned)p.V) lab = p.blank;      // out-of-range ids cannot index outside the tile
         }
         scale = p.grad_costs[g.b];
       }
@@ -770,7 +777,7 @@ __device__ __forceinline__ void joint_bwd3_body(const CUtensorMap& tmap_e, const
             p.gt_lo[(((size_t)ti.w * 2 + (r >> 6)) * KBG + (col >> 6)) * 4096 + (r & 63) * 64 +
                     ((((col & 63) >> 3) ^ (r & 7)) << 3) + (col & 7)] = __float2bfloat16(val - __bfloat162float(hb));
         };
-        if (((p.blank >> 4) % 3) == wg) put(p.blank, entry(lpb, bnext, (lab == p.blank) ? bl1 : kNegInf));
+        if ((!VT || p.blank >= 0) && ((p.blank >> 4) % 3) == wg) put(p.blank, entry(lpb, bnext, (lab == p.blank) ? bl1 : kNegInf));
         if (lab >= 0 && lab != p.blank && ((lab >> 4) % 3) == wg) put(lab, entry(lpl, bl1, kNegInf));
       }
       fence_proxy_async();
@@ -884,7 +891,10 @@ __device__ __forceinline__ void joint_bwd3_body(const CUtensorMap& tmap_e, const
 #pragma unroll
             for (int i = 0; i < TT; ++i) {
               const int tt = g.t0 + i;
-              if (tt < g.Tb) p.d_enc_part[(((size_t)ti.y * p.B + g.b) * p.T + tt) * p.D + d] = es[i];
+              if (tt < g.Tb) {
+                float& o = p.d_enc_part[(((size_t)ti.y * p.B + g.b) * p.T + tt) * p.D + d];
+                if (VT && p.accum) o += es[i]; else o = es[i];
+              }
             }
           }
         }
@@ -932,6 +942,20 @@ CTCVR_BWD3_ACT(joint_bwd3_gelu_kernel, false, ACT_GELU)
 CTCVR_BWD3_ACT(joint_bwd3_x3_relu_kernel, true, ACT_RELU)
 CTCVR_BWD3_ACT(joint_bwd3_x3_gelu_kernel, true, ACT_GELU)
 #undef CTCVR_BWD3_ACT
+// vocabulary tiles (ctcvr_joint_rnnt_bwd_vt): one launch per tile of the vocabulary
+#define CTCVR_BWD3_VT(name, split, act)                                                                            \
+  template <int P, int TT>                                                                                          \
+  __global__ void __launch_bounds__(NTHREADS, 1)                                                                    \
+  name(const __grid_constant__ CUtensorMap tmap_e, const __grid_constant__ CUtensorMap tmap_p, const BwdParams p) { \
+    joint_bwd3_body<P, TT, split, act, true>(tmap_e, tmap_p, p);                                                    \
+  }
+CTCVR_BWD3_VT(joint_bwd3_vt_kernel, false, ACT_TANH)
+CTCVR_BWD3_VT(joint_bwd3_vt_relu_kernel, false, ACT_RELU)
+CTCVR_BWD3_VT(joint_bwd3_vt_gelu_kernel, false, ACT_GELU)
+CTCVR_BWD3_VT(joint_bwd3_x3_vt_kernel, true, ACT_TANH)
+CTCVR_BWD3_VT(joint_bwd3_x3_vt_relu_kernel, true, ACT_RELU)
+CTCVR_BWD3_VT(joint_bwd3_x3_vt_gelu_kernel, true, ACT_GELU)
+#undef CTCVR_BWD3_VT
 
 }  // namespace tc
 }  // namespace ctcvr

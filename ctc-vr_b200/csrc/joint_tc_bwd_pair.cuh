@@ -88,7 +88,8 @@ __device__ __forceinline__ void carve_bwd4(Bwd4Smem& L, uint8_t* raw, int NH, in
 }
 
 // ACT: the joint activation of the P1 producers and the P4 derivative (ACT_TANH / ACT_RELU / ACT_GELU)
-template <int P, int TT, int ACT>
+// VT: one vocabulary tile of a larger vocabulary, as in joint_bwd3_body
+template <int P, int TT, int ACT, bool VT = false>
 __device__ __forceinline__ void joint_bwd4_body(const CUtensorMap& tmap_e, const CUtensorMap& tmap_e2,
                                                 const CUtensorMap& tmap_p, const BwdParams& p) {
   static_assert(2 * TT * 128 <= (int)BP_ENC_REGION, "the enc rows of both tiles share one 2 KB region");
@@ -433,7 +434,8 @@ __device__ __forceinline__ void joint_bwd4_body(const CUtensorMap& tmap_e, const
           bl1 = p.beta[cell + 1];
           lpl = p.lp_label[cell];
           lab = p.targets[(size_t)g.b * (p.U1 - 1) + u];
-          if ((unsigned)lab >= (unsigned)p.V) lab = p.blank;      // out-of-range ids cannot index outside the tile
+          if (VT) lab = vt_column(lab, p.Vg, p.blank_g, p.v0, p.V);
+          else if ((unsigned)lab >= (unsigned)p.V) lab = p.blank;      // out-of-range ids cannot index outside the tile
         }
         scale = p.grad_costs[g.b];
       }
@@ -504,7 +506,7 @@ __device__ __forceinline__ void joint_bwd4_body(const CUtensorMap& tmap_e, const
           const uint32_t a = L.g_kblock(col >> 6) + r * 128 + ((((col & 63) >> 3) ^ (r & 7)) << 4) + (col & 7) * 2;
           asm volatile("st.shared.u16 [%0], %1;" ::"r"(a), "h"(h) : "memory");
         };
-        if (((p.blank >> 4) % 3) == wg) put(p.blank, entry(lpb, bnext, (lab == p.blank) ? bl1 : kNegInf));
+        if ((!VT || p.blank >= 0) && ((p.blank >> 4) % 3) == wg) put(p.blank, entry(lpb, bnext, (lab == p.blank) ? bl1 : kNegInf));
         if (lab >= 0 && lab != p.blank && ((lab >> 4) % 3) == wg) put(lab, entry(lpl, bl1, kNegInf));
       }
       fence_proxy_async();
@@ -603,7 +605,10 @@ __device__ __forceinline__ void joint_bwd4_body(const CUtensorMap& tmap_e, const
 #pragma unroll
             for (int i = 0; i < TT; ++i) {
               const int tt = zt * TT + i;
-              if (tt < g.Tb) p.d_enc_part[(((size_t)ti.y * p.B + g.b) * p.T + tt) * p.D + d] = es[i];
+              if (tt < g.Tb) {
+                float& o = p.d_enc_part[(((size_t)ti.y * p.B + g.b) * p.T + tt) * p.D + d];
+                if (VT && p.accum) o += es[i]; else o = es[i];
+              }
             }
           }
         }
@@ -627,16 +632,19 @@ __device__ __forceinline__ void joint_bwd4_body(const CUtensorMap& tmap_e, const
   if (warp == 2) tmem_dealloc2(tmem_base, TMEM_COLS);
 }
 
-#define CTCVR_BWD4(name, act)                                                                                      \
+#define CTCVR_BWD4(name, act, vt)                                                                                  \
   template <int P, int TT>                                                                                          \
   __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NTHREADS, 1)                                          \
   name(const __grid_constant__ CUtensorMap tmap_e, const __grid_constant__ CUtensorMap tmap_e2,                     \
        const __grid_constant__ CUtensorMap tmap_p, const BwdParams p) {                                             \
-    joint_bwd4_body<P, TT, act>(tmap_e, tmap_e2, tmap_p, p);                                                        \
+    joint_bwd4_body<P, TT, act, vt>(tmap_e, tmap_e2, tmap_p, p);                                                    \
   }
-CTCVR_BWD4(joint_bwd4_kernel, ACT_TANH)
-CTCVR_BWD4(joint_bwd4_relu_kernel, ACT_RELU)     // relu / gelu joints, named apart for profiler traces
-CTCVR_BWD4(joint_bwd4_gelu_kernel, ACT_GELU)
+CTCVR_BWD4(joint_bwd4_kernel, ACT_TANH, false)
+CTCVR_BWD4(joint_bwd4_relu_kernel, ACT_RELU, false)     // relu / gelu joints, named apart for profiler traces
+CTCVR_BWD4(joint_bwd4_gelu_kernel, ACT_GELU, false)
+CTCVR_BWD4(joint_bwd4_vt_kernel, ACT_TANH, true)         // vocabulary tiles (ctcvr_joint_rnnt_bwd_vt)
+CTCVR_BWD4(joint_bwd4_vt_relu_kernel, ACT_RELU, true)
+CTCVR_BWD4(joint_bwd4_vt_gelu_kernel, ACT_GELU, true)
 #undef CTCVR_BWD4
 
 }  // namespace tc

@@ -54,7 +54,25 @@ struct FwdParams {
   unsigned int* err_host;   // mapped host word for bounded-wait time-outs (tc_common.cuh)
   const float* enc;         // bf16x3 only: the fp32 activations [B,T,D] / [B,U1,D], read in place
   const float* pred;
+  // vocabulary tiles (VT kernels only): this launch covers columns [v0, v0 + V) of a vocabulary of Vg entries whose
+  // blank is blank_g; bias / w_t / bias_l2 are the tile's, blank is the tile's blank column or -1.  merge: lse holds
+  // the log-sum-exp of the earlier tiles (merged in place); lp_blank / lp_label receive raw logit + bias.
+  int v0, Vg, blank_g, merge;
 };
+
+// vocabulary tiles: a label of the full vocabulary -> its column in the tile [v0, v0 + Vc), -1 when another tile holds
+// it.  Ids outside [0, Vg) act as the blank, as in the untiled kernels.
+__device__ __forceinline__ int vt_column(int lab, int Vg, int blank_g, int v0, int Vc) {
+  if ((unsigned)lab >= (unsigned)Vg) lab = blank_g;
+  lab -= v0;
+  return ((unsigned)lab < (unsigned)Vc) ? lab : -1;
+}
+
+// log(exp(a) + exp(b)) in fp32 (accurate functions: once per cell and tile)
+__device__ __forceinline__ float logaddexp_f32(float a, float b) {
+  const float m = fmaxf(a, b);
+  return (m == kNegInf) ? m : m + log1pf(expf(-fabsf(a - b)));
+}
 
 struct FwdSmem {
   uint32_t a_base, w_base, w_bytes, s_base, bar_base;
@@ -121,7 +139,9 @@ __device__ __forceinline__ void tanh_split8(const float4& e0, const float4& e1, 
 //   A stages : per k-block two TMEM stages (z_hi, z_lo of its 64 k): the same 3 x 32 columns as bf16
 //   producers: read the fp32 enc / pred rows straight from global memory (L2-resident), no slab ring (warp 3 idles)
 // ACT: the joint activation (ACT_TANH / ACT_RELU / ACT_GELU), applied by the A producers.
-template <bool SPLIT, int ACT = ACT_TANH>
+// VT: one vocabulary tile of a larger vocabulary (FwdParams v0 ..): the epilogue merges the tile's log-sum-exp into lse
+// and writes the raw blank / label logits of the columns it holds; vt_finalize_kernel subtracts the final lse.
+template <bool SPLIT, int ACT = ACT_TANH, bool VT = false>
 __device__ __forceinline__ void joint_fwd2_body(const CUtensorMap& tmap_e, const CUtensorMap& tmap_p, const FwdParams& p) {
   extern __shared__ uint8_t smem_raw[];
   FwdSmem L;
@@ -264,7 +284,7 @@ __device__ __forceinline__ void joint_fwd2_body(const CUtensorMap& tmap_e, const
     const uint32_t tq = tmem_base + ((uint32_t)(q * 32) << 16);
     uint32_t tphase = 0;
     int prof_n = 0;
-    const float bias_blank = __ldg(p.bias + p.blank);
+    const float bias_blank = (VT && p.blank < 0) ? 0.f : __ldg(p.bias + p.blank);
     // column chunks of 16, dealt to the groups in contiguous runs
     const int nch = p.Vp / 16;
     const int c_begin = (nch * eg / F_EPI_GROUPS) * 16, c_end = (nch * (eg + 1) / F_EPI_GROUPS) * 16;
@@ -282,15 +302,16 @@ __device__ __forceinline__ void joint_fwd2_body(const CUtensorMap& tmap_e, const
       float bias_lab = 0.f;
       if (eg == 0 && u < Ub) {
         lab = p.targets[(size_t)b * (p.U1 - 1) + u];
-        if ((unsigned)lab >= (unsigned)p.V) lab = p.blank;    // out-of-range ids cannot index outside the tile
-        bias_lab = __ldg(p.bias + lab);
+        if (VT) lab = vt_column(lab, p.Vg, p.blank_g, p.v0, p.V);
+        else if ((unsigned)lab >= (unsigned)p.V) lab = p.blank;    // out-of-range ids cannot index outside the tile
+        if (!VT || lab >= 0) bias_lab = __ldg(p.bias + lab);
       }
       pin(lab);
       mbar_wait(L.tmem_full(), tphase, 6);
       if (tid == 128) TC_PROF(2, 1);
       tc_fence_after();
       float xb = 0.f, xl = 0.f;
-      if (eg == 0) { xb = tmem_ld1(tq + p.blank); xl = tmem_ld1(tq + (lab >= 0 ? lab : 0)); }
+      if (eg == 0) { xb = tmem_ld1(tq + (VT ? max(p.blank, 0) : p.blank)); xl = tmem_ld1(tq + (lab >= 0 ? lab : 0)); }
       float m = kNegInf, s = 0.f;
       float v[16];
       if (c_begin < c_end) tmem_ld16(tq + c_begin, v);
@@ -339,9 +360,15 @@ __device__ __forceinline__ void joint_fwd2_body(const CUtensorMap& tmap_e, const
         if (valid) {
           const size_t cell = ((size_t)b * p.T + t) * p.U1 + u;
           const float l = (m + lg2_fast(s)) * LN2;
-          p.lse[cell] = l;
-          p.lp_blank[cell] = xb + bias_blank - l;
-          p.lp_label[cell] = (lab >= 0) ? xl + bias_lab - l : kNegInf;
+          if constexpr (VT) {
+            p.lse[cell] = p.merge ? logaddexp_f32(p.lse[cell], l) : l;
+            if (p.blank >= 0) p.lp_blank[cell] = xb + bias_blank;
+            if (lab >= 0) p.lp_label[cell] = xl + bias_lab;
+          } else {
+            p.lse[cell] = l;
+            p.lp_blank[cell] = xb + bias_blank - l;
+            p.lp_label[cell] = (lab >= 0) ? xl + bias_lab - l : kNegInf;
+          }
         }
       }
       named_barrier_sync(3, F_EPI_WARPS * 32);             // partials consumed before the next tile overwrites them
@@ -461,6 +488,19 @@ CTCVR_FWD2_ACT(joint_fwd2_gelu_kernel, false, ACT_GELU)
 CTCVR_FWD2_ACT(joint_fwd2_x3_relu_kernel, true, ACT_RELU)
 CTCVR_FWD2_ACT(joint_fwd2_x3_gelu_kernel, true, ACT_GELU)
 #undef CTCVR_FWD2_ACT
+// vocabulary tiles (ctcvr_joint_rnnt_fwd_vt): one launch per tile of the vocabulary
+#define CTCVR_FWD2_VT(name, split, act)                                                                            \
+  __global__ void __launch_bounds__(F_THREADS, 1)                                                                   \
+  name(const __grid_constant__ CUtensorMap tmap_e, const __grid_constant__ CUtensorMap tmap_p, const FwdParams p) { \
+    joint_fwd2_body<split, act, true>(tmap_e, tmap_p, p);                                                           \
+  }
+CTCVR_FWD2_VT(joint_fwd2_vt_kernel, false, ACT_TANH)
+CTCVR_FWD2_VT(joint_fwd2_vt_relu_kernel, false, ACT_RELU)
+CTCVR_FWD2_VT(joint_fwd2_vt_gelu_kernel, false, ACT_GELU)
+CTCVR_FWD2_VT(joint_fwd2_x3_vt_kernel, true, ACT_TANH)
+CTCVR_FWD2_VT(joint_fwd2_x3_vt_relu_kernel, true, ACT_RELU)
+CTCVR_FWD2_VT(joint_fwd2_x3_vt_gelu_kernel, true, ACT_GELU)
+#undef CTCVR_FWD2_VT
 
 // Tile table of the forward kernel: per utterance (W/4) groups of 4 label columns x 32-frame blocks, then a
 // 2-column group x 64-frame blocks if W & 2, then a 1-column group x 128-frame blocks if W & 1 (64-frame blocks for

@@ -41,11 +41,17 @@ def _ws(nbytes, device):
     return torch.empty(max(int(nbytes), 256), dtype=torch.uint8, device=device)
 
 
+def _vocab_tiled(precision, V, vocab_tiling):
+    """Whether a call takes the vocabulary-tile entry points (`ctcvr_joint_rnnt_*_vt`): only a tensor-core precision
+    with vocab_tiling=True and pad32(V) > 416.  Every other call keeps its entry points and kernels."""
+    return bool(vocab_tiling) and precision in (BF16, BF16X3) and (V + 31) // 32 * 32 > 416
+
+
 def _joint_fwd(enc_proj, pred_proj, w_out, b_out, targets, t_len, u_len, blank, precision, act,
-               op="fused_joint_rnnt_loss"):
-    """The fused joint forward (`ctcvr_joint_rnnt_fwd` / `_bf16in`) with the fused loss's input handling and errors.
-    Returns the kernel inputs (e, p, w, b, tg, tl, ul), whether the bf16-input entry point ran, and lse / lp_blank /
-    lp_label [B,T,U1]."""
+               op="fused_joint_rnnt_loss", vocab_tiling=False):
+    """The fused joint forward (`ctcvr_joint_rnnt_fwd` / `_bf16in` / `_vt`) with the fused loss's input handling and
+    errors.  Returns the kernel inputs (e, p, w, b, tg, tl, ul), whether the bf16-input entry point ran, and lse /
+    lp_blank / lp_label [B,T,U1]."""
     _lib.require_cuda(enc_proj, pred_proj, w_out, b_out)
     dev = enc_proj.device
     w, b = _f32c(w_out), _f32c(b_out)
@@ -55,8 +61,9 @@ def _joint_fwd(enc_proj, pred_proj, w_out, b_out, targets, t_len, u_len, blank, 
     # bf16 activations (autocast) are consumed in place by the tensor-core path: no fp32 round trip.  The bf16-input
     # entry points are tanh only; other joints pass bf16 inputs through the fp32-input entry point, whose bf16 path
     # rounds them to bf16 again (exact), so the arithmetic is the same.
+    tiled = _vocab_tiled(precision, V, vocab_tiling)
     bf16_in = precision == BF16 and act == ACT_TANH and enc_proj.dtype == torch.bfloat16 and \
-        pred_proj.dtype == torch.bfloat16
+        pred_proj.dtype == torch.bfloat16 and not tiled
     if bf16_in:
         e, p = enc_proj.detach().contiguous(), pred_proj.detach().contiguous()
     else:
@@ -73,27 +80,36 @@ def _joint_fwd(enc_proj, pred_proj, w_out, b_out, targets, t_len, u_len, blank, 
         raise RuntimeError(f"{op}: blank must be within [0, vocab)")
     # Length / label VALUES are not read back (that would be a host sync in the training step): the kernels clamp
     # lengths to the tensor extents and treat a label outside [0, V) as blank, so bad values cannot fault the GPU.
-    if precision in (BF16, BF16X3) and not bool(query("ctcvr_joint_tc_supported", U1, D, V)):
+    if tiled and not bool(query("ctcvr_joint_tc_vt_supported", U1, D, V)):
+        raise RuntimeError(f"{op}: precision='{_PREC_NAME[precision]}' with vocab_tiling=True needs D % 128 == 0, "
+                           f"D <= 512, V <= 32768 and U+1 <= 128 (got D={D}, V={V}, U+1={U1}); use precision='fp32' "
+                           "for this shape")
+    if precision in (BF16, BF16X3) and not tiled and not bool(query("ctcvr_joint_tc_supported", U1, D, V)):
+        more = ", or vocab_tiling=True for V > 416" if D % 128 == 0 and D <= 512 and U1 <= 128 else ""
         raise RuntimeError(f"{op}: precision='{_PREC_NAME[precision]}' needs D % 128 == 0, D <= 512, "
-                           f"V <= 416 and U+1 <= 128 (got D={D}, V={V}, U+1={U1}); use precision='fp32' for this shape")
+                           f"V <= 416 and U+1 <= 128 (got D={D}, V={V}, U+1={U1}); use precision='fp32' for this "
+                           f"shape{more}")
     lse = torch.empty((B, T, U1), dtype=torch.float32, device=dev)
     lpb, lpl = torch.empty_like(lse), torch.empty_like(lse)
     with torch.cuda.device(dev):
-        ws = _ws(query("ctcvr_joint_rnnt_fwd_ws_bytes", B, T, U1, D, V, precision | act), dev)
+        vt = "_vt" if tiled else ""
+        ws = _ws(query(f"ctcvr_joint_rnnt_fwd{vt}_ws_bytes", B, T, U1, D, V, precision | act), dev)
         if bf16_in:
             call("ctcvr_joint_rnnt_fwd_bf16in", ptr(e), ptr(p), ptr(w), ptr(b), ptr(tg), ptr(tl), ptr(ul), ptr(lse),
                  ptr(lpb), ptr(lpl), B, T, U1, D, V, blank, ptr(ws), ws.numel(), stream())
         else:
-            call("ctcvr_joint_rnnt_fwd", ptr(e), ptr(p), ptr(w), ptr(b), ptr(tg), ptr(tl), ptr(ul), ptr(lse),
+            call(f"ctcvr_joint_rnnt_fwd{vt}", ptr(e), ptr(p), ptr(w), ptr(b), ptr(tg), ptr(tl), ptr(ul), ptr(lse),
                  ptr(lpb), ptr(lpl), B, T, U1, D, V, blank, precision | act, ptr(ws), ws.numel(), stream())
     return (e, p, w, b, tg, tl, ul), bf16_in, lse, lpb, lpl
 
 
 class _FusedJointRnnt(torch.autograd.Function):
     @staticmethod
-    def forward(ctx, enc_proj, pred_proj, w_out, b_out, targets, t_len, u_len, blank, clamp, precision, act):
+    def forward(ctx, enc_proj, pred_proj, w_out, b_out, targets, t_len, u_len, blank, clamp, precision, act,
+                vocab_tiling=False):
         (e, p, w, b, tg, tl, ul), bf16_in, lse, lpb, lpl = _joint_fwd(enc_proj, pred_proj, w_out, b_out, targets, t_len,
-                                                                      u_len, blank, precision, act)
+                                                                      u_len, blank, precision, act,
+                                                                      vocab_tiling=vocab_tiling)
         B, T, U1 = lse.shape
         alpha, beta = torch.empty_like(lse), torch.empty_like(lse)
         costs = torch.empty((B,), dtype=torch.float32, device=lse.device)
@@ -101,13 +117,14 @@ class _FusedJointRnnt(torch.autograd.Function):
             call("ctcvr_rnnt_lattice", ptr(lpb), ptr(lpl), ptr(tl), ptr(ul), ptr(alpha), ptr(beta), ptr(costs),
                  B, T, U1, stream())
         ctx.save_for_backward(e, p, w, b, tg, tl, ul, lse, lpb, lpl, alpha, beta, costs)
-        ctx.cfg = (blank, float(clamp), precision, bf16_in, act, enc_proj.dtype, pred_proj.dtype)
+        ctx.cfg = (blank, float(clamp), precision, bf16_in, act, enc_proj.dtype, pred_proj.dtype,
+                   _vocab_tiled(precision, w.shape[0], vocab_tiling))
         return costs
 
     @staticmethod
     def backward(ctx, grad_costs):
         e, p, w, b, tg, tl, ul, lse, lpb, lpl, alpha, beta, costs = ctx.saved_tensors
-        blank, clamp, precision, bf16_in, act, e_dtype, p_dtype = ctx.cfg
+        blank, clamp, precision, bf16_in, act, e_dtype, p_dtype, tiled = ctx.cfg
         B, T, D = e.shape
         U1, V = p.shape[1], w.shape[0]
         dev = e.device
@@ -118,23 +135,24 @@ class _FusedJointRnnt(torch.autograd.Function):
         d_p = torch.empty(p.shape, dtype=gdt, device=dev)
         d_w, d_b = torch.empty_like(w), torch.empty_like(b)
         with torch.cuda.device(dev):
-            ws = _ws(query("ctcvr_joint_rnnt_bwd_ws_bytes", B, T, U1, D, V, precision | act), dev)
+            vt = "_vt" if tiled else ""
+            ws = _ws(query(f"ctcvr_joint_rnnt_bwd{vt}_ws_bytes", B, T, U1, D, V, precision | act), dev)
             if bf16_in:
                 call("ctcvr_joint_rnnt_bwd_bf16in", ptr(e), ptr(p), ptr(w), ptr(b), ptr(tg), ptr(tl), ptr(ul), ptr(lse),
                      ptr(lpb), ptr(lpl), ptr(alpha), ptr(beta), ptr(costs), ptr(gc), clamp, ptr(d_e), ptr(d_p), ptr(d_w), ptr(d_b),
                      B, T, U1, D, V, blank, ptr(ws), ws.numel(), stream())
             else:
-                call("ctcvr_joint_rnnt_bwd", ptr(e), ptr(p), ptr(w), ptr(b), ptr(tg), ptr(tl), ptr(ul), ptr(lse),
+                call(f"ctcvr_joint_rnnt_bwd{vt}", ptr(e), ptr(p), ptr(w), ptr(b), ptr(tg), ptr(tl), ptr(ul), ptr(lse),
                      ptr(lpb), ptr(lpl), ptr(alpha), ptr(beta), ptr(costs), ptr(gc), clamp, ptr(d_e), ptr(d_p), ptr(d_w), ptr(d_b),
                      B, T, U1, D, V, blank, precision | act, ptr(ws), ws.numel(), stream())
         if not bf16_in:                                   # gradients in the dtype of the inputs
             d_e, d_p = d_e.to(e_dtype), d_p.to(p_dtype)
-        return d_e, d_p, d_w, d_b, None, None, None, None, None, None, None
+        return d_e, d_p, d_w, d_b, None, None, None, None, None, None, None, None
 
 
 def fused_joint_rnnt_loss(enc_proj, pred_proj, w_out, b_out, targets, logit_lengths, target_lengths,
                           blank: int, clamp: float = -1.0, reduction: str = "mean", precision="fp32",
-                          activation: str = "tanh"):
+                          activation: str = "tanh", vocab_tiling: bool = False):
     """costs_b = RNN-T negative log-likelihood of utterance b for
     logits = ffn_out(act(enc_proj[:, :, None] + pred_proj[:, None])) without materialising them.
     enc_proj [B,T,D] / pred_proj [B,U+1,D] are the enc_ffn / pred_ffn outputs (joint.py:54-55).
@@ -155,11 +173,18 @@ def fused_joint_rnnt_loss(enc_proj, pred_proj, w_out, b_out, targets, logit_leng
     precision='bf16x3' runs the same tcgen05 tiling at fp32 accuracy: every fp32 GEMM operand is split into
     hi = bf16(x) and lo = bf16(x - hi) and each product is hi*hi + hi*lo + lo*hi, with tanh, d cost / d logits and the
     reductions in fp32.  Loss and gradients are within 1e-4 of the reference, like fp32; inputs are taken as fp32, and
-    the shape limits and the error on other shapes are those of 'bf16'."""
+    the shape limits and the error on other shapes are those of 'bf16'.
+
+    vocab_tiling=True lets 'bf16' and 'bf16x3' take vocabularies up to 32768 (D % 128 == 0, D <= 512 and U+1 <= 128
+    still hold): where pad32(V) > 416 the softmax runs over vocabulary tiles of at most 416 columns, each through the
+    tensor-core kernels, with a running log-sum-exp; the logits still never reach HBM.  The bars are those above:
+    'bf16' 2e-3 per cost (or 1e-3 nats per lattice step) and 3e-2 rel-L2 on the gradients, 'bf16x3' 1e-4.  Where
+    pad32(V) <= 416 it changes nothing (the same kernels run), and with 'fp32', which takes every V, it has no effect,
+    so a model can set it once whatever its precision.  Without it, V > 416 raises on the tensor-core precisions."""
     if activation not in _ACT:
         raise ValueError(f"fused_joint_rnnt_loss: activation must be one of {sorted(_ACT)}, got {activation!r}")
     costs = _FusedJointRnnt.apply(enc_proj, pred_proj, w_out, b_out, targets, logit_lengths, target_lengths,
-                                  int(blank), float(clamp), _PREC[precision], _ACT[activation])
+                                  int(blank), float(clamp), _PREC[precision], _ACT[activation], bool(vocab_tiling))
     return _reduce(costs, reduction)
 
 
@@ -510,16 +535,17 @@ def rnnt_viterbi(lp_blank, lp_label, logit_lengths, target_lengths):
 
 @torch.no_grad()
 def rnnt_forced_align(enc_proj, pred_proj, w_out, b_out, targets, logit_lengths, target_lengths, blank: int,
-                      precision="fp32", activation: str = "tanh"):
+                      precision="fp32", activation: str = "tanh", vocab_tiling: bool = False):
     """Forced alignment of `targets` [B,U] through the fused joint: the forward of `fused_joint_rnnt_loss` (same inputs,
-    precisions, activations and errors; the logits never reach HBM) followed by `rnnt_viterbi` on its log-probs.
+    precisions, activations, vocab_tiling and errors; the logits never reach HBM) followed by `rnnt_viterbi` on its log-probs.
     Returns (frames [B,U] int32, token_logprobs [B,U] fp32, scores [B] fp32) as `rnnt_viterbi`; scores <= -cost of the
     loss on the same inputs (one path against the sum over all of them)."""
     if activation not in _ACT:
         raise ValueError(f"rnnt_forced_align: activation must be one of {sorted(_ACT)}, got {activation!r}")
     (_, _, _, _, _, tl, ul), _, _, lpb, lpl = _joint_fwd(enc_proj, pred_proj, w_out, b_out, targets, logit_lengths,
                                                          target_lengths, int(blank), _PREC[precision],
-                                                         _ACT[activation], op="rnnt_forced_align")
+                                                         _ACT[activation], op="rnnt_forced_align",
+                                                         vocab_tiling=vocab_tiling)
     return rnnt_viterbi(lpb, lpl, tl, ul)
 
 

@@ -25,7 +25,8 @@ class GraphedJointRnntStep:
     graph pins their AccumulateGrad nodes to the stream it ran on, and the capture may not synchronise with that stream.
     `input_dtype=torch.bfloat16` keeps the captured input buffers in bf16 (the bf16 path rounds its inputs to bf16 in
     the first kernel anyway): a host pipeline then stages half the bytes per step.  `precision="bf16x3"` (tensor cores
-    at fp32 accuracy) needs fp32 inputs.
+    at fp32 accuracy) needs fp32 inputs.  `vocab_tiling=True` lets 'bf16' / 'bf16x3' take vocabularies beyond 416
+    (functional.fused_joint_rnnt_loss).
     `predictor=RNNPredictor(...)` puts the label side of Transducer._compute_rnnt_loss (transducer.py:168-172) into the
     step: `ys_in = [blank, targets]` is built in the captured region, the predictor (embedding, the LSTM sequence kernels
     of csrc/lstm_seq.cu, projection) produces `pred_out`, and its parameters get their gradients (and join the gradient
@@ -33,7 +34,8 @@ class GraphedJointRnntStep:
 
     def __init__(self, joint, B: int, T: int, U: int, blank: int, global_batch: Optional[int] = None,
                  precision: str = "fp32", clamp: float = -1.0, warmup: int = 3,
-                 input_dtype: torch.dtype = torch.float32, grad_exchange=None, predictor=None):
+                 input_dtype: torch.dtype = torch.float32, grad_exchange=None, predictor=None,
+                 vocab_tiling: bool = False):
         if precision == "bf16x3" and input_dtype != torch.float32:
             raise ValueError("precision='bf16x3' keeps fp32 accuracy end to end: input_dtype must be torch.float32")
         p0 = next(joint.parameters())
@@ -43,6 +45,7 @@ class GraphedJointRnntStep:
         E = joint.enc_ffn.in_features if joint.enc_ffn is not None else joint.ffn_out.in_features
         P = joint.pred_ffn.in_features if joint.pred_ffn is not None else joint.ffn_out.in_features
         self.joint, self.blank, self.precision, self.clamp = joint, int(blank), precision, float(clamp)
+        self.vocab_tiling = bool(vocab_tiling)
         self.gB = float(global_batch if global_batch is not None else B)
         self.grad_exchange = grad_exchange
         self.predictor = predictor
@@ -94,7 +97,8 @@ class GraphedJointRnntStep:
             self.ys_in[:, 1:].copy_(self.targets)
             pred = self.predictor(self.ys_in)
         costs = self.joint.rnnt_loss_fused(self.enc, pred, self.targets, self.logit_lengths, self.target_lengths,
-                                           self.blank, clamp=self.clamp, reduction="none", precision=self.precision)
+                                           self.blank, clamp=self.clamp, reduction="none", precision=self.precision,
+                                           vocab_tiling=self.vocab_tiling)
         # loss = sum_b cost_b / global_batch: the constant d loss / d cost_b vector seeds the backward directly (no
         # sum / div / fill / mul / expand kernels of the scalar-loss autograd chain), the value is one dot product
         torch.autograd.backward(costs, grad_tensors=self._seed)

@@ -139,12 +139,13 @@ class TransducerJoint(nn.Module):
 
     def rnnt_loss_fused(self, enc_out, pred_out, targets, logit_lengths, target_lengths, blank: int,
                         clamp: float = -1.0, reduction: str = "mean", precision: str = "fp32",
-                        pre_project: bool = True):
+                        pre_project: bool = True, vocab_tiling: bool = False):
         """joint + log-softmax + RNN-T lattice loss in one op (the seam of transducer.py:172-187).
         precision='fp32' keeps the reference's arithmetic; 'bf16' opts into the tcgen05 tensor-core path; 'bf16x3'
         runs the tensor-core path at fp32 accuracy (the pre-projections then stay fp32, as with 'fp32').
         Every activation ('tanh', 'relu', 'gelu') with or without pre-join and post-join linears is fused; the post-join
-        linear folds into the two inputs (`fused_joint_inputs`).  joint_mode must be 'add'."""
+        linear folds into the two inputs (`fused_joint_inputs`).  joint_mode must be 'add'.
+        vocab_tiling=True lets 'bf16' / 'bf16x3' take vocabularies beyond 416 (functional.fused_joint_rnnt_loss)."""
         if self.joint_mode != "add":
             raise RuntimeError("rnnt_loss_fused: only joint_mode='add'")
         if not self.fusable:
@@ -152,7 +153,7 @@ class TransducerJoint(nn.Module):
             e, p = fused_joint_inputs(self, enc_out, pred_out, lin, pre_project)
             return CF.fused_joint_rnnt_loss(e, p, self.ffn_out.weight, self.ffn_out.bias, targets, logit_lengths,
                                             target_lengths, blank, clamp, reduction, precision,
-                                            activation=self.activation_name)
+                                            activation=self.activation_name, vocab_tiling=vocab_tiling)
         if precision in ("bf16", CF.BF16) and enc_out.is_cuda:
             # bf16 path: the two pre-projections are plain library GEMMs; run them on the tensor cores too
             if pre_project and self.prejoin_linear and self.enc_ffn is not None and self.pred_ffn is not None:
@@ -163,15 +164,15 @@ class TransducerJoint(nn.Module):
         else:
             e, p = self.project(enc_out, pred_out, pre_project)
         return CF.fused_joint_rnnt_loss(e, p, self.ffn_out.weight, self.ffn_out.bias, targets, logit_lengths,
-                                        target_lengths, blank, clamp, reduction, precision)
+                                        target_lengths, blank, clamp, reduction, precision, vocab_tiling=vocab_tiling)
 
     @torch.no_grad()
     def forced_align(self, enc_out, pred_out, targets, logit_lengths, target_lengths, blank: int,
-                     precision: str = "fp32", pre_project: bool = True):
+                     precision: str = "fp32", pre_project: bool = True, vocab_tiling: bool = False):
         """Forced alignment of `targets` [B,U] through this joint (functional.rnnt_forced_align): the inputs go through
         the same pre-join / post-join handling as `rnnt_loss_fused` (every activation, joint_mode='add').  Returns
         (frames [B,U] int32, token_logprobs [B,U], scores [B])."""
         lin = _Bf16Linear.apply if precision in ("bf16", CF.BF16) and enc_out.is_cuda else F.linear
         e, p = fused_joint_inputs(self, enc_out, pred_out, lin, pre_project)
         return CF.rnnt_forced_align(e, p, self.ffn_out.weight, self.ffn_out.bias, targets, logit_lengths, target_lengths,
-                                    blank, precision, activation=self.activation_name)
+                                    blank, precision, activation=self.activation_name, vocab_tiling=vocab_tiling)

@@ -205,12 +205,14 @@ def _make_prefix_beam_search(seq_cls):
 
 
 # ------------------------------------------------------------------------------------------------ install
-def install(namespace=None, precision: Optional[str] = None) -> Dict[str, List[str]]:
+def install(namespace=None, precision: Optional[str] = None, vocab_tiling: Optional[bool] = None) -> Dict[str, List[str]]:
     """Patch whatever of the reference is present in `namespace` (None: import it).  Returns what was patched.
     `precision` ("fp32" | "bf16" | "bf16x3") becomes the class default of the patched `Transducer` (the fused loss
     reads `self.precision`, fp32 when absent), so an unchanged train script opts into the tcgen05 path with
     `install(precision="bf16")`, or into the tcgen05 path at fp32 accuracy with `install(precision="bf16x3")`; a model
-    instance can still override it with its own `precision` attribute."""
+    instance can still override it with its own `precision` attribute.  `vocab_tiling` (bool) becomes the class default of
+    `Transducer.vocab_tiling` the same way: `install(precision="bf16", vocab_tiling=True)` trains a vocabulary beyond 416
+    on the tensor cores."""
     if precision not in (None, "fp32", "bf16", "bf16x3"):
         raise ValueError("precision must be None, 'fp32', 'bf16' or 'bf16x3'")
     done: Dict[str, List[str]] = {}
@@ -235,6 +237,9 @@ def install(namespace=None, precision: Optional[str] = None) -> Dict[str, List[s
             if precision is not None:
                 _set(m.Transducer, "precision", precision)
                 note("transducer", f"Transducer.precision = {precision}")
+            if vocab_tiling is not None:
+                _set(m.Transducer, "vocab_tiling", bool(vocab_tiling))
+                note("transducer", f"Transducer.vocab_tiling = {bool(vocab_tiling)}")
         if hasattr(m, "basic_greedy_search"):
             _set(m, "basic_greedy_search", D.basic_greedy_search)
             note("transducer", "basic_greedy_search")

@@ -22,7 +22,7 @@ basic_greedy_search = D.basic_greedy_search
 class Transducer(nn.Module):
     def __init__(self, vocab_size: int, blank: int, encoder: nn.Module, predictor: nn.Module, joint: nn.Module,
                  ctc: Optional[nn.Module] = None, ctc_weight: float = 0.3, ignore_id: int = -1,
-                 transducer_weight: float = 0.7, precision: str = "fp32") -> None:
+                 transducer_weight: float = 0.7, precision: str = "fp32", vocab_tiling: bool = False) -> None:
         super().__init__()
         assert ctc_weight + transducer_weight == 1.0
         self.vocab_size = vocab_size
@@ -35,6 +35,7 @@ class Transducer(nn.Module):
         self.joint = joint
         self.ctc = ctc
         self.precision = precision
+        self.vocab_tiling = vocab_tiling      # 'bf16' / 'bf16x3' on vocabularies beyond 416 (vocabulary tiles)
 
     def forward(self, batch: dict, device: torch.device) -> Dict[str, Optional[torch.Tensor]]:
         speech = batch["feats"].to(device)
@@ -92,6 +93,7 @@ def compute_rnnt_loss(self, encoder_out, encoder_out_lens, text, text_lengths, c
     predictor_out = self.predictor(ys_in_pad)
     joint = self.joint
     precision = getattr(self, "precision", "fp32")      # reference arithmetic unless the model opts into bf16
+    vocab_tiling = getattr(self, "vocab_tiling", False)  # tensor cores for V > 416 only when the model opts in
     from . import functional as CF
     from .joint import fused_joint_inputs, joint_activation
     act = joint_activation(joint)                       # tanh / relu / exact gelu, anything else raises
@@ -102,7 +104,7 @@ def compute_rnnt_loss(self, encoder_out, encoder_out_lens, text, text_lengths, c
     else:
         e, p = fused_joint_inputs(joint, encoder_out, predictor_out)
     return CF.fused_joint_rnnt_loss(e, p, joint.ffn_out.weight, joint.ffn_out.bias, rnnt_text, t_len32, u_len32,
-                                    self.blank, clamp, "mean", precision, activation=act)
+                                    self.blank, clamp, "mean", precision, activation=act, vocab_tiling=vocab_tiling)
 
 
 @torch.no_grad()
@@ -116,6 +118,7 @@ def compute_rnnt_alignment(self, encoder_out, encoder_out_lens, text, text_lengt
     predictor_out = self.predictor(ys_in_pad)
     joint = self.joint
     precision = getattr(self, "precision", "fp32")
+    vocab_tiling = getattr(self, "vocab_tiling", False)
     from . import functional as CF
     from .joint import fused_joint_inputs, joint_activation
     act = joint_activation(joint)
@@ -125,4 +128,4 @@ def compute_rnnt_alignment(self, encoder_out, encoder_out_lens, text, text_lengt
     else:
         e, p = fused_joint_inputs(joint, encoder_out, predictor_out)
     return CF.rnnt_forced_align(e, p, joint.ffn_out.weight, joint.ffn_out.bias, rnnt_text, t_len32, u_len32,
-                                self.blank, precision, activation=act)
+                                self.blank, precision, activation=act, vocab_tiling=vocab_tiling)

@@ -122,6 +122,39 @@ int ctcvr_joint_rnnt_bwd_bf16in(const void* enc_proj_bf16, const void* pred_proj
                                 void* d_pred_proj_bf16, float* d_w_out, float* d_b_out, int B, int T, int U1, int D,
                                 int V, int blank, void* ws, size_t ws_bytes, void* stream);
 
+/* ---- vocabulary tiles: the fused forward / backward on the tensor cores for vocabularies beyond 416 entries.
+ * Same arguments, outputs and conventions as ctcvr_joint_rnnt_fwd / _bwd; `precision` is CTCVR_BF16 or CTCVR_BF16X3
+ * OR'ed with one CTCVR_ACT_* value (CTCVR_F32 is an error: ctcvr_joint_rnnt_fwd / _bwd take every V in fp32).
+ * ctcvr_joint_tc_vt_supported(): D % 128 == 0, D <= 512, U1 <= 128 and 1 <= V <= 32768.
+ *   - The vocabulary is cut into n = ceil(pad32(V) / 416) tiles of Vc = pad32(ceil(V / n)) columns; tile c covers
+ *     [c Vc, min(V, c Vc + Vc)) (V = 417: two tiles of 224 columns, the second with 193 real ones).  Each tile runs the
+ *     kernels of ctcvr_joint_rnnt_fwd / _bwd at a vocabulary of Vc: one launch per tile and direction.
+ *   - Forward: each tile's log-sum-exp is merged into lse in place (logaddexp), the tiles holding the blank and a
+ *     cell's label write its raw logit, and one final launch subtracts lse.  The outputs are those of the untiled call.
+ *   - Labels are clamped against the full V (an id outside [0, V) acts as blank), then located in their tile.
+ *   - Backward: g = softmax * gamma with the full lse; d_pred / d_b_out accumulate over the tiles, the d_enc partials
+ *     are stored by tile 0 and added by the others, and each tile's dW lands in its rows of d_w_out.
+ *   - Workspace (the _ws_bytes queries, independent of the activation bits): every tile's tiled weights, plus one
+ *     tile's G spill and dW partials, reused tile after tile in stream order.
+ *   - One tile (pad32(V) <= 416) runs the untiled entry point's kernels unchanged, with its workspace size.
+ * fp32 inputs only (bf16 activations convert to fp32 exactly; the bf16 path rounds them back). */
+int ctcvr_joint_tc_vt_supported(int U1, int D, int V);
+size_t ctcvr_joint_rnnt_fwd_vt_ws_bytes(int B, int T, int U1, int D, int V, int precision);
+int ctcvr_joint_rnnt_fwd_vt(const float* enc_proj, const float* pred_proj, const float* w_out,
+                            const float* b_out, const int32_t* targets, const int32_t* t_len,
+                            const int32_t* u_len, float* lse, float* lp_blank, float* lp_label,
+                            int B, int T, int U1, int D, int V, int blank, int precision,
+                            void* ws, size_t ws_bytes, void* stream);
+size_t ctcvr_joint_rnnt_bwd_vt_ws_bytes(int B, int T, int U1, int D, int V, int precision);
+int ctcvr_joint_rnnt_bwd_vt(const float* enc_proj, const float* pred_proj, const float* w_out,
+                            const float* b_out, const int32_t* targets, const int32_t* t_len,
+                            const int32_t* u_len, const float* lse, const float* lp_blank,
+                            const float* lp_label, const float* alpha,
+                            const float* beta, const float* costs, const float* grad_costs,
+                            float clamp, float* d_enc_proj, float* d_pred_proj, float* d_w_out,
+                            float* d_b_out, int B, int T, int U1, int D, int V, int blank,
+                            int precision, void* ws, size_t ws_bytes, void* stream);
+
 /* ---- section 8(f)3: glue of Transducer._compute_rnnt_loss / forward (model/component/transducer.py:8-19,113,168,
  * 174-178,122-128).  ctcvr_rnnt_prologue: ys_in [B,U+1] int64 = [blank, text]; targets [B,U] int32 = text with
  * ignore_id -> 0; t_len / u_len [B] int32 from the int64 encoder lengths and the int32 (or int64) text lengths - one

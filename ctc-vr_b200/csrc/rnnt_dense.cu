@@ -4,6 +4,8 @@
 // Used when a caller hands us materialised [B,T,U1,V] logits (e.g. TransducerJoint.forward called
 // directly).  The fused op in joint_simt.cu / joint_tc.cu is the hot path; this one reads the logits
 // twice (stats, gradient) instead of torchaudio's four passes.
+// Lengths are clamped to [0, T] and [0, U1 - 1] exactly as the lattice (lattice.cu) clamps them, and a label outside
+// [0, V) is read as blank, so both kernels and the lattice see one utterance and nothing indexes outside the tensors.
 #include "common.cuh"
 
 namespace ctcvr {
@@ -22,7 +24,8 @@ __global__ void dense_stats_kernel(const float* __restrict__ logits, const int32
   int u = cell % U1;
   int t = (cell / U1) % T;
   int b = cell / ((long)U1 * T);
-  if (t >= t_len[b] || u > u_len[b]) return;
+  const int Tb = max(min(t_len[b], T), 0), Ub = max(min(u_len[b], U1 - 1), 0);
+  if (t >= Tb || u > Ub) return;
   const float* x = logits + cell * V;
   float m = kNegInf;
   for (int v = lane; v < V; v += 32) m = fmaxf(m, x[v]);
@@ -34,7 +37,13 @@ __global__ void dense_stats_kernel(const float* __restrict__ logits, const int32
     float l = m + logf(s);
     lse[cell] = l;
     lpb[cell] = x[blank] - l;
-    lpl[cell] = (u < u_len[b]) ? x[targets[(long)b * (U1 - 1) + u]] - l : kNegInf;
+    if (u < Ub) {
+      int lab = targets[(long)b * (U1 - 1) + u];
+      if ((unsigned)lab >= (unsigned)V) lab = blank;
+      lpl[cell] = x[lab] - l;
+    } else {
+      lpl[cell] = kNegInf;
+    }
   }
 }
 
@@ -51,7 +60,7 @@ __global__ void dense_grad_kernel(const float* __restrict__ logits, const int32_
   int t = (cell / U1) % T;
   int b = cell / ((long)U1 * T);
   float* g = grads + cell * V;
-  const int Tb = t_len[b], Ub = u_len[b];
+  const int Tb = max(min(t_len[b], T), 0), Ub = max(min(u_len[b], U1 - 1), 0);
   if (t >= Tb || u > Ub) {
     for (int v = lane; v < V; v += 32) g[v] = 0.f;
     return;
@@ -65,7 +74,11 @@ __global__ void dense_grad_kernel(const float* __restrict__ logits, const int32_
   float k_blank = al + bnext + cost - l;
   float k_label = kNegInf;
   int lab = -1;
-  if (u < Ub) { k_label = al + beta[cell + 1] + cost - l; lab = targets[(long)b * (U1 - 1) + u]; }
+  if (u < Ub) {
+    k_label = al + beta[cell + 1] + cost - l;
+    lab = targets[(long)b * (U1 - 1) + u];
+    if ((unsigned)lab >= (unsigned)V) lab = blank;
+  }
   for (int v = lane; v < V; v += 32) {
     float xv = x[v];
     float gv = expf(xv + k_all);

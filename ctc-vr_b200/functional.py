@@ -221,7 +221,11 @@ class _RnntLossDense(torch.autograd.Function):
 def rnnt_loss(logits, targets, logit_lengths, target_lengths, blank: int = -1, clamp: float = -1,
               reduction: str = "mean", fused_log_softmax: bool = True):
     """Same signature and checks as torchaudio.functional.rnnt_loss (functional.py:1747-1800); the
-    validation errors of rnnt/cpu/compute.cpp:36-84 are raised as RuntimeError."""
+    validation errors of rnnt/cpu/compute.cpp:36-84 are raised as RuntimeError.  Those checks compare only the
+    longest lengths with the shape.  Values the reference leaves undefined are defined here and cannot index outside
+    the tensors: lengths are clamped to [0, T] and [0, U], so a negative length behaves exactly like 0 (no frames:
+    cost 0 and zero gradient; no labels: the blank-only path), and a label outside [0, V) behaves exactly like
+    `blank`, in the cost and the gradient."""
     if reduction not in ("none", "mean", "sum"):
         raise ValueError('reduction should be one of "none", "mean", or "sum"')
     _lib.require_cuda(logits)

@@ -219,7 +219,9 @@ int ctcvr_peer_destroy(void* ctx);
  * (site-packages/torchaudio/functional/functional.py:1725,1737-1744), fused_log_softmax=True.
  * logits [B,T,U1,V] fp32; costs [B]; grads [B,T,U1,V] (may be NULL) = d cost_b / d logits,
  * exact zeros at padded cells, clamped to +-clamp when clamp > 0.
- * ws: 5*B*T*U1 floats (ctcvr_rnnt_loss_dense_ws_bytes). */
+ * ws: 5*B*T*U1 floats (ctcvr_rnnt_loss_dense_ws_bytes).  t_len are clamped to [0, T] and u_len
+ * to [0, U1 - 1]: a negative length behaves exactly like 0, a longer one like the extent.  A
+ * label outside [0, V) behaves exactly like blank, in the cost and the gradient. */
 size_t ctcvr_rnnt_loss_dense_ws_bytes(int B, int T, int U1);
 int ctcvr_rnnt_loss_dense(const float* logits, const int32_t* targets, const int32_t* t_len,
                           const int32_t* u_len, float* costs, float* grads, int B, int T,
